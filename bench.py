@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the batched myCobot step on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pick|reach|push] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pick|reach|push] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one `step()` of every env of the workload = 20 physics substeps (joint controller) +
 observation / reward / success / auto-reset, i.e. one launch of the fused env kernel.  Default workload
@@ -43,6 +43,28 @@ WORKLOADS = {
 }
 METRIC = "env-steps/sec (pick-and-place, 16K envs/GPU) at 1/2/4/8 B200 vs CPU MuJoCo"
 UNIT = "env-steps/s"
+DUMP_BYTES = 60 * 10**6      # array data of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, step_out):
+    """Writes what `env.step` returned in the last timed step, one DIR/<name>.npy per array: float64 stays float64, the
+    rest becomes float32.  Above DUMP_BYTES in all, every array keeps the same seeded sample of envs (sorted), whose
+    indices go to env_index.npy.  Inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import torch
+
+    obs, reward, term, trunc, info = step_out
+    arrays = dict(obs, reward=reward, terminated=term, truncated=trunc, **info)
+    arrays = {k: v if v.dtype == torch.float64 else v.to(torch.float32) for k, v in arrays.items()}
+    n = reward.shape[0]
+    row_bytes = sum(v[0].numel() * v.element_size() for v in arrays.values())
+    if n * row_bytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+        rows = torch.as_tensor(idx, device=reward.device)
+        arrays = {k: v.index_select(0, rows) for k, v in arrays.items()}
+        arrays["env_index"] = torch.as_tensor(idx, dtype=torch.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.cpu().numpy())
 
 
 def her_relabel_leg(env, acts, dev, flush):
@@ -271,13 +293,15 @@ def run_ours(args):
     for t in range(K):
         flush.zero_()                      # L2 flush between timed iterations (outside the per-step events)
         ev[t][0].record()
-        env.step(acts[W + t])
+        last = env.step(acts[W + t])
         ev[t][1].record()
     stats = env.stats(reset=False).clone()
     fallback_envs = env.last_fallback_envs()   # after the timed loop's last launch (synchronises; outside the event intervals)
     all_reduce_stats(stats)                # the path's only collective: 8 doubles, once per rollout
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)   # before the e2e and HER legs step the env and overwrite its output buffers
     if world > 1:
         dist.barrier()
     allreduce_us = None
@@ -382,7 +406,13 @@ def main():
     ap.add_argument("--preroll", type=int, default=50, help="untimed steps before the warm-up (steady-state episode mix)")
     ap.add_argument("--no-her", action="store_true", help="skip the separately timed HER relabel leg")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU-port timing leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's envs) as DIR/<name>.npy, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -7,7 +7,8 @@ import pytest
 
 from mycobotgym_b200 import flatten, mjcf
 
-REF_XML = "/root/reference/mycobotgym/envs/assets/mycobot280.xml"
+# MyCobotGym's MJCF tree (mycobotgym/envs/assets) is not part of this repository: set MYCOBOT_ASSETS to recompile it
+REF_XML = os.path.join(os.environ["MYCOBOT_ASSETS"], "mycobot280.xml") if os.environ.get("MYCOBOT_ASSETS") else None
 
 
 @pytest.fixture(scope="module")
@@ -95,7 +96,7 @@ def test_setconst_products(flat):
     assert np.allclose(M, M.T) and np.all(np.linalg.eigvalsh(M) > 0)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_XML), reason="reference assets not mounted (GPU box)")
+@pytest.mark.skipif(not (REF_XML and os.path.exists(REF_XML)), reason="reference MJCF tree not found (set MYCOBOT_ASSETS)")
 def test_committed_json_matches_recompile(flat):
     log = []
     fresh = mjcf.compile_mjcf(REF_XML, log)
@@ -105,6 +106,71 @@ def test_committed_json_matches_recompile(flat):
         elif k != "compile_log":
             assert flat[k] == v, k
     assert any("base_link" in line for line in log)  # documented deviation: mesh absent from the mount
+
+
+def test_compiler_on_the_stored_mjcf_tree(tmp_path):
+    """compile_mjcf end to end on tests/golden/mjcf_tree (an include tree with the constructs of the reference's model: default
+    classes and childclass, box / mesh / explicit inertia, a missing mesh, duplicate mesh geoms, free and mocap bodies, exclude,
+    fixed tendon, connect, keyframe) against answers worked out by hand from the XML, then through the JSON round trip."""
+    log = []
+    m = mjcf.compile_mjcf(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "mjcf_tree", "model.xml"), log)
+    assert (m.nq, m.nv, m.nbody, m.njnt, m.nu, m.nsite, m.neq, m.nmocap, m.ntendon, m.ngeom, m.nM) == (11, 10, 7, 5, 2, 1, 1, 1, 1, 5, 30)
+    assert m.timestep == 0.004
+    np.testing.assert_array_equal(m.body_parentid, [0, 0, 1, 2, 2, 0, 0])
+    np.testing.assert_array_equal(m.body_weldid, [0, 1, 2, 3, 4, 5, 0])
+    np.testing.assert_array_equal(m.body_rootid, [0, 1, 1, 1, 1, 5, 6])
+    np.testing.assert_array_equal(m.body_mocapid, [-1, -1, -1, -1, -1, -1, 0])
+    np.testing.assert_array_equal(m.dof_parentid, [-1, 0, 1, 1, -1, 4, 5, 6, 7, 8])
+    np.testing.assert_array_equal(m.qpos0, [0, 0, 0, 0, 0.3, 0, 0.02, 1, 0, 0, 0])
+    np.testing.assert_allclose(m.body_quat[2], [np.sqrt(0.5), 0, 0, np.sqrt(0.5)], atol=1e-15)
+    # joint defaults: class "arm" on the links, "finger" (nested in "arm") on the fingers, built-ins on the free joint
+    np.testing.assert_array_equal(m.jnt_axis[0], [0, 0, 1])
+    np.testing.assert_array_equal(m.dof_armature, [0.1, 0.1, 0.005, 0.005, 0, 0, 0, 0, 0, 0])
+    np.testing.assert_array_equal(m.dof_damping, [1, 1, 0.1, 0.1, 0, 0, 0, 0, 0, 0])
+    np.testing.assert_array_equal(m.jnt_limited, [1, 1, 1, 1, 0])
+    np.testing.assert_array_equal(m.jnt_range[[0, 2]], [[-3, 3], [0, 0.7]])
+    np.testing.assert_array_equal(m.jnt_solref[[0, 2]], [[0.02, 1], [0.005, 1]])
+    # masses: boxes at density 500 (pad_b's mass given), the cube mesh (side 0.04) at 500, the missing mesh and the density-0
+    # copy add nothing; box inertia m/3 (b^2 + c^2) in decreasing order, cube m a^2 / 6 about its centroid
+    np.testing.assert_allclose(m.body_mass, [0, 0.04, 0.032, 0.004, 0.02, 0.008, 0], rtol=1e-6)
+    np.testing.assert_allclose(m.body_inertia[1], np.array([29, 26, 5]) * 1e-4 * 0.04 / 3, rtol=1e-12)
+    np.testing.assert_allclose(m.body_inertia[2], [0.032 * 0.04 ** 2 / 6] * 3, rtol=1e-6)
+    np.testing.assert_allclose(m.body_ipos[2], [0.03, 0, 0], atol=1e-9)
+    np.testing.assert_allclose(m.body_inertia[3:6], [[0.004 / 3 * 2e-4] * 3, [0.02 / 3 * 2e-4] * 3, [1e-6] * 3], rtol=1e-12)
+    np.testing.assert_allclose(m.body_subtreemass[:3], [0.104, 0.096, 0.056], rtol=1e-6)
+    assert any("mesh gone: file missing" in line for line in log)
+    # collision: plane / box geoms with their classes, one hull for the two cube geoms
+    assert m.geom_names == ["floor", "box1", "pad_a", "pad_b", "object0"]
+    np.testing.assert_array_equal(m.geom_friction[[1, 2]], [[1, 0.005, 0.0001], [0.95, 0.3, 0.1]])
+    np.testing.assert_array_equal(m.geom_condim, [3, 3, 4, 4, 3])
+    assert (m.nhull, list(m.hull_mult), list(m.hull_vertnum), m.hull_names) == (1, [2], [8], ["link2"])
+    hv = m.hull_vert[np.lexsort(m.hull_vert.T)]
+    want = np.array([[x, y, z] for z in (-0.02, 0.02) for y in (-0.02, 0.02) for x in (0.01, 0.05)])
+    np.testing.assert_allclose(hv, want, atol=1e-9)
+    np.testing.assert_allclose(m.hull_center[0], [0.03, 0, 0], atol=1e-9)
+    np.testing.assert_allclose(m.hull_rbound, [0.02 * np.sqrt(3)], rtol=1e-6)
+    # site, exclude, tendon, actuators, connect anchor 2 (set_const), keyframe
+    fk = mjcf.fk_numpy(m, m.qpos0)
+    np.testing.assert_allclose(fk[0][2] + fk[2][2] @ m.site_pos[0], [0.1, 0.05, 0.1], atol=1e-15)
+    np.testing.assert_array_equal(m.exclude, [[1, 2]])
+    np.testing.assert_array_equal(m.ten_J, [[0, 0, 0.5, 0.5, 0, 0, 0, 0, 0, 0]])
+    np.testing.assert_array_equal(m.actuator_moment, [[1, 0, 0, 0, 0, 0, 0, 0, 0, 0], [0, 0, 1, 1, 0, 0, 0, 0, 0, 0]])
+    np.testing.assert_array_equal(m.actuator_gain, [100, 70])
+    np.testing.assert_array_equal(m.actuator_biasprm, [[0, -100, -10]] * 2)
+    np.testing.assert_array_equal(m.actuator_forcelimited, [1, 0])
+    np.testing.assert_array_equal(m.actuator_ctrlrange, [[-3, 3], [0, 0.7]])
+    np.testing.assert_allclose(m.eq_data[0, :6], [0, 0.01, 0, 0, -0.01, 0], atol=1e-15)
+    np.testing.assert_array_equal(m.key_qpos, [[0.1, -0.2, 0.3, 0.3, 0.3, 0, 0.02, 1, 0, 0, 0]])
+    np.testing.assert_array_equal(m.key_ctrl, [[0.5, 0.2]])
+    np.testing.assert_array_equal(m.key_mpos, [[0, 0, 0.5]])
+    # set_const on the free body (centroid at its origin: translation and rotation decouple)
+    np.testing.assert_allclose(m.M0[4:7, 4:7], 0.008 * np.eye(3), rtol=1e-12)
+    np.testing.assert_allclose([m.body_invweight0[5, 0], m.dof_invweight0[4], m.dof_invweight0[7]], [125, 125, 1e6], rtol=1e-9)
+    assert np.allclose(m.M0, m.M0.T) and np.all(np.linalg.eigvalsh(m.M0) > 0)
+    # the committed assets are written and read through the same JSON + hull side file
+    m.to_json(str(tmp_path / "model.json"))
+    back = mjcf.FlatModel.from_json(str(tmp_path / "model.json"))
+    assert mjcf.diff_flatmodels(m, back, rtol=0) == {} and back.compile_log == m.compile_log
 
 
 def test_reduced_model_is_consistent(flat):

@@ -8,7 +8,7 @@ that has `mujoco` and the reference's MJCF tree these tests pin the three layers
   2. the CPU oracle's mj_forward / mj_step against MuJoCo's, from injected (qpos, qvel, ctrl, qacc_warmstart);
   3. nothing GPU-side: the CUDA engine is compared with the oracle in tests/test_gpu_parity.py.
 
-The MJCF tree is looked up in $MYCOBOT_ASSETS, an installed `mycobotgym` package, baseline/_ref, or /root/reference.
+The MJCF tree is looked up in $MYCOBOT_ASSETS, an installed `mycobotgym` package, or baseline/_ref.
 Mesh geoms do not collide in the oracle (documented gap), so the stepping comparison disables their contype /
 conaffinity on the MuJoCo side -- that isolates the gap instead of hiding it: `test_mesh_contacts_are_the_gap`
 reports how often the unmodified model produces a mesh contact on the same states.
@@ -25,8 +25,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _assets_dir():
-    cands = [os.environ.get("MYCOBOT_ASSETS"), os.path.join(ROOT, "baseline", "_ref", "mycobotgym", "envs", "assets"),
-             "/root/reference/mycobotgym/envs/assets"]
+    cands = [os.environ.get("MYCOBOT_ASSETS"), os.path.join(ROOT, "baseline", "_ref", "mycobotgym", "envs", "assets")]
     try:
         import mycobotgym  # noqa: F401  (needs gymnasium + glfw at import time, usually absent)
 
