@@ -255,7 +255,8 @@ int32_t mcb_stats(mcb_batch* b, double* out, int32_t reset_after, void* stream);
  * to host memory (`what` is reserved, pass 0).  Layout in doubles: nefc, ncon, solver iterations, overflow |
  * M[18*18] | qfrc_bias, qfrc_smooth, qacc_smooth, qacc, qfrc_constraint [18 each] | xpos[13*3] | xmat[13*9] |
  * efc_J[nefc*18] in MuJoCo row order (equality, limits, contacts) | efc_aref[nefc] | efc_D[nefc] |
- * (dist, pos3, normal3) * ncon.  cap must be >= 3170.  Returns the number of doubles written. */
+ * (dist, pos3, normal3) * ncon.  cap must be >= 4262, the dump's size for the last tier's 176 rows and 24 contacts; a smaller
+ * cap fails before anything runs.  Returns the number of doubles written. */
 int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out, int32_t cap, void* stream);
 
 /* Picks the lockstep grouping of the step kernel for this batch (cfg.lockstep_warps == 0): rolls the batch 32 steps

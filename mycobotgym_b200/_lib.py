@@ -13,7 +13,7 @@ from .flatten import HullDesc, ModelDesc, TaskCfg
 
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG_DIR)
-LIB_PATH = os.environ.get("MCB_LIB") or os.path.join(PKG_DIR, "libmycobot_b200.so")   # MCB_LIB: tuning experiments only
+LIB_PATH = os.environ.get("MCB_LIB") or os.path.join(PKG_DIR, "libmycobot_b200.so")   # MCB_LIB: load another build of the library, e.g. the canary build
 CANARY_PATH = os.path.join(PKG_DIR, "libmycobot_b200_canary.so")   # -DMCB_CANARY: guard words in the shared-memory records (tests only)
 SRC = os.path.join(PKG_DIR, "csrc", "mcb_engine.cu")
 HDR = os.path.join(ROOT, "include", "mycobot_b200.h")

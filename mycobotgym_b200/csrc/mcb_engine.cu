@@ -280,7 +280,7 @@ __device__ __forceinline__ void quat2mat(double* m, const double* q) {
 }
 
 
-#define WPB_SMALL_ 16      // warps (= envs) per CTA of the common-layout launch
+#define WPB_SMALL 16      // warps (= envs) per CTA of the common-layout launch
 
 // kinematic tree of the reduced model (flatten.reduce_model): arm 0..5, gripper sub-chains 6->7, 8->9, 10, 11 under body 5,
 // free cube 12.  fk() is written against this table; mcb_model_create checks the descriptor against it.
@@ -1979,8 +1979,8 @@ struct Newton {
 // `sync`: the warps of a CTA run the substep loop in lockstep (CTA barriers at the stage boundaries) so that they
 // share instruction-cache lines -- the kernel is thousands of straight-line instructions per substep and
 // independent warps drifting apart made instruction fetch the top stall (profiles/r01c).  Every path through
-// forward() executes exactly NSYNC_FWD barriers when sync is set.
-#define NSYNC_FWD __builtin_popcount(MCB_SYNC_MASK)
+// forward() executes exactly NSYNC_FWD barriers when sync is set: one at each of its six stage boundaries.
+#define NSYNC_FWD 6
 // Lockstep groups: `lw` consecutive warps of the CTA share one named barrier (ids 1..), so the CTA runs 16 / lw groups
 // that drift against each other (different stages -> different pipes busy at the same time) while the warps inside a
 // group still share instruction-cache lines.  lw = 1: free-running warps, no barriers.  Which grouping wins depends on
@@ -1988,31 +1988,27 @@ struct Newton {
 // (2.47 M vs 2.27 M env-steps/s in full lockstep), push and the mocap variant are 2x / 1.4x faster in full lockstep
 // (free-running they stall on instruction fetch, `no_instructions` 38 %).  mcb_autotune() measures and picks per batch.
 __device__ __forceinline__ void group_sync(int lw) {
-  if (lw >= WPB_SMALL_) __syncthreads();
+  if (lw >= WPB_SMALL) __syncthreads();
   else asm volatile("bar.sync %0, %1;" ::"r"(1 + (int)(threadIdx.x >> 5) / lw), "r"(32 * lw) : "memory");
 }
-#ifndef MCB_SYNC_MASK
-#define MCB_SYNC_MASK 0x3f      // which of forward()'s six stage boundaries carry a barrier (tuning experiments, profiles/README.md)
-#endif
-#define FSYNC(k) do { if (((MCB_SYNC_MASK) >> (k) & 1) && sync) group_sync(sync); } while (0)
 template <class S>
 __device__ __noinline__ bool forward(S& s, const DevModel* __restrict__ m, int lane, int nba, int nva, int sync) {
-  FSYNC(0);
+  if (sync) group_sync(sync);
   fk(s, m, lane, nba);
   cinert_cdof(s, m, lane, nba, nva);
-  FSYNC(1);
+  if (sync) group_sync(sync);
   crb_mass(s, m, lane, nba, nva);
   velocity_rne(s, m, lane, nba, nva);
-  FSYNC(2);
+  if (sync) group_sync(sync);
   actuation_smooth(s, m, lane, nva);
   double qs = factor_solve_M<true>(s.M, s.H, s.qfrc_smooth, s.Mv, 0.0, lane, nva);
   if (lane < nva) s.qacc_smooth[lane] = qs;
   __syncwarp();
-  FSYNC(3);
+  if (sync) group_sync(sync);
   collide(s, lane, nba, s.mesh != 0);
-  FSYNC(4);
+  if (sync) group_sync(sync);
   bool ok = make_rows(s, m, lane, nva);
-  FSYNC(5);
+  if (sync) group_sync(sync);
   if (!ok && !S::IS_BIG) return false;
   Newton<S> nw{s, m, lane, nva, s.nefc};
   nw.solve();
@@ -2392,14 +2388,10 @@ __device__ void debug_dump(S& s, const StepArgs& a, int lane, int nva) {
 // The env kernel: one warp per env.  TIER 0 is the first launch over all envs, WPB_SMALL warps per CTA; envs whose
 // constraint set overflows a tier's layout leave every output untouched and enqueue themselves on that tier's redo list,
 // which the next tier's launch serves (grid-stride over the list; tier 1: WPB_MID warps per CTA, tier 2: one).
-#define WPB_SMALL WPB_SMALL_
-#ifndef ENV_LB_THREADS
-#define ENV_LB_THREADS (32 * WPB_SMALL)      // register budget of the common-layout kernel = 65536 / ENV_LB_THREADS (tuning knob)
-#endif
 #define WPB_MID 10
 #define WPB_BIG 5       // last tier: five envs per CTA (one CTA per SM), so that they can run in lockstep like the other tiers
 template <int TIER>
-__global__ void __launch_bounds__(TIER == 0 ? ENV_LB_THREADS : TIER == 1 ? 32 * WPB_MID : 32 * WPB_BIG, 1) mcb_env_kernel(const __grid_constant__ StepArgs a) {   // (reset_env takes the arguments by reference: without __grid_constant__ the whole struct is copied to the stack)
+__global__ void __launch_bounds__(TIER == 0 ? 32 * WPB_SMALL : TIER == 1 ? 32 * WPB_MID : 32 * WPB_BIG, 1) mcb_env_kernel(const __grid_constant__ StepArgs a) {   // (reset_env takes the arguments by reference: without __grid_constant__ the whole struct is copied to the stack)
   typedef EnvS<TIER> S;
   constexpr bool BIG = TIER == 2;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -2433,7 +2425,7 @@ __global__ void __launch_bounds__(TIER == 0 ? ENV_LB_THREADS : TIER == 1 ? 32 * 
   }
   // the upper tiers always run their CTA in lockstep (their envs are the divergent, contact-rich ones: free-running they stall on
   // instruction fetch -- held grasp 59 -> 20 ms/step); the batch's grouping (mcb_autotune) only concerns the common-layout kernel
-  const int lockstep = TIER == 0 ? (a.lockstep_warps > 1 ? a.lockstep_warps : 0) : WPB_SMALL_;
+  const int lockstep = TIER == 0 ? (a.lockstep_warps > 1 ? a.lockstep_warps : 0) : WPB_SMALL;
 
   // Tier 0: CTA b takes the 16 consecutive envs [16 b, 16 b + 16).  Tier 1: the list is dealt round-robin over the CTAs
   // (item = slot * gridDim.x + b), so a list shorter than one full wave spreads over all SMs with few warps each instead of
@@ -2763,6 +2755,53 @@ struct DevGuard {
   ~DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
+// Row constants of mj_makeImpedance that do not depend on the state, computed once per model: `si` is clamped to getimpedance's
+// limits (slot 2 becomes 1 / width), and `KB` holds the row's solref on entry and its (K, B), refsafe applied, on return.  In the
+// DEVICE copy of the model every *_solref pair is overwritten with its (K, B) -- the kernels never need the raw solref.
+static void row_constants(double* KB, double* si, double timestep) {
+  si[0] = fmin(MAXIMP, fmax(MINIMP, si[0])); si[1] = fmin(MAXIMP, fmax(MINIMP, si[1])); si[2] = fmax(0.0, si[2]) <= MINVAL ? 0.0 : 1.0 / si[2];
+  si[3] = fmin(MAXIMP, fmax(MINIMP, si[3])); si[4] = fmax(1.0, si[4]);
+  double sr0 = KB[0], sr1 = KB[1];
+  if (sr0 > 0) sr0 = fmax(sr0, 2 * timestep);
+  const double dmax = si[1];
+  if (sr0 > 0) { KB[0] = 1 / fmax(MINVAL, dmax * dmax * sr0 * sr0 * sr1 * sr1); KB[1] = 2 / fmax(MINVAL, dmax * sr0); }
+  else { KB[0] = -sr0 / fmax(MINVAL, dmax * dmax); KB[1] = -sr1 / fmax(MINVAL, dmax); }
+}
+
+// One side of a candidate contact pair: a primitive geom of the model or a convex hull standing for `mult` identical mesh geoms.
+struct Side {
+  int condim; const double *friction, *solref, *solimp; double solmix; const double* invweight; int body, mult;
+};
+static Side geom_side(const mcb_model_desc& d, int g) {
+  return {d.geom_condim[g], d.geom_friction[g], d.geom_solref[g], d.geom_solimp[g], d.geom_solmix[g], d.geom_invweight[g], d.geom_body[g], 1};
+}
+static Side hull_side(const mcb_hull_desc& hd, int h) {
+  return {hd.condim[h], hd.friction[h], hd.solref[h], hd.solimp[h], hd.solmix[h], hd.invweight[h], hd.body[h], hd.mult[h]};
+}
+
+// Contact parameters of one pair (mj_contactParam, same priority: condim and friction as maxima, solref / solimp mixed by solmix)
+// and their row constants.  The caller fills g1 / g2.  Returns false for a condim other than 3 or 4.
+static bool pair_param(PairParam& pp, const Side& a, const Side& b, double timestep, double impratio) {
+  pp.b1 = a.body; pp.b2 = b.body;
+  pp.dim = a.condim > b.condim ? a.condim : b.condim;
+  if (pp.dim != 3 && pp.dim != 4) return false;
+  for (int k = 0; k < 3; k++) pp.friction[k] = fmax(a.friction[k], b.friction[k]);
+  double mix;
+  if (a.solmix >= MINVAL && b.solmix >= MINVAL) mix = a.solmix / (a.solmix + b.solmix);
+  else if (a.solmix < MINVAL && b.solmix < MINVAL) mix = 0.5;
+  else if (a.solmix < MINVAL) mix = 0.0; else mix = 1.0;
+  if (a.solref[0] > 0 && b.solref[0] > 0) for (int k = 0; k < 2; k++) pp.KB[k] = mix * a.solref[k] + (1 - mix) * b.solref[k];
+  else for (int k = 0; k < 2; k++) pp.KB[k] = fmin(a.solref[k], b.solref[k]);
+  for (int k = 0; k < 5; k++) pp.solimp[k] = mix * a.solimp[k] + (1 - mix) * b.solimp[k];
+  { const bool c1 = a.body == CUBE, c2 = b.body == CUBE, r1 = a.body >= 0 && !c1, r2 = b.body >= 0 && !c2;
+    pp.ptype = ((c1 || c2) && (r1 || r2)) ? 2 : ((c1 || c2) ? 1 : 0); }
+  pp.tran = a.invweight[0] + b.invweight[0];
+  row_constants(pp.KB, pp.solimp, timestep);
+  const double pyr = pp.friction[0] / sqrt(impratio);
+  pp.pyr2 = 2 * pyr * pyr / (double)(a.mult * b.mult);      // `mult` identical contacts (twin mesh geoms) == one contact with R / mult
+  return true;
+}
+
 struct mcb_model {
   int device;
   DevModel* dev;
@@ -2812,6 +2851,55 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
   return 0;
 }
 
+// The staging buffers of mcb_step_host exist all together or not at all (the pointers are null).
+static void free_staging(mcb_batch* b) {
+  cudaFree(b->d_actions); cudaFree(b->d_obs); cudaFree(b->d_fobs); cudaFree(b->d_ag); cudaFree(b->d_dg); cudaFree(b->d_reward); cudaFree(b->d_flags);
+  void* host[7] = {b->h_actions, b->h_obs, b->h_fobs, b->h_ag, b->h_dg, b->h_reward, b->h_flags};
+  for (void* p : host) if (p) cudaFreeHost(p);
+  b->d_actions = nullptr; b->d_obs = b->d_fobs = b->d_ag = b->d_dg = nullptr; b->d_reward = nullptr; b->d_flags = nullptr;
+  b->h_actions = nullptr; b->h_obs = b->h_fobs = b->h_ag = b->h_dg = nullptr; b->h_reward = nullptr; b->h_flags = nullptr;
+}
+static cudaError_t alloc_staging(mcb_batch* b) {
+  const size_t N = (size_t)b->n_envs, od = (size_t)b->obs_dim, ad = (size_t)mcb_batch_action_dim(b);
+  cudaError_t e = cudaSuccess;
+  auto dev = [&](auto** p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes); };
+  auto host = [&](auto** p, size_t bytes) { if (e == cudaSuccess) e = cudaMallocHost(p, bytes); };
+  dev(&b->d_actions, N * ad * sizeof(float)); host(&b->h_actions, N * ad * sizeof(float));
+  dev(&b->d_obs, N * od * sizeof(double)); host(&b->h_obs, N * od * sizeof(double));
+  dev(&b->d_fobs, N * od * sizeof(double)); host(&b->h_fobs, N * od * sizeof(double));
+  dev(&b->d_ag, N * 3 * sizeof(double)); host(&b->h_ag, N * 3 * sizeof(double));
+  dev(&b->d_dg, N * 3 * sizeof(double)); host(&b->h_dg, N * 3 * sizeof(double));
+  dev(&b->d_reward, N * sizeof(double)); host(&b->h_reward, N * sizeof(double));
+  dev(&b->d_flags, N * 3); host(&b->h_flags, N * 3);
+  if (e == cudaSuccess) e = cudaMemset(b->d_fobs, 0, N * od * sizeof(double));      // rows of envs that did not auto-reset are never written
+  if (e != cudaSuccess) free_staging(b);
+  return e;
+}
+
+// A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics.
+// The buffers are allocated by the first save() and freed with the snapshot.
+struct Snapshot {
+  const mcb_batch* b;
+  void* copy[5] = {};
+  explicit Snapshot(const mcb_batch* batch) : b(batch) {}
+  ~Snapshot() { for (void* p : copy) cudaFree(p); }
+  cudaError_t save(cudaStream_t st) { return transfer(true, st); }
+  cudaError_t restore(cudaStream_t st) { return transfer(false, st); }
+
+ private:
+  cudaError_t transfer(bool save, cudaStream_t st) {
+    const size_t N = (size_t)b->n_envs;
+    void* live[5] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats};
+    const size_t bytes[5] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double)};
+    cudaError_t e = cudaSuccess;
+    for (int k = 0; k < 5 && e == cudaSuccess; k++) {
+      if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes[k]);
+      if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live[k], save ? live[k] : copy[k], bytes[k], cudaMemcpyDeviceToDevice, st);
+    }
+    return e;
+  }
+};
+
 extern "C" {
 
 const char* mcb_version(void) {
@@ -2859,55 +2947,16 @@ int32_t mcb_model_create(const mcb_model_desc* d, int32_t device, mcb_model** ou
   // contact parameter mixing per candidate pair (mj_collideGeoms / mj_contactParam)
   if (d->npair > MCB_MAXPAIR) { delete m; return fail("mcb_model_create: too many pairs"); }
   for (int p = 0; p < d->npair; p++) {
-    int g1 = d->pair_g1[p], g2 = d->pair_g2[p];
+    const int g1 = d->pair_g1[p], g2 = d->pair_g2[p];
     PairParam& pp = h.pair[p];
     pp.g1 = g1; pp.g2 = g2;
-    pp.b1 = d->geom_body[g1]; pp.b2 = d->geom_body[g2];
-    pp.dim = d->geom_condim[g1] > d->geom_condim[g2] ? d->geom_condim[g1] : d->geom_condim[g2];
-    if (pp.dim != 3 && pp.dim != 4) { delete m; return fail("mcb_model_create: only condim 3 and 4 are supported"); }
-    double fr[3];
-    for (int k = 0; k < 3; k++) fr[k] = fmax(d->geom_friction[g1][k], d->geom_friction[g2][k]);
-    pp.friction[0] = fr[0]; pp.friction[1] = fr[1]; pp.friction[2] = fr[2];
-    double sa = d->geom_solmix[g1], sb = d->geom_solmix[g2], mix;
-    if (sa >= MINVAL && sb >= MINVAL) mix = sa / (sa + sb);
-    else if (sa < MINVAL && sb < MINVAL) mix = 0.5;
-    else if (sa < MINVAL) mix = 0.0; else mix = 1.0;
-    const double *ra = d->geom_solref[g1], *rb = d->geom_solref[g2];
-    if (ra[0] > 0 && rb[0] > 0) for (int k = 0; k < 2; k++) pp.KB[k] = mix * ra[k] + (1 - mix) * rb[k];
-    else for (int k = 0; k < 2; k++) pp.KB[k] = fmin(ra[k], rb[k]);
-    for (int k = 0; k < 5; k++) pp.solimp[k] = mix * d->geom_solimp[g1][k] + (1 - mix) * d->geom_solimp[g2][k];
-    { int b1 = d->geom_body[g1], b2 = d->geom_body[g2]; bool c1 = b1 == CUBE, c2 = b2 == CUBE, r1 = b1 >= 0 && !c1, r2 = b2 >= 0 && !c2;
-      pp.ptype = ((c1 || c2) && (r1 || r2)) ? 2 : ((c1 || c2) ? 1 : 0); }
-    pp.tran = d->geom_invweight[g1][0] + d->geom_invweight[g2][0];
+    if (!pair_param(pp, geom_side(*d, g1), geom_side(*d, g2), d->timestep, d->impratio)) { delete m; return fail("mcb_model_create: only condim 3 and 4 are supported"); }
   }
-  // row constants of mj_makeImpedance that do not depend on the state: solimp clamped once, (K, B) from solref (refsafe applied).
-  // In the DEVICE copy of the model every *_solref pair is overwritten with its (K, B) -- the kernels never need the raw solref.
-  {
-    auto clamp_solimp = [](double* si) {
-      si[0] = fmin(MAXIMP, fmax(MINIMP, si[0])); si[1] = fmin(MAXIMP, fmax(MINIMP, si[1])); si[2] = fmax(0.0, si[2]) <= MINVAL ? 0.0 : 1.0 / si[2];   // slot 2: 1 / width
-      si[3] = fmin(MAXIMP, fmax(MINIMP, si[3])); si[4] = fmax(1.0, si[4]);
-    };
-    const double hstep = h.d.timestep;
-    auto row_constants = [hstep](double* solref_to_KB, const double* solimp_clamped) {
-      double* KB = solref_to_KB;
-      double sr0 = KB[0], sr1 = KB[1];
-      if (sr0 > 0) sr0 = fmax(sr0, 2 * hstep);
-      const double dmax = solimp_clamped[1];
-      if (sr0 > 0) { KB[0] = 1 / fmax(MINVAL, dmax * dmax * sr0 * sr0 * sr1 * sr1); KB[1] = 2 / fmax(MINVAL, dmax * sr0); }
-      else { KB[0] = -sr0 / fmax(MINVAL, dmax * dmax); KB[1] = -sr1 / fmax(MINVAL, dmax); }
-    };
-    for (int e = 0; e < 2; e++) { clamp_solimp(h.d.con_solimp[e]); row_constants(h.d.con_solref[e], h.d.con_solimp[e]); }
-    clamp_solimp(h.d.jeq_solimp); row_constants(h.d.jeq_solref, h.d.jeq_solimp);
-    clamp_solimp(h.d.weld_solimp); row_constants(h.d.weld_solref, h.d.weld_solimp);
-    for (int j = 0; j < NH; j++) { clamp_solimp(h.d.jnt_solimp[j]); row_constants(h.d.jnt_solref[j], h.d.jnt_solimp[j]); }
-    for (int p = 0; p < d->npair; p++) {
-      PairParam& pp = h.pair[p];
-      clamp_solimp(pp.solimp);
-      row_constants(pp.KB, pp.solimp);
-      const double pyr = pp.friction[0] / sqrt(h.d.impratio);
-      pp.pyr2 = 2 * pyr * pyr;
-    }
-  }
+  const double ts = h.d.timestep;
+  for (int e = 0; e < 2; e++) row_constants(h.d.con_solref[e], h.d.con_solimp[e], ts);
+  row_constants(h.d.jeq_solref, h.d.jeq_solimp, ts);
+  row_constants(h.d.weld_solref, h.d.weld_solimp, ts);
+  for (int j = 0; j < NH; j++) row_constants(h.d.jnt_solref[j], h.d.jnt_solimp[j], ts);
   cudaError_t ce = cudaMalloc(&m->dev, sizeof(DevModel));
   if (ce == cudaSuccess) ce = cudaMemcpy(m->dev, &h, sizeof(DevModel), cudaMemcpyHostToDevice);
   if (ce != cudaSuccess) { cudaFree(m->dev); delete m; return fail("mcb_model_create: upload", ce); }
@@ -2923,8 +2972,9 @@ int32_t mcb_model_set_hulls(mcb_model* m, const mcb_hull_desc* hd) {
     return fail("mcb_model_set_hulls: counts out of range");
   DevGuard guard(m->device);
   if (!guard.ok) return fail("mcb_model_set_hulls: cannot select the model's device", cudaGetLastError());
-  DevModel& h = m->host;
-  const mcb_model_desc& d = h.d;
+  // everything is validated and uploaded into a copy of the host model first: a rejected descriptor or a failed upload leaves the
+  // model as it was
+  DevModel h = m->host;
   std::vector<PairParam> pps((size_t)hd->npair);
   for (int hq = 0; hq < hd->nhull; hq++) {
     if (hd->body[hq] < 0 || hd->body[hq] >= NB || hd->vadr[hq] < 0 || hd->vnum[hq] <= 0 || hd->vadr[hq] + hd->vnum[hq] > hd->nvert || hd->mult[hq] < 1 ||
@@ -2934,62 +2984,27 @@ int32_t mcb_model_set_hulls(mcb_model* m, const mcb_hull_desc* hd) {
     for (int k = 0; k < 3; k++) h.hull_center[hq][k] = hd->center[hq][k];
     h.hull_rbound[hq] = hd->rbound[hq];
   }
-  auto clamp_solimp = [](double* si) {
-    si[0] = fmin(MAXIMP, fmax(MINIMP, si[0])); si[1] = fmin(MAXIMP, fmax(MINIMP, si[1])); si[2] = fmax(0.0, si[2]) <= MINVAL ? 0.0 : 1.0 / si[2];
-    si[3] = fmin(MAXIMP, fmax(MINIMP, si[3])); si[4] = fmax(1.0, si[4]);
-  };
   for (int p = 0; p < hd->npair; p++) {
     const int oa = hd->pair_a[p], ob = hd->pair_b[p];
     if (ob < MCB_NGEOM || ob >= MCB_NGEOM + hd->nhull || oa >= MCB_NGEOM + hd->nhull || (oa >= MCB_NGEOM && oa >= ob)) return fail("mcb_model_set_hulls: bad pair");
     h.hpair_a[p] = (unsigned char)oa; h.hpair_b[p] = (unsigned char)ob;
-    const int hb = ob - MCB_NGEOM, ha = oa - MCB_NGEOM;
-    // object a: primitive geom or hull; object b: always a hull (mj_contactParam, same priority)
-    const int cd1 = ha >= 0 ? hd->condim[ha] : d.geom_condim[oa];
-    const double* f1 = ha >= 0 ? hd->friction[ha] : d.geom_friction[oa];
-    const double* r1 = ha >= 0 ? hd->solref[ha] : d.geom_solref[oa];
-    const double* i1 = ha >= 0 ? hd->solimp[ha] : d.geom_solimp[oa];
-    const double s1 = ha >= 0 ? hd->solmix[ha] : d.geom_solmix[oa];
-    const double* w1 = ha >= 0 ? hd->invweight[ha] : d.geom_invweight[oa];
-    const int m1 = ha >= 0 ? hd->mult[ha] : 1;
-    const int bo1 = ha >= 0 ? hd->body[ha] : d.geom_body[oa];
+    // object a: primitive geom or hull; object b: always a hull
     PairParam& pp = pps[(size_t)p];
-    memset(&pp, 0, sizeof pp);
-    pp.g1 = oa; pp.g2 = ob; pp.b1 = bo1; pp.b2 = hd->body[hb];
-    pp.dim = cd1 > hd->condim[hb] ? cd1 : hd->condim[hb];
-    if (pp.dim != 3 && pp.dim != 4) return fail("mcb_model_set_hulls: only condim 3 and 4 are supported");
-    for (int k = 0; k < 3; k++) pp.friction[k] = fmax(f1[k], hd->friction[hb][k]);
-    const double sa = s1, sb = hd->solmix[hb];
-    double mix;
-    if (sa >= MINVAL && sb >= MINVAL) mix = sa / (sa + sb);
-    else if (sa < MINVAL && sb < MINVAL) mix = 0.5;
-    else if (sa < MINVAL) mix = 0.0; else mix = 1.0;
-    const double* r2 = hd->solref[hb];
-    if (r1[0] > 0 && r2[0] > 0) for (int k = 0; k < 2; k++) pp.KB[k] = mix * r1[k] + (1 - mix) * r2[k];
-    else for (int k = 0; k < 2; k++) pp.KB[k] = fmin(r1[k], r2[k]);
-    for (int k = 0; k < 5; k++) pp.solimp[k] = mix * i1[k] + (1 - mix) * hd->solimp[hb][k];
-    { const bool c1 = pp.b1 == CUBE, c2 = pp.b2 == CUBE, q1 = pp.b1 >= 0 && !c1, q2 = pp.b2 >= 0 && !c2;
-      pp.ptype = ((c1 || c2) && (q1 || q2)) ? 2 : ((c1 || c2) ? 1 : 0); }
-    pp.tran = w1[0] + hd->invweight[hb][0];
-    clamp_solimp(pp.solimp);
-    { double sr0 = pp.KB[0], sr1 = pp.KB[1];        // (K, B) from the mixed solref, refsafe applied -- as for the primitive pairs
-      if (sr0 > 0) sr0 = fmax(sr0, 2 * d.timestep);
-      const double dmax = pp.solimp[1];
-      if (sr0 > 0) { pp.KB[0] = 1 / fmax(MINVAL, dmax * dmax * sr0 * sr0 * sr1 * sr1); pp.KB[1] = 2 / fmax(MINVAL, dmax * sr0); }
-      else { pp.KB[0] = -sr0 / fmax(MINVAL, dmax * dmax); pp.KB[1] = -sr1 / fmax(MINVAL, dmax); } }
-    const double pyr = pp.friction[0] / sqrt(d.impratio);
-    pp.pyr2 = 2 * pyr * pyr / (double)(m1 * hd->mult[hb]);      // `mult` identical contacts (twin mesh geoms) == one contact with R / mult
+    pp.g1 = oa; pp.g2 = ob;
+    const Side a = oa >= MCB_NGEOM ? hull_side(*hd, oa - MCB_NGEOM) : geom_side(h.d, oa);
+    if (!pair_param(pp, a, hull_side(*hd, ob - MCB_NGEOM), h.d.timestep, h.d.impratio)) return fail("mcb_model_set_hulls: only condim 3 and 4 are supported");
   }
-  cudaFree(m->d_hull_vert); cudaFree(m->d_hpair); m->d_hull_vert = nullptr; m->d_hpair = nullptr;
-  if (hd->nvert > 0) {
-    CK(cudaMalloc(&m->d_hull_vert, (size_t)hd->nvert * 3 * sizeof(double)));
-    CK(cudaMemcpy(m->d_hull_vert, hd->vert, (size_t)hd->nvert * 3 * sizeof(double), cudaMemcpyHostToDevice));
-  }
-  if (hd->npair > 0) {
-    CK(cudaMalloc(&m->d_hpair, (size_t)hd->npair * sizeof(PairParam)));
-    CK(cudaMemcpy(m->d_hpair, pps.data(), (size_t)hd->npair * sizeof(PairParam), cudaMemcpyHostToDevice));
-  }
-  h.nhull = hd->nhull; h.nhpair = hd->npair; h.hull_vert = m->d_hull_vert; h.hpair_param = m->d_hpair;
-  CK(cudaMemcpy(m->dev, &h, sizeof(DevModel), cudaMemcpyHostToDevice));
+  double* vert = nullptr;
+  PairParam* hpair = nullptr;
+  const size_t vbytes = (size_t)hd->nvert * 3 * sizeof(double), pbytes = (size_t)hd->npair * sizeof(PairParam);
+  cudaError_t e = cudaSuccess;
+  if (vbytes) { e = cudaMalloc(&vert, vbytes); if (e == cudaSuccess) e = cudaMemcpy(vert, hd->vert, vbytes, cudaMemcpyHostToDevice); }
+  if (pbytes && e == cudaSuccess) { e = cudaMalloc(&hpair, pbytes); if (e == cudaSuccess) e = cudaMemcpy(hpair, pps.data(), pbytes, cudaMemcpyHostToDevice); }
+  h.nhull = hd->nhull; h.nhpair = hd->npair; h.hull_vert = vert; h.hpair_param = hpair;
+  if (e == cudaSuccess) e = cudaMemcpy(m->dev, &h, sizeof(DevModel), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) { cudaFree(vert); cudaFree(hpair); return fail("mcb_model_set_hulls: upload", e); }
+  cudaFree(m->d_hull_vert); cudaFree(m->d_hpair);
+  m->d_hull_vert = vert; m->d_hpair = hpair; m->host = h;
   return 0;
 }
 
@@ -3061,8 +3076,7 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
 int32_t mcb_batch_destroy(mcb_batch* b) {
   if (!b) return 0;
   cudaFree(b->state); cudaFree(b->elapsed); cudaFree(b->ep_return); cudaFree(b->rng_ctr); cudaFree(b->env_seed); cudaFree(b->stats); cudaFree(b->debug); cudaFree(b->redo_count); cudaFree(b->redo_list);
-  if (b->d_actions) { cudaFree(b->d_actions); cudaFree(b->d_obs); cudaFree(b->d_fobs); cudaFree(b->d_ag); cudaFree(b->d_dg); cudaFree(b->d_reward); cudaFree(b->d_flags); }
-  if (b->h_actions) { cudaFreeHost(b->h_actions); cudaFreeHost(b->h_obs); cudaFreeHost(b->h_fobs); cudaFreeHost(b->h_ag); cudaFreeHost(b->h_dg); cudaFreeHost(b->h_reward); cudaFreeHost(b->h_flags); }
+  free_staging(b);
   delete b;
   return 0;
 }
@@ -3108,68 +3122,46 @@ int32_t mcb_autotune(mcb_batch* b, const float* actions, int32_t steps_per_candi
   const int K = steps_per_candidate > 0 ? steps_per_candidate : 4;
   const size_t N = (size_t)b->n_envs;
   const size_t adim = (size_t)mcb_batch_action_dim(b);
-  // snapshot of everything a step mutates; every candidate replays the same K steps from it and it is restored at the end
-  double *sv_state = nullptr, *sv_ret = nullptr, *sv_stats = nullptr; int* sv_el = nullptr; unsigned long long* sv_ctr = nullptr;
+  // every candidate replays the same K steps from the tuning state; the caller's state is restored at the end
+  Snapshot caller(b), tuning(b);
   void* t_reward = nullptr; uint8_t* t_flags = nullptr; float* t_act = nullptr;
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   int best = b->lockstep_warps;
   float best_ms = 1e30f;
   bool okay = true;
 #define TCK(call) do { if (okay && (call) != cudaSuccess) okay = false; } while (0)
-  TCK(cudaMalloc(&sv_state, N * MCB_STATE_STRIDE * sizeof(double))); TCK(cudaMalloc(&sv_ret, N * sizeof(double)));
-  TCK(cudaMalloc(&sv_stats, 8 * sizeof(double))); TCK(cudaMalloc(&sv_el, N * sizeof(int))); TCK(cudaMalloc(&sv_ctr, N * sizeof(unsigned long long)));
   TCK(cudaMalloc(&t_reward, N * sizeof(double))); TCK(cudaMalloc(&t_flags, 3 * N));
   if (!actions) TCK(cudaMalloc(&t_act, N * adim * sizeof(float)));
   TCK(cudaEventCreate(&e0)); TCK(cudaEventCreate(&e1));
-  if (okay) {
-    TCK(cudaMemcpyAsync(sv_state, b->state, N * MCB_STATE_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(sv_ret, b->ep_return, N * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(sv_stats, b->stats, 8 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(sv_el, b->elapsed, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(sv_ctr, b->rng_ctr, N * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
-    auto one_step = [&](int k) {
-      if (!actions) { random_actions_kernel<<<(unsigned)((N * adim + 255) / 256), 256, 0, st>>>(t_act, (int)(N * adim), b->seed ^ 0x74756e65ull, (unsigned)k); b->launches_total++; }
-      StepArgs a; memset(&a, 0, sizeof a);
-      a.mode = MODE_STEP; a.actions = actions ? actions : t_act; a.reward = t_reward;
-      a.terminated = t_flags; a.truncated = t_flags + N; a.success = t_flags + 2 * N;
-      if (launch(b, a, st)) okay = false;
-    };
-    // roll ahead (state right after a reset is not representative: nothing moves yet), then snapshot the tuning state
-    double* tn_state = nullptr; double* tn_ret = nullptr; int* tn_el = nullptr; unsigned long long* tn_ctr = nullptr;
-    TCK(cudaMalloc(&tn_state, N * MCB_STATE_STRIDE * sizeof(double))); TCK(cudaMalloc(&tn_ret, N * sizeof(double)));
-    TCK(cudaMalloc(&tn_el, N * sizeof(int))); TCK(cudaMalloc(&tn_ctr, N * sizeof(unsigned long long)));
-    for (int k = 0; k < 32 && okay; k++) one_step(k);
-    TCK(cudaMemcpyAsync(tn_state, b->state, N * MCB_STATE_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(tn_ret, b->ep_return, N * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(tn_el, b->elapsed, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(tn_ctr, b->rng_ctr, N * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
-    const int cand[3] = {WPB_SMALL, 4, 1};
-    for (int c = 0; c < 3 && okay; c++) {
-      b->lockstep_warps = cand[c];
-      TCK(cudaMemcpyAsync(b->state, tn_state, N * MCB_STATE_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, st));
-      TCK(cudaMemcpyAsync(b->ep_return, tn_ret, N * sizeof(double), cudaMemcpyDeviceToDevice, st));
-      TCK(cudaMemcpyAsync(b->elapsed, tn_el, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
-      TCK(cudaMemcpyAsync(b->rng_ctr, tn_ctr, N * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
-      for (int k = 0; k <= K && okay; k++) {          // step 0 is the untimed warm-up of this candidate
-        if (k == 1) TCK(cudaEventRecord(e0, st));
-        one_step(100 + k);
-      }
-      TCK(cudaEventRecord(e1, st));
-      TCK(cudaEventSynchronize(e1));
-      float ms = 0;
-      TCK(cudaEventElapsedTime(&ms, e0, e1));
-      if (okay && ms < best_ms) { best_ms = ms; best = cand[c]; }
+  TCK(caller.save(st));
+  auto one_step = [&](int k) {
+    if (!actions) { random_actions_kernel<<<(unsigned)((N * adim + 255) / 256), 256, 0, st>>>(t_act, (int)(N * adim), b->seed ^ 0x74756e65ull, (unsigned)k); b->launches_total++; }
+    StepArgs a; memset(&a, 0, sizeof a);
+    a.mode = MODE_STEP; a.actions = actions ? actions : t_act; a.reward = t_reward;
+    a.terminated = t_flags; a.truncated = t_flags + N; a.success = t_flags + 2 * N;
+    if (launch(b, a, st)) okay = false;
+  };
+  // roll ahead (state right after a reset is not representative: nothing moves yet), then snapshot the tuning state
+  for (int k = 0; k < 32 && okay; k++) one_step(k);
+  TCK(tuning.save(st));
+  const int cand[3] = {WPB_SMALL, 4, 1};
+  for (int c = 0; c < 3 && okay; c++) {
+    b->lockstep_warps = cand[c];
+    TCK(tuning.restore(st));
+    for (int k = 0; k <= K && okay; k++) {          // step 0 is the untimed warm-up of this candidate
+      if (k == 1) TCK(cudaEventRecord(e0, st));
+      one_step(100 + k);
     }
-    TCK(cudaMemcpyAsync(b->state, sv_state, N * MCB_STATE_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(b->ep_return, sv_ret, N * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(b->stats, sv_stats, 8 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(b->elapsed, sv_el, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaMemcpyAsync(b->rng_ctr, sv_ctr, N * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
-    TCK(cudaStreamSynchronize(st));
-    cudaFree(tn_state); cudaFree(tn_ret); cudaFree(tn_el); cudaFree(tn_ctr);
+    TCK(cudaEventRecord(e1, st));
+    TCK(cudaEventSynchronize(e1));
+    float ms = 0;
+    TCK(cudaEventElapsedTime(&ms, e0, e1));
+    if (okay && ms < best_ms) { best_ms = ms; best = cand[c]; }
   }
+  TCK(caller.restore(st));
+  TCK(cudaStreamSynchronize(st));
 #undef TCK
-  cudaFree(sv_state); cudaFree(sv_ret); cudaFree(sv_stats); cudaFree(sv_el); cudaFree(sv_ctr); cudaFree(t_reward); cudaFree(t_flags); cudaFree(t_act);
+  cudaFree(t_reward); cudaFree(t_flags); cudaFree(t_act);
   if (e0) cudaEventDestroy(e0);
   if (e1) cudaEventDestroy(e1);
   b->lockstep_warps = best;
@@ -3187,14 +3179,13 @@ int32_t mcb_forward(mcb_batch* b, double* obs, double* ag, double* dg, void* str
 int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out, int32_t cap, void* stream) {
   if (!b || env < 0 || env >= b->n_envs) return fail("mcb_debug_forward: bad argument");
   (void)what;
+  if (cap < DEBUG_DOUBLES) return fail("mcb_debug_forward: buffer too small");
   StepArgs a; memset(&a, 0, sizeof a);
   a.mode = MODE_FORWARD; a.debug = b->debug; a.debug_env = env;
   if (launch(b, a, (cudaStream_t)stream)) return -1;
-  int total = DEBUG_DOUBLES;
-  if (cap < total) return fail("mcb_debug_forward: buffer too small");
   CK(cudaStreamSynchronize((cudaStream_t)stream));
-  CK(cudaMemcpy(h_out, b->debug, total * sizeof(double), cudaMemcpyDeviceToHost));
-  return total;
+  CK(cudaMemcpy(h_out, b->debug, DEBUG_DOUBLES * sizeof(double), cudaMemcpyDeviceToHost));
+  return DEBUG_DOUBLES;
 }
 
 int32_t mcb_get_state(mcb_batch* b, double* qpos, double* qvel, double* ctrl, double* warm, double* goal, int32_t* elapsed, double* qprev, double* mocap, void* stream) {
@@ -3237,23 +3228,7 @@ int32_t mcb_step_host(mcb_batch* b, const float* h_actions, double* h_obs, doubl
   size_t N = (size_t)b->n_envs, od = (size_t)b->obs_dim;
   const size_t ad = (size_t)mcb_batch_action_dim(b);
   size_t rbytes = b->cfg.reward_type == 0 ? sizeof(float) : sizeof(double);
-  if (!b->d_actions) {
-    CK(cudaMalloc(&b->d_actions, N * ad * sizeof(float)));
-    CK(cudaMalloc(&b->d_obs, N * od * sizeof(double)));
-    CK(cudaMalloc(&b->d_fobs, N * od * sizeof(double)));
-    CK(cudaMemset(b->d_fobs, 0, N * od * sizeof(double)));      // rows of envs that did not auto-reset are never written
-    CK(cudaMallocHost(&b->h_fobs, N * od * sizeof(double)));
-    CK(cudaMalloc(&b->d_ag, N * 3 * sizeof(double)));
-    CK(cudaMalloc(&b->d_dg, N * 3 * sizeof(double)));
-    CK(cudaMalloc(&b->d_reward, N * sizeof(double)));
-    CK(cudaMalloc(&b->d_flags, N * 3));
-    CK(cudaMallocHost(&b->h_actions, N * ad * sizeof(float)));
-    CK(cudaMallocHost(&b->h_obs, N * od * sizeof(double)));
-    CK(cudaMallocHost(&b->h_ag, N * 3 * sizeof(double)));
-    CK(cudaMallocHost(&b->h_dg, N * 3 * sizeof(double)));
-    CK(cudaMallocHost(&b->h_reward, N * sizeof(double)));
-    CK(cudaMallocHost(&b->h_flags, N * 3));
-  }
+  if (!b->d_actions) CK(alloc_staging(b));
   // Caller buffers that are already page-locked (cudaHostAlloc / cudaHostRegister / torch pin_memory) are used directly;
   // pageable ones go through the batch's pinned staging buffers and cost one extra host memcpy each way.
   auto pinned = [](const void* p) {

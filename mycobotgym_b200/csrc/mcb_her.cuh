@@ -171,16 +171,19 @@ int32_t mcb_her_create(int32_t n_envs, int32_t buffer_steps, int32_t obs_dim, in
   h->n_sampled_goal = n_sampled_goal; h->thr = distance_threshold; h->seed = seed;
   cudaGetDevice(&h->device);
   const size_t R = (size_t)n_envs * buffer_steps;
-#define HALLOC(p, n) do { cudaError_t e_ = cudaMalloc(&(p), (n)); if (e_ != cudaSuccess) { mcb_her_destroy(h); return fail("mcb_her_create: cudaMalloc", e_); } } while (0)
+  // partial allocations are released on failure (mcb_her_destroy frees whatever is non-null)
+#define HCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { mcb_her_destroy(h); return fail("mcb_her_create: " #call, e_); } } while (0)
+#define HALLOC(p, n) HCK(cudaMalloc(&(p), (n)))
   HALLOC(h->obs, R * obs_dim * sizeof(double)); HALLOC(h->next_obs, R * obs_dim * sizeof(double));
   HALLOC(h->ag, R * 3 * sizeof(double)); HALLOC(h->next_ag, R * 3 * sizeof(double)); HALLOC(h->dg, R * 3 * sizeof(double));
   HALLOC(h->actions, R * action_dim * sizeof(float)); HALLOC(h->rewards, R * sizeof(float));
   HALLOC(h->dones, R); HALLOC(h->timeouts, R);
   HALLOC(h->ep_start, R * sizeof(int)); HALLOC(h->ep_length, R * sizeof(int)); HALLOC(h->cur_start, n_envs * sizeof(int));
   HALLOC(h->n_valid, sizeof(long long));
+  HCK(cudaMemset(h->ep_start, 0, R * sizeof(int))); HCK(cudaMemset(h->ep_length, 0, R * sizeof(int)));
+  HCK(cudaMemset(h->cur_start, 0, n_envs * sizeof(int))); HCK(cudaMemset(h->n_valid, 0, sizeof(long long)));
 #undef HALLOC
-  CK(cudaMemset(h->ep_start, 0, R * sizeof(int))); CK(cudaMemset(h->ep_length, 0, R * sizeof(int)));
-  CK(cudaMemset(h->cur_start, 0, n_envs * sizeof(int))); CK(cudaMemset(h->n_valid, 0, sizeof(long long)));
+#undef HCK
   *out = h;
   return 0;
 }
