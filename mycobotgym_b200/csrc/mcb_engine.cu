@@ -117,6 +117,11 @@ static_assert(sizeof(DevModel) % sizeof(double) == 0, "DevModel must be a whole 
 
 enum { MODE_STEP = 0, MODE_FORWARD = 1, MODE_RESET = 2 };
 
+// offsets of the arrays in an env's resident state record (MCB_STATE_STRIDE doubles; the record ends in padding)
+enum { ST_QPOS = 0, ST_QVEL = ST_QPOS + NQ, ST_CTRL = ST_QVEL + NV, ST_WARM = ST_CTRL + NU, ST_GOAL = ST_WARM + NV, ST_QPREV = ST_GOAL + 3,
+       ST_MOCAP = ST_QPREV + 6, ST_END = ST_MOCAP + 7 };
+static_assert(ST_END <= MCB_STATE_STRIDE, "the state record must fit its stride");
+
 struct StepArgs {
   const DevModel* m;
   int n_envs, mode;
@@ -124,14 +129,14 @@ struct StepArgs {
   int mid_threshold;         // the middle tier only runs when more envs than this left the common layout (else: straight to the last tier)
   mcb_task_cfg cfg;
   const unsigned long long* env_seed;  // [N] Philox key per env (mcb_seed)
-  double* state;             // [N, 72]
+  double* state;             // [N, MCB_STATE_STRIDE]
   int* elapsed;              // [N]
   double* ep_return;         // [N]
   unsigned long long* rng_ctr;  // [N]
   double* stats;             // [8]
   int* redo_count;           // [2] envs that overflowed tier 0 / tier 1 in this step
   int* redo_list;            // [2][N]
-  const float* actions;      // [N, 7]
+  const float* actions;      // [N, action_dim]
   const uint8_t* mask;       // reset
   const double* inj_xy;      // reset
   const double* inj_goal;    // reset
@@ -144,13 +149,15 @@ struct StepArgs {
 };
 
 // ------------------------------------------------------------------------------------------------
-// per-env shared-memory working set, one layout per capacity tier (see the table in DESIGN.md section 3).
-// TIER 0: the common case (16 envs per CTA); TIER 1: contact-rich envs -- a grasp, pushing, the gripper resting on the
-// table (10 envs per CTA); TIER 2: the last resort, one env per CTA, rows beyond its capacity are dropped and counted.
-// last tier: both finger pads flat on the table (8 box-box points each) plus the cube's four corners are 20 condim-4 contacts
-// = 120 rows on top of the 13 equality rows and the joint limits -- the IK / mocap soak runs dropped rows at 16 contacts / 128 rows
-#define NROW_LAST 176
-#define MAXC_LAST 24
+// Per-env shared-memory working set, one layout per capacity tier (DESIGN.md section 3): warps (= envs) per CTA, constraint rows,
+// doubles of the blocked Jacobian pool, contacts.  TIER 0: the common case; TIER 1: contact-rich envs -- a grasp, pushing, the
+// gripper resting on the table; TIER 2: the last resort (one CTA per SM), rows beyond its capacity are dropped and counted: both
+// finger pads flat on the table (8 box-box points each) plus the cube's four corners are 20 condim-4 contacts = 120 rows on top
+// of the 13 equality rows and the joint limits -- the IK / mocap soak runs dropped rows at 16 contacts / 128 rows.
+template <int TIER> struct Tier;
+template <> struct Tier<0> { enum { WARPS = 16, NROW = 48, POOL = 460, MAXC = 8 }; };
+template <> struct Tier<1> { enum { WARPS = 10, NROW = 88, POOL = 1230, MAXC = 14 }; };
+template <> struct Tier<2> { enum { WARPS = 5, NROW = 176, POOL = 2432, MAXC = 24 }; };
 template <int TIER>
 struct EnvS {
   // MCB_CANARY build (tests/test_gpu_canary.py; compute-sanitizer is closed on the GPU pool): guard words between the arrays of
@@ -163,9 +170,8 @@ struct EnvS {
 #define GUARD(name)
 #define MCB_NGUARD 0
 #endif
-  enum { NROW = TIER == 0 ? 48 : TIER == 1 ? 88 : NROW_LAST, POOL = (TIER == 0 ? 460 : TIER == 1 ? 1230 : 2432) - (MCB_NGUARD ? (TIER == 0 ? 10 : 2 * MCB_NGUARD) : 0),   // (tier 0: the row arrays must stay the union's largest member)
-         MAXC = TIER == 0 ? 8 : TIER == 1 ? 14 : MAXC_LAST,
-         IS_BIG = TIER == 2, TIER_ID = TIER };
+  enum { NROW = Tier<TIER>::NROW, POOL = Tier<TIER>::POOL - (MCB_NGUARD ? (TIER == 0 ? 10 : 2 * MCB_NGUARD) : 0),   // (tier 0: the row arrays must stay the union's largest member)
+         MAXC = Tier<TIER>::MAXC, IS_BIG = TIER == 2, TIER_ID = TIER };
   double qpos[20], qvel[NV], ctrl[8], warm[NV], goal[4];
   GUARD(g0)
   double xpos[NB * 3], xmat[NB * 9], cdof[NV * 6], refcube[4];
@@ -197,7 +203,8 @@ struct EnvS {
 };
 static_assert(offsetof(EnvS<0>, H) % 16 == 0 && offsetof(EnvS<1>, H) % 16 == 0 && offsetof(EnvS<2>, H) % 16 == 0, "factor storage must be 16-byte aligned (128-bit loads)");
 static_assert(sizeof(EnvS<0>) % 16 == 0 && sizeof(EnvS<1>) % 16 == 0 && sizeof(EnvS<2>) % 16 == 0, "per-env records must keep 16-byte alignment");
-static_assert(MODEL_BYTES + 16 * sizeof(EnvS<0>) <= 232448 && MODEL_BYTES + 10 * sizeof(EnvS<1>) <= 232448, "a CTA must fit the 227 KB of shared memory an SM offers");
+template <int TIER> constexpr size_t cta_bytes() { return MODEL_BYTES + Tier<TIER>::WARPS * sizeof(EnvS<TIER>); }
+static_assert(cta_bytes<0>() <= 232448 && cta_bytes<1>() <= 232448 && cta_bytes<2>() <= 232448, "a CTA must fit the 227 KB of shared memory an SM offers");
 
 
 // ------------------------------------------------------------------------------------------------
@@ -279,8 +286,6 @@ __device__ __forceinline__ void quat2mat(double* m, const double* q) {
   m[5] = 2 * (q23 - q01); m[6] = 2 * (q13 - q02); m[7] = 2 * (q23 + q01);
 }
 
-
-#define WPB_SMALL 16      // warps (= envs) per CTA of the common-layout launch
 
 // kinematic tree of the reduced model (flatten.reduce_model): arm 0..5, gripper sub-chains 6->7, 8->9, 10, 11 under body 5,
 // free cube 12.  fk() is written against this table; mcb_model_create checks the descriptor against it.
@@ -1987,8 +1992,9 @@ struct Newton {
 // the workload's code footprint (profiles/README.md, r01o / r01q): pick-and-place and reach are fastest free-running
 // (2.47 M vs 2.27 M env-steps/s in full lockstep), push and the mocap variant are 2x / 1.4x faster in full lockstep
 // (free-running they stall on instruction fetch, `no_instructions` 38 %).  mcb_autotune() measures and picks per batch.
+#define LOCKSTEP_CTA 16   // lw >= this: the whole CTA is one group, whatever its tier's warp count (__syncthreads)
 __device__ __forceinline__ void group_sync(int lw) {
-  if (lw >= WPB_SMALL) __syncthreads();
+  if (lw >= LOCKSTEP_CTA) __syncthreads();
   else asm volatile("bar.sync %0, %1;" ::"r"(1 + (int)(threadIdx.x >> 5) / lw), "r"(32 * lw) : "memory");
 }
 template <class S>
@@ -2046,9 +2052,9 @@ __device__ __noinline__ void euler(S& s, const DevModel* __restrict__ m, int lan
   __syncwarp();
 }
 
-// start-of-episode constants: the model's qpos0 set, or keyframe 0 for fetch envs (mycobot.py:451-472)
-__device__ __forceinline__ const double* init_qpos_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_qpos : MDL.d.init_qpos; }
-__device__ __forceinline__ const double* init_ctrl_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_ctrl : MDL.d.init_ctrl; }
+// start-of-episode constants: the model's qpos0 set, or keyframe 0 for fetch envs (mycobot.py:451-472); init_state_kernel reads the model in global memory
+__device__ __forceinline__ const double* init_qpos_of(const DevModel& md, int fetch) { return fetch ? md.d.key_qpos : md.d.init_qpos; }
+__device__ __forceinline__ const double* init_ctrl_of(const DevModel& md, int fetch) { return fetch ? md.d.key_ctrl : md.d.init_ctrl; }
 __device__ __forceinline__ const double* grip0_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_initial_gripper_xpos : MDL.d.initial_gripper_xpos; }
 __device__ __forceinline__ double hoff_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_height_offset : MDL.d.height_offset; }
 
@@ -2077,6 +2083,15 @@ __device__ void sample_goal(const DevModel* __restrict__ m, const mcb_task_cfg& 
   }
 }
 
+// EEF site position from the frames in shared memory (its orientation is the body's: the site has no own rotation)
+template <class S>
+__device__ __forceinline__ void eef_pos_of(const S& s, double* pos) {
+  const int eb = MDL.d.eef_body;
+  const double* R = s.xmat + eb * 9;
+  const double* ep = MDL.d.eef_pos;
+#pragma unroll
+  for (int r = 0; r < 3; r++) pos[r] = s.xpos[eb * 3 + r] + R[3 * r] * ep[0] + R[3 * r + 1] * ep[1] + R[3 * r + 2] * ep[2];
+}
 // observation (mycobot.py:342-388): written from the frames currently in shared memory (stale by one
 // substep after a step, fresh after forward), qpos / qvel current.  Lanes 0-2: gripper position / velocity,
 // 3-5: cube position / velocities, 6: cube Euler angles, 7: gripper joint state; staged through s.grad..s.Mv.
@@ -2088,11 +2103,8 @@ __device__ __noinline__ void write_obs(S& s, const DevModel* __restrict__ m, con
   __syncwarp();
   if (lane < 3) {
     const int r = lane, eb = MDL.d.eef_body;
-    const double* R = s.xmat + eb * 9;
-    const double* ep = MDL.d.eef_pos;
     double grip[3];
-#pragma unroll
-    for (int q = 0; q < 3; q++) grip[q] = s.xpos[eb * 3 + q] + R[3 * q] * ep[0] + R[3 * q + 1] * ep[1] + R[3 * q + 2] * ep[2];
+    eef_pos_of(s, grip);
     double off[3] = {grip[0] - MDL.d.ref_robot[0], grip[1] - MDL.d.ref_robot[1], grip[2] - MDL.d.ref_robot[2]};
     double gv = 0;
     unsigned mask = MDL.d.ancmask[eb];
@@ -2161,13 +2173,13 @@ template <class S>
 __device__ void load_state(S& s, const double* __restrict__ st, int lane) {
   for (int w = lane; w < MCB_STATE_STRIDE; w += 32) {
     double v = st[w];
-    if (w < 19) s.qpos[w] = v;
-    else if (w < 37) s.qvel[w - 19] = v;
-    else if (w < 44) s.ctrl[w - 37] = v;
-    else if (w < 62) s.warm[w - 44] = v;
-    else if (w < 65) s.goal[w - 62] = v;
-    else if (w < 71) s.qprev[w - 65] = v;
-    else if (w < 78) s.mocap[w - 71] = v;
+    if (w < ST_QVEL) s.qpos[w - ST_QPOS] = v;
+    else if (w < ST_CTRL) s.qvel[w - ST_QVEL] = v;
+    else if (w < ST_WARM) s.ctrl[w - ST_CTRL] = v;
+    else if (w < ST_GOAL) s.warm[w - ST_WARM] = v;
+    else if (w < ST_QPREV) s.goal[w - ST_GOAL] = v;
+    else if (w < ST_MOCAP) s.qprev[w - ST_QPREV] = v;
+    else if (w < ST_END) s.mocap[w - ST_MOCAP] = v;
   }
   __syncwarp();
 }
@@ -2175,13 +2187,13 @@ template <class S>
 __device__ void store_state(const S& s, double* __restrict__ st, int lane) {
   for (int w = lane; w < MCB_STATE_STRIDE; w += 32) {
     double v = 0;
-    if (w < 19) v = s.qpos[w];
-    else if (w < 37) v = s.qvel[w - 19];
-    else if (w < 44) v = s.ctrl[w - 37];
-    else if (w < 62) v = s.warm[w - 44];
-    else if (w < 65) v = s.goal[w - 62];
-    else if (w < 71) v = s.qprev[w - 65];
-    else if (w < 78) v = s.mocap[w - 71];
+    if (w < ST_QVEL) v = s.qpos[w - ST_QPOS];
+    else if (w < ST_CTRL) v = s.qvel[w - ST_QVEL];
+    else if (w < ST_WARM) v = s.ctrl[w - ST_CTRL];
+    else if (w < ST_GOAL) v = s.warm[w - ST_WARM];
+    else if (w < ST_QPREV) v = s.goal[w - ST_GOAL];
+    else if (w < ST_MOCAP) v = s.qprev[w - ST_QPREV];
+    else if (w < ST_END) v = s.mocap[w - ST_MOCAP];
     st[w] = v;
   }
 }
@@ -2213,15 +2225,6 @@ __device__ __forceinline__ void mulquat_d(double* r, const double* a, const doub
   double t2 = a[0] * b[2] - a[1] * b[3] + a[2] * b[0] + a[3] * b[1];
   double t3 = a[0] * b[3] + a[1] * b[2] - a[2] * b[1] + a[3] * b[0];
   r[0] = t0; r[1] = t1; r[2] = t2; r[3] = t3;
-}
-// EEF site position from the frames in shared memory (its orientation is the body's: the site has no own rotation)
-template <class S>
-__device__ __forceinline__ void eef_pos_of(const S& s, double* pos) {
-  const int eb = MDL.d.eef_body;
-  const double* R = s.xmat + eb * 9;
-  const double* ep = MDL.d.eef_pos;
-#pragma unroll
-  for (int r = 0; r < 3; r++) pos[r] = s.xpos[eb * 3 + r] + R[3 * r] * ep[0] + R[3 * r + 1] * ep[1] + R[3 * r + 2] * ep[2];
 }
 // target pose of this env-step from the (stale) site pose and the clipped float32 action
 template <class S>
@@ -2300,9 +2303,9 @@ __device__ void ik_update_ctrl(S& s, int lane, double grip_ctrl) {
 // reset_model (mycobot.py:207-236): init state, forward, cube xy, forward, goal.  false: layout overflow.
 template <class S>
 __device__ __noinline__ bool reset_env(S& s, const StepArgs& a, const DevModel* __restrict__ m, int lane, int env, int nba, int nva, unsigned long long& ctr) {
-  for (int w = lane; w < NQ; w += 32) s.qpos[w] = init_qpos_of(a.cfg)[w];
+  for (int w = lane; w < NQ; w += 32) s.qpos[w] = init_qpos_of(MDL, a.cfg.fetch_env)[w];
   if (lane < NV) s.qvel[lane] = 0;
-  if (lane < NU) s.ctrl[lane] = init_ctrl_of(a.cfg)[lane];
+  if (lane < NU) s.ctrl[lane] = init_ctrl_of(MDL, a.cfg.fetch_env)[lane];
   __syncwarp();
   if (!forward(s, m, lane, nba, nva, false)) return false;
   const double gx0 = grip0_of(a.cfg)[0], gy0 = grip0_of(a.cfg)[1];
@@ -2385,17 +2388,15 @@ __device__ void debug_dump(S& s, const StepArgs& a, int lane, int nva) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// The env kernel: one warp per env.  TIER 0 is the first launch over all envs, WPB_SMALL warps per CTA; envs whose
+// The env kernel: one warp per env, Tier<TIER>::WARPS warps per CTA.  TIER 0 is the first launch over all envs; envs whose
 // constraint set overflows a tier's layout leave every output untouched and enqueue themselves on that tier's redo list,
-// which the next tier's launch serves (grid-stride over the list; tier 1: WPB_MID warps per CTA, tier 2: one).
-#define WPB_MID 10
-#define WPB_BIG 5       // last tier: five envs per CTA (one CTA per SM), so that they can run in lockstep like the other tiers
+// which the next tier's launch serves (grid-stride over the list; several envs per CTA in the last tier too, for lockstep).
 template <int TIER>
-__global__ void __launch_bounds__(TIER == 0 ? 32 * WPB_SMALL : TIER == 1 ? 32 * WPB_MID : 32 * WPB_BIG, 1) mcb_env_kernel(const __grid_constant__ StepArgs a) {   // (reset_env takes the arguments by reference: without __grid_constant__ the whole struct is copied to the stack)
+__global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(const __grid_constant__ StepArgs a) {   // (reset_env takes the arguments by reference: without __grid_constant__ the whole struct is copied to the stack)
   typedef EnvS<TIER> S;
   constexpr bool BIG = TIER == 2;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int wpb = TIER == 0 ? WPB_SMALL : TIER == 1 ? WPB_MID : WPB_BIG;
+  const int wpb = Tier<TIER>::WARPS;
   S& s = *reinterpret_cast<S*>(smem_raw + MODEL_BYTES + (size_t)wid * sizeof(S));
   const DevModel* __restrict__ m = a.m;
   {  // stage the model (global -> shared), once per CTA
@@ -2416,8 +2417,8 @@ __global__ void __launch_bounds__(TIER == 0 ? 32 * WPB_SMALL : TIER == 1 ? 32 * 
   if (TIER > 0 && nwork == 0) return;
   if (TIER == 1 && nwork <= a.mid_threshold) {
     // A tier pass costs the latency of one whole env-step of a single warp whatever the list length, and envs that do not
-    // fit here either pay it twice.  A short list is therefore handed to the last tier as it is: its one-warp CTAs take
-    // it in a single wave.  The middle tier pays off when many envs are in contact at once (a batch of grasps).
+    // fit here either pay it twice.  A short list is therefore handed to the last tier as it is: its CTAs take it in one or
+    // two waves.  The middle tier pays off when many envs are in contact at once (a batch of grasps).
     int* next = a.redo_list + (size_t)a.n_envs;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nwork; i += gridDim.x * blockDim.x) next[i] = work_list[i];
     if (blockIdx.x == 0 && threadIdx.x == 0) a.redo_count[1] = nwork;
@@ -2425,7 +2426,7 @@ __global__ void __launch_bounds__(TIER == 0 ? 32 * WPB_SMALL : TIER == 1 ? 32 * 
   }
   // the upper tiers always run their CTA in lockstep (their envs are the divergent, contact-rich ones: free-running they stall on
   // instruction fetch -- held grasp 59 -> 20 ms/step); the batch's grouping (mcb_autotune) only concerns the common-layout kernel
-  const int lockstep = TIER == 0 ? (a.lockstep_warps > 1 ? a.lockstep_warps : 0) : WPB_SMALL;
+  const int lockstep = TIER == 0 ? (a.lockstep_warps > 1 ? a.lockstep_warps : 0) : LOCKSTEP_CTA;
 
   // Tier 0: CTA b takes the 16 consecutive envs [16 b, 16 b + 16).  Tier 1: the list is dealt round-robin over the CTAs
   // (item = slot * gridDim.x + b), so a list shorter than one full wave spreads over all SMs with few warps each instead of
@@ -2578,8 +2579,8 @@ __global__ void __launch_bounds__(TIER == 0 ? 32 * WPB_SMALL : TIER == 1 ? 32 * 
         double rew = cfg.reward_type == 0 ? -(double)(dist > cfg.distance_threshold) : -dist;
         if (bad) { dist = 1e10; rew = cfg.reward_type == 0 ? -1.0 : 0.0; }
         if (cfg.reward_type == 2 && !bad) {
-          // stage_rewards (mycobot.py:402-448): reach / grasp / lift from the sites and the contact list of the last
-          // forward pass; write_obs left grip_pos in o[0..2]; object_pos = the cube body's origin (site object0 sits on it)
+          // OracleEnv.stage_rewards (oracle/oracle.py; mycobot.py:402-448): reach / grasp / lift from the sites and the contact list of
+          // the last forward pass; write_obs left grip_pos in o[0..2]; object_pos = the cube body's origin (site object0 sits on it)
           const double* o = s.grad;
           const double* op = s.xpos + CUBE * 3;
           double gx = o[0] - op[0], gy = o[1] - op[1], gz = o[2] - op[2];
@@ -2665,15 +2666,15 @@ __global__ void init_state_kernel(double* state, int* elapsed, double* ep_return
   if (i >= n) return;
   double* st = state + (size_t)i * MCB_STATE_STRIDE;
   for (int k = 0; k < MCB_STATE_STRIDE; k++) st[k] = 0;
-  const double* q0 = fetch ? m->d.key_qpos : m->d.init_qpos;
-  const double* c0 = fetch ? m->d.key_ctrl : m->d.init_ctrl;
-  for (int k = 0; k < NQ; k++) st[k] = q0[k];
-  for (int k = 0; k < NU; k++) st[37 + k] = c0[k];
-  for (int k = 0; k < 6; k++) st[65 + k] = q0[k];
+  const double* q0 = init_qpos_of(*m, fetch);
+  const double* c0 = init_ctrl_of(*m, fetch);
+  for (int k = 0; k < NQ; k++) st[ST_QPOS + k] = q0[k];
+  for (int k = 0; k < NU; k++) st[ST_CTRL + k] = c0[k];
+  for (int k = 0; k < 6; k++) st[ST_QPREV + k] = q0[k];
   const double* mp = fetch ? m->d.key_mocap_pos : m->d.mocap_pos0;
   const double* mq = fetch ? m->d.key_mocap_quat : m->d.mocap_quat0;
-  for (int k = 0; k < 3; k++) st[71 + k] = mp[k];
-  for (int k = 0; k < 4; k++) st[74 + k] = mq[k];
+  for (int k = 0; k < 3; k++) st[ST_MOCAP + k] = mp[k];
+  for (int k = 0; k < 4; k++) st[ST_MOCAP + 3 + k] = mq[k];
   elapsed[i] = 0; ep_return[i] = 0; ctr[i] = 0; env_seed[i] = seed;
 }
 
@@ -2683,23 +2684,23 @@ __global__ void state_io_kernel(double* state, int* elapsed, int n, double* qpos
   if (i >= n) return;
   double* st = state + (size_t)i * MCB_STATE_STRIDE;
   if (write) {
-    if (qpos) { for (int k = 0; k < NQ; k++) st[k] = qpos[(size_t)i * NQ + k]; for (int k = 0; k < 6; k++) st[65 + k] = st[k]; }
-    if (qvel) for (int k = 0; k < NV; k++) st[19 + k] = qvel[(size_t)i * NV + k];
-    if (ctrl) for (int k = 0; k < NU; k++) st[37 + k] = ctrl[(size_t)i * NU + k];
-    if (warm) for (int k = 0; k < NV; k++) st[44 + k] = warm[(size_t)i * NV + k];
-    if (goal) for (int k = 0; k < 3; k++) st[62 + k] = goal[(size_t)i * 3 + k];
+    if (qpos) { for (int k = 0; k < NQ; k++) st[ST_QPOS + k] = qpos[(size_t)i * NQ + k]; for (int k = 0; k < 6; k++) st[ST_QPREV + k] = st[ST_QPOS + k]; }
+    if (qvel) for (int k = 0; k < NV; k++) st[ST_QVEL + k] = qvel[(size_t)i * NV + k];
+    if (ctrl) for (int k = 0; k < NU; k++) st[ST_CTRL + k] = ctrl[(size_t)i * NU + k];
+    if (warm) for (int k = 0; k < NV; k++) st[ST_WARM + k] = warm[(size_t)i * NV + k];
+    if (goal) for (int k = 0; k < 3; k++) st[ST_GOAL + k] = goal[(size_t)i * 3 + k];
     if (el) elapsed[i] = el[i];
-    if (qprev) for (int k = 0; k < 6; k++) st[65 + k] = qprev[(size_t)i * 6 + k];
-    if (mocap) for (int k = 0; k < 7; k++) st[71 + k] = mocap[(size_t)i * 7 + k];
+    if (qprev) for (int k = 0; k < 6; k++) st[ST_QPREV + k] = qprev[(size_t)i * 6 + k];
+    if (mocap) for (int k = 0; k < 7; k++) st[ST_MOCAP + k] = mocap[(size_t)i * 7 + k];
   } else {
-    if (qpos) for (int k = 0; k < NQ; k++) qpos[(size_t)i * NQ + k] = st[k];
-    if (qvel) for (int k = 0; k < NV; k++) qvel[(size_t)i * NV + k] = st[19 + k];
-    if (ctrl) for (int k = 0; k < NU; k++) ctrl[(size_t)i * NU + k] = st[37 + k];
-    if (warm) for (int k = 0; k < NV; k++) warm[(size_t)i * NV + k] = st[44 + k];
-    if (goal) for (int k = 0; k < 3; k++) goal[(size_t)i * 3 + k] = st[62 + k];
+    if (qpos) for (int k = 0; k < NQ; k++) qpos[(size_t)i * NQ + k] = st[ST_QPOS + k];
+    if (qvel) for (int k = 0; k < NV; k++) qvel[(size_t)i * NV + k] = st[ST_QVEL + k];
+    if (ctrl) for (int k = 0; k < NU; k++) ctrl[(size_t)i * NU + k] = st[ST_CTRL + k];
+    if (warm) for (int k = 0; k < NV; k++) warm[(size_t)i * NV + k] = st[ST_WARM + k];
+    if (goal) for (int k = 0; k < 3; k++) goal[(size_t)i * 3 + k] = st[ST_GOAL + k];
     if (el) el[i] = elapsed[i];
-    if (qprev) for (int k = 0; k < 6; k++) qprev[(size_t)i * 6 + k] = st[65 + k];
-    if (mocap) for (int k = 0; k < 7; k++) mocap[(size_t)i * 7 + k] = st[71 + k];
+    if (qprev) for (int k = 0; k < 6; k++) qprev[(size_t)i * 6 + k] = st[ST_QPREV + k];
+    if (mocap) for (int k = 0; k < 7; k++) mocap[(size_t)i * 7 + k] = st[ST_MOCAP + k];
   }
 }
 
@@ -2743,7 +2744,7 @@ __global__ void iota_kernel(int* list, int* count, int n) {
   if (i == 0) *count = n;
 }
 
-#define DEBUG_DOUBLES (4 + NV * NV + 5 * NV + NB * 12 + NROW_LAST * NV + 2 * NROW_LAST + 7 * MAXC_LAST)
+#define DEBUG_DOUBLES (4 + NV * NV + 5 * NV + NB * 12 + Tier<2>::NROW * NV + 2 * Tier<2>::NROW + 7 * Tier<2>::MAXC)
 
 }  // namespace
 
@@ -2812,8 +2813,7 @@ struct mcb_model {
 
 struct mcb_batch {
   mcb_model* model;
-  int n_envs, obs_dim, big_only, mid_only, big_grid, mid_grid;
-  size_t smem_small, smem_mid, smem_big;
+  int n_envs, obs_dim, big_only, mid_only, sm_count;
   int* redo_count; int* redo_list;
   mcb_task_cfg cfg;
   uint64_t seed;
@@ -2827,6 +2827,11 @@ struct mcb_batch {
   float* h_actions; double *h_obs, *h_ag, *h_dg, *h_fobs; void* h_reward; uint8_t* h_flags;
 };
 
+template <int TIER> static cudaError_t set_tier_smem() {
+  cudaError_t e = cudaFuncSetAttribute(mcb_env_kernel<TIER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cta_bytes<TIER>());
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<TIER>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+  return e;
+}
 static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
   a.m = b->model->dev; a.n_envs = b->n_envs; a.cfg = b->cfg; a.env_seed = b->env_seed;
   a.state = b->state; a.elapsed = b->elapsed; a.ep_return = b->ep_return; a.rng_ctr = b->rng_ctr; a.stats = b->stats;
@@ -2835,18 +2840,18 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
 #ifdef MCB_CANARY
   { const char* st_ = getenv("MCB_CANARY_SELFTEST"); a.canary_selftest = (st_ && st_[0] == '1') ? 1 : 0; }
 #endif
-  a.mid_threshold = b->mid_only ? -1 : 2 * b->big_grid;    // up to two waves of the last tier are cheaper than a middle-tier pass (profiles/README.md)
+  a.mid_threshold = b->mid_only ? -1 : 2 * Tier<2>::WARPS * b->sm_count;    // up to two waves of the last tier are cheaper than a middle-tier pass (profiles/README.md)
   CK(cudaMemsetAsync(b->redo_count, 0, 2 * sizeof(int), st));
   if (b->big_only) iota_kernel<<<(b->n_envs + 255) / 256, 256, 0, st>>>(b->redo_list + b->n_envs, b->redo_count + 1, b->n_envs);
   else if (b->mid_only) iota_kernel<<<(b->n_envs + 255) / 256, 256, 0, st>>>(b->redo_list, b->redo_count, b->n_envs);
-  else mcb_env_kernel<0><<<(b->n_envs + WPB_SMALL - 1) / WPB_SMALL, 32 * WPB_SMALL, b->smem_small, st>>>(a);
+  else mcb_env_kernel<0><<<(b->n_envs + Tier<0>::WARPS - 1) / Tier<0>::WARPS, 32 * Tier<0>::WARPS, cta_bytes<0>(), st>>>(a);
   CK(cudaGetLastError());
   b->launches_total += 1 + (b->big_only ? 0 : 1) + 1;      // this one, the middle tier (unless last-tier-only), the last tier
   // envs that overflowed the common layout (grid-stride over the device list; empty in contact-free workloads) ...
-  if (!b->big_only) mcb_env_kernel<1><<<b->mid_only ? (b->n_envs + WPB_MID - 1) / WPB_MID : b->mid_grid, 32 * WPB_MID, b->smem_mid, st>>>(a);
+  if (!b->big_only) mcb_env_kernel<1><<<b->mid_only ? (b->n_envs + Tier<1>::WARPS - 1) / Tier<1>::WARPS : b->sm_count, 32 * Tier<1>::WARPS, cta_bytes<1>(), st>>>(a);
   CK(cudaGetLastError());
   // ... and the few that overflowed the middle one
-  mcb_env_kernel<2><<<b->big_only ? (b->n_envs + WPB_BIG - 1) / WPB_BIG : b->big_grid / WPB_BIG, 32 * WPB_BIG, b->smem_big, st>>>(a);
+  mcb_env_kernel<2><<<b->big_only ? (b->n_envs + Tier<2>::WARPS - 1) / Tier<2>::WARPS : b->sm_count, 32 * Tier<2>::WARPS, cta_bytes<2>(), st>>>(a);
   CK(cudaGetLastError());
   return 0;
 }
@@ -2904,9 +2909,9 @@ extern "C" {
 
 const char* mcb_version(void) {
   static char buf[320];
-  snprintf(buf, sizeof buf, "mycobot_b200 0.5 (sm_100a; shared memory per env: %zu B common layout (16 per CTA), %zu B middle tier (%d per CTA), %zu B last tier (%d per CTA); model %zu B; CTAs %zu / %zu / %zu B)",
-           sizeof(EnvS<0>), sizeof(EnvS<1>), WPB_MID, sizeof(EnvS<2>), WPB_BIG, (size_t)MODEL_BYTES, (size_t)(MODEL_BYTES + sizeof(EnvS<0>) * WPB_SMALL),
-           (size_t)(MODEL_BYTES + sizeof(EnvS<1>) * WPB_MID), (size_t)(MODEL_BYTES + sizeof(EnvS<2>) * WPB_BIG));
+  snprintf(buf, sizeof buf, "mycobot_b200 0.5 (sm_100a; shared memory per env: %zu B common layout (%d per CTA), %zu B middle tier (%d per CTA), %zu B last tier (%d per CTA); model %zu B; CTAs %zu / %zu / %zu B)",
+           sizeof(EnvS<0>), (int)Tier<0>::WARPS, sizeof(EnvS<1>), (int)Tier<1>::WARPS, sizeof(EnvS<2>), (int)Tier<2>::WARPS, (size_t)MODEL_BYTES,
+           cta_bytes<0>(), cta_bytes<1>(), cta_bytes<2>());
   return buf;
 }
 const char* mcb_last_error(void) { return g_err.c_str(); }
@@ -3034,19 +3039,12 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
   if (cfg->nefc_max != 0 && cfg->nefc_max != 48 && cfg->nefc_max != 88 && cfg->nefc_max != 128) { delete b; return fail("mcb_batch_create: nefc_max must be 0 (tiered), 48, 88 (start in the middle tier) or 128 (last tier only)"); }
   b->big_only = cfg->nefc_max == 128;
   b->mid_only = cfg->nefc_max == 88;
-  b->smem_small = MODEL_BYTES + sizeof(EnvS<0>) * WPB_SMALL;
-  b->smem_mid = MODEL_BYTES + sizeof(EnvS<1>) * WPB_MID;
-  b->smem_big = MODEL_BYTES + sizeof(EnvS<2>) * WPB_BIG;
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, m->device) != cudaSuccess) { delete b; return fail("mcb_batch_create: cudaGetDeviceProperties", cudaGetLastError()); }
-  b->big_grid = prop.multiProcessorCount * WPB_BIG;      // envs of one last-tier wave: one five-warp CTA per SM
-  b->mid_grid = prop.multiProcessorCount;
-  cudaError_t e = cudaFuncSetAttribute(mcb_env_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_small);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_mid);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b->smem_big);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<2>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+  b->sm_count = prop.multiProcessorCount;
+  cudaError_t e = set_tier_smem<0>();
+  if (e == cudaSuccess) e = set_tier_smem<1>();
+  if (e == cudaSuccess) e = set_tier_smem<2>();
   if (e != cudaSuccess) { delete b; return fail("cudaFuncSetAttribute(shared memory)", e); }
   size_t N = (size_t)n_envs;
   // partial allocations are released on failure (mcb_batch_destroy frees whatever is non-null)
@@ -3144,7 +3142,7 @@ int32_t mcb_autotune(mcb_batch* b, const float* actions, int32_t steps_per_candi
   // roll ahead (state right after a reset is not representative: nothing moves yet), then snapshot the tuning state
   for (int k = 0; k < 32 && okay; k++) one_step(k);
   TCK(tuning.save(st));
-  const int cand[3] = {WPB_SMALL, 4, 1};
+  const int cand[3] = {LOCKSTEP_CTA, 4, 1};
   for (int c = 0; c < 3 && okay; c++) {
     b->lockstep_warps = cand[c];
     TCK(tuning.restore(st));

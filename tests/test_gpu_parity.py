@@ -389,7 +389,7 @@ def test_state_roundtrip_and_ragged_sizes(flat):
 
 
 def test_tiered_layouts_are_bit_identical(flat):
-    # the same states through (a) the tiered launch (48-row common layout, then 88-row middle tier, then 128-row last tier),
+    # the same states through (a) the tiered launch (48-row common layout, then 88-row middle tier, then 176-row last tier),
     # (b) the middle tier only and (c) the last tier only
     n = 64
     qpos, qvel, ctrl = _states(flat, n, 31)
