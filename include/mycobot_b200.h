@@ -40,6 +40,13 @@ extern "C" {
 #define MCB_OBS_REACH 10
 #define MCB_STATE_STRIDE 80 /* doubles per env in the resident state record: qpos19 qvel18 ctrl7 warm18 goal3 qprev6 mocap7 pad2 */
 
+/* Per-env physics parameters: MCB_NPARAM multipliers of fields of the model in use (nominal value 1.0). */
+#define MCB_NPARAM 14
+#define MCB_P_CUBE_MASS 0    /* mass[12] and the six inertia[12] entries of the cube */
+#define MCB_P_FRICTION 1     /* 1..5: sliding friction geom_friction[g][0] of the MCB_NGEOM primitive geoms, g in mcb_model_desc order */
+#define MCB_P_GAIN 6         /* 6..12: actuator u: act_gain[u], act_bias[u][1] and act_bias[u][2] (the servo's kp and kv); mocap variant: u = 0 only */
+#define MCB_P_ARM_DAMPING 13 /* damping[0..5], in the passive force and in Euler's implicit term */
+
 /* Flattened, reduced model (host memory; copied to the device by mcb_model_create).
  * Replaces the compiled mjModel the reference builds in MujocoEnv.__init__ (mycobot.py:69-75). */
 typedef struct mcb_model_desc {
@@ -204,7 +211,8 @@ int32_t mcb_reset_host(mcb_batch* b, const uint8_t* h_mask, const double* h_obj_
                        double* h_obs, double* h_achieved_goal, double* h_desired_goal, void* stream);
 /* replaces `self._np_random, seed = seeding.np_random(seed)` of MyCobotEnv.reset(seed=) (mycobot.py:509-510) for the
  * device sampler: the masked envs (all if mask == NULL, a device pointer) get Philox key `seed` and draw counter 0, so
- * the goals / cube positions drawn by the following resets are a function of (seed, env index) only. */
+ * the goals / cube positions drawn by the following resets are a function of (seed, env index) only.  Their per-env parameter
+ * draw counters (mcb_batch_set_param_ranges) restart at 0 too. */
 int32_t mcb_seed(mcb_batch* b, uint64_t seed, const uint8_t* mask, void* stream);
 
 /* replaces MyCobotEnv.step, joint (mycobot.py:132-133,190-205) and IK (mycobot.py:134-170, utils.py:499-556) controllers
@@ -239,6 +247,29 @@ int32_t mcb_set_state(mcb_batch* b, const double* qpos, const double* qvel, cons
 int32_t mcb_get_rng_state(mcb_batch* b, uint64_t* env_seed, uint64_t* draw_counter, double* ep_return, void* stream);
 int32_t mcb_set_rng_state(mcb_batch* b, const uint64_t* env_seed, const uint64_t* draw_counter, const double* ep_return, void* stream);
 
+/* Per-env physics parameters (domain randomisation).  Each env carries MCB_NPARAM multipliers (slots: MCB_P_*).  A contact pair's
+ * friction mixes the scaled sides like mj_contactParam (the larger wins) and everything derived from it follows: the pyramid rows,
+ * their first-row diagApprox and their regulariser scale.  Torsional / rolling friction and the constants the model compiler derives
+ * (body_invweight0, dof_invweight0, meaninertia and through them con_diag and the pairs' inverse weights) stay as compiled -- MuJoCo
+ * behaves the same way when model.body_mass is written between steps without mj_setConst.  Not available with mesh_collision.
+ *
+ * mcb_batch_set_param_ranges: HOST arrays of MCB_NPARAM bounds; from the next reset on, every reset of an env (mcb_reset,
+ * mcb_reset_host, the auto-reset and the bad-simulation reset inside mcb_step) draws slot k from U[lo[k], hi[k]] before its first
+ * forward pass, MCB_NPARAM draws per reset whatever the ranges.  The draws come from the env's Philox key (mcb_seed) with a stream tag
+ * and a draw counter of their own: the goal / cube stream is unchanged, and mcb_seed restarts the parameter stream of the envs it
+ * reseeds.  NULL, NULL stops drawing (the current values stay).  Non-finite bounds, bounds <= 0 and lo > hi are rejected and leave
+ * the batch as it was.  The first call turns per-env parameters on (nominal values for every env): it allocates and synchronises
+ * the device, so it is not capturable.  Steps and resets enqueued later use the new ranges; a captured CUDA graph keeps the ranges
+ * it was captured with. */
+int32_t mcb_batch_set_param_ranges(mcb_batch* b, const double* h_lo, const double* h_hi);
+/* device pointers params double[N, MCB_NPARAM] and draw_counter uint64[N], either may be NULL.  A batch without per-env parameters
+ * reports 1.0 and 0. */
+int32_t mcb_get_env_params(mcb_batch* b, double* params, uint64_t* draw_counter, void* stream);
+/* fixed per-env values (evaluation, system identification, checkpoints): device pointers as above, either may be NULL.  Turns
+ * per-env parameters on if needed (like mcb_batch_set_param_ranges' first call; drawing stays off until ranges are set).  Like
+ * mcb_set_state it does not validate device data. */
+int32_t mcb_set_env_params(mcb_batch* b, const double* params, const uint64_t* draw_counter, void* stream);
+
 /* replaces mujoco.mj_forward on every env (mycobot.py:213,229,306); refreshes qacc_warmstart; optional obs out */
 int32_t mcb_forward(mcb_batch* b, double* obs, double* achieved_goal, double* desired_goal, void* stream);
 
@@ -261,7 +292,7 @@ int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out
 
 /* Picks the lockstep grouping of the step kernel for this batch (cfg.lockstep_warps == 0): rolls the batch 32 steps
  * ahead (the state right after a reset is not representative), times `steps_per_candidate` (0 -> 4) steps per candidate
- * from that state, keeps the fastest and restores state, episode clocks, RNG streams and statistics exactly.  `actions`
+ * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters and statistics exactly.  `actions`
  * (device float32 [N, action_dim]) are applied at every tuning step; NULL -> uniform random actions from a private
  * Philox stream.  Synchronises the stream and allocates scratch: it is never called implicitly -- mcb_step only enqueues
  * its three kernels on the caller's stream (no hidden sync, CUDA-graph capturable).  Returns the chosen grouping. */

@@ -16,8 +16,9 @@ ROOT = os.path.dirname(PKG_DIR)
 LIB_PATH = os.environ.get("MCB_LIB") or os.path.join(PKG_DIR, "libmycobot_b200.so")   # MCB_LIB: load another build of the library, e.g. the canary build
 CANARY_PATH = os.path.join(PKG_DIR, "libmycobot_b200_canary.so")   # -DMCB_CANARY: guard words in the shared-memory records (tests only)
 SRC = os.path.join(PKG_DIR, "csrc", "mcb_engine.cu")
+SRC_PRM = os.path.join(PKG_DIR, "csrc", "mcb_engine_prm.cu")   # the step kernels of batches with per-env parameters (own module)
 HDR = os.path.join(ROOT, "include", "mycobot_b200.h")
-DEPS = (SRC, HDR, os.path.join(PKG_DIR, "csrc", "mcb_her.cuh"))
+DEPS = (SRC, SRC_PRM, HDR, os.path.join(PKG_DIR, "csrc", "mcb_her.cuh"))
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "--fmad=true",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -29,6 +30,7 @@ EXPORTS = [
     "mcb_compute_reward", "mcb_stats", "mcb_debug_forward", "mcb_last_step_launches", "mcb_fp64_peak_probe",
     "mcb_autotune", "mcb_batch_lockstep_warps", "mcb_last_fallback_envs", "mcb_her_create", "mcb_her_destroy", "mcb_her_add", "mcb_her_size", "mcb_her_episode_table",
     "mcb_her_sample", "mcb_reset_host", "mcb_seed", "mcb_get_rng_state", "mcb_set_rng_state", "mcb_last_fallback_list", "mcb_total_launches", "mcb_hull_desc_size", "mcb_model_set_hulls",
+    "mcb_batch_set_param_ranges", "mcb_get_env_params", "mcb_set_env_params",
 ]
 
 
@@ -45,7 +47,7 @@ def build(force=False, verbose=False):
     if not force and not needs_build():
         return LIB_PATH
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + ["-I", os.path.join(ROOT, "include"), "-o", LIB_PATH, SRC]
+    cmd = [nvcc] + NVCC_FLAGS + ["-I", os.path.join(ROOT, "include"), "-o", LIB_PATH, SRC, SRC_PRM]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     subprocess.check_call(cmd)
@@ -58,7 +60,7 @@ def build_canary(force=False):
     if not force and not needs_build(CANARY_PATH):
         return CANARY_PATH
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    subprocess.check_call([nvcc] + NVCC_FLAGS + ["-DMCB_CANARY", "-I", os.path.join(ROOT, "include"), "-o", CANARY_PATH, SRC])
+    subprocess.check_call([nvcc] + NVCC_FLAGS + ["-DMCB_CANARY", "-I", os.path.join(ROOT, "include"), "-o", CANARY_PATH, SRC, SRC_PRM])
     return CANARY_PATH
 
 
@@ -104,6 +106,9 @@ def load():
     L.mcb_get_rng_state.argtypes = [vp] + [vp] * 4
     L.mcb_set_rng_state.argtypes = [vp] + [vp] * 4
     L.mcb_last_fallback_list.argtypes = [vp, vp, i32, vp]
+    L.mcb_batch_set_param_ranges.argtypes = [vp, vp, vp]
+    L.mcb_get_env_params.argtypes = [vp, vp, vp, vp]
+    L.mcb_set_env_params.argtypes = [vp, vp, vp, vp]
     L.mcb_total_launches.argtypes = [vp]
     L.mcb_total_launches.restype = i64
     L.mcb_her_create.argtypes = [i32, i32, i32, i32, i32, i32, dbl, u64, C.POINTER(vp)]

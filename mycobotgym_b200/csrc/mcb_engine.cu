@@ -40,6 +40,7 @@
 #include <stdio.h>
 #include <string.h>
 #include <math.h>
+#include <cmath>
 #include <string>
 #include <vector>
 #include <stdlib.h>
@@ -146,6 +147,11 @@ struct StepArgs {
   double* debug;             // optional debug dump of env debug_env
   int debug_env;
   int canary_selftest;       // MCB_CANARY build + MCB_CANARY_SELFTEST=1 in the environment: every env writes one double past cpos[] on purpose
+  // per-env physics parameters (read by the PRM kernels only)
+  double* params;            // [N, MCB_NPARAM] multipliers
+  unsigned long long* param_ctr;  // [N] parameter draw counters
+  int draw_params;           // resets draw new parameters from U[param_lo, param_hi]
+  double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -159,7 +165,7 @@ template <> struct Tier<0> { enum { WARPS = 16, NROW = 48, POOL = 460, MAXC = 8 
 template <> struct Tier<1> { enum { WARPS = 10, NROW = 88, POOL = 1230, MAXC = 14 }; };
 template <> struct Tier<2> { enum { WARPS = 5, NROW = 176, POOL = 2432, MAXC = 24 }; };
 template <int TIER>
-struct EnvS {
+struct EnvCore {
   // MCB_CANARY build (tests/test_gpu_canary.py; compute-sanitizer is closed on the GPU pool): guard words between the arrays of
   // the record, set when an env is loaded and checked when it is stored; a hit is counted in stats[5] and reported.  The pools
   // shrink by the guards' size, which only moves the point where an env changes tier (results do not depend on the tier).
@@ -201,10 +207,28 @@ struct EnvS {
   int nR, nC, nF, nU, nefc, ncon, overflow, iters;
   int mesh, pad_[3];   // mesh: the batch collides the convex hulls too (cfg.mesh_collision)
 };
-static_assert(offsetof(EnvS<0>, H) % 16 == 0 && offsetof(EnvS<1>, H) % 16 == 0 && offsetof(EnvS<2>, H) % 16 == 0, "factor storage must be 16-byte aligned (128-bit loads)");
+// PRM: the batch has per-env physics parameters (mcb_batch_set_param_ranges / mcb_set_env_params).  Batches without them run the
+// PRM = false kernels, whose record is EnvCore itself and whose code does not contain the parameter reads.  With them, the env's
+// MCB_NPARAM multipliers and its parameter draw counter are staged after the working set; `prm_drawn` marks a record a reset redrew
+// (only such records are written back).
+template <int TIER, bool PRM = false>
+struct EnvS : EnvCore<TIER> { enum { HAS_PRM = 0 }; };
+template <int TIER>
+struct EnvS<TIER, true> : EnvCore<TIER> {
+  enum { HAS_PRM = 1 };
+  GUARD(gp)
+  double prm[MCB_NPARAM];
+  unsigned long long prm_ctr;
+  int prm_drawn, prm_pad_;
+};
+static_assert(offsetof(EnvCore<0>, H) % 16 == 0 && offsetof(EnvCore<1>, H) % 16 == 0 && offsetof(EnvCore<2>, H) % 16 == 0, "factor storage must be 16-byte aligned (128-bit loads)");
 static_assert(sizeof(EnvS<0>) % 16 == 0 && sizeof(EnvS<1>) % 16 == 0 && sizeof(EnvS<2>) % 16 == 0, "per-env records must keep 16-byte alignment");
-template <int TIER> constexpr size_t cta_bytes() { return MODEL_BYTES + Tier<TIER>::WARPS * sizeof(EnvS<TIER>); }
+static_assert(sizeof(EnvS<0, true>) % 16 == 0 && sizeof(EnvS<1, true>) % 16 == 0 && sizeof(EnvS<2, true>) % 16 == 0, "per-env records must keep 16-byte alignment");
+static_assert(sizeof(EnvS<0, true>) - sizeof(EnvS<0>) == 128 + 8 * (MCB_NGUARD ? 2 : 0), "the parameter record is 14 doubles, a counter and a flag");
+template <int TIER, bool PRM = false> constexpr size_t cta_bytes() { return MODEL_BYTES + Tier<TIER>::WARPS * sizeof(EnvS<TIER, PRM>); }
 static_assert(cta_bytes<0>() <= 232448 && cta_bytes<1>() <= 232448 && cta_bytes<2>() <= 232448, "a CTA must fit the 227 KB of shared memory an SM offers");
+static_assert(cta_bytes<0, true>() <= 232448 && cta_bytes<1, true>() <= 232448 && cta_bytes<2, true>() <= 232448,
+              "a CTA with per-env parameters must fit the 227 KB of shared memory an SM offers");
 
 
 // ------------------------------------------------------------------------------------------------
@@ -413,6 +437,13 @@ __device__ void cinert_cdof(S& s, const DevModel* __restrict__ m, int lane, int 
       for (int r = 0; r < 3; r++) off[r] = com[r] - MDL.d.ref_robot[r];
     }
     const double* I = MDL.d.inertia[b];  // xx yy zz xy xz yz
+    double Ip[6];
+    if constexpr (S::HAS_PRM) {          // the cube's inertia and mass scale together (MCB_P_CUBE_MASS)
+      const double p = b == CUBE ? s.prm[MCB_P_CUBE_MASS] : 1.0;
+#pragma unroll
+      for (int k = 0; k < 6; k++) Ip[k] = I[k] * p;
+      I = Ip;
+    }
     double A[9];                         // A = R * Ib
 #pragma unroll
     for (int r = 0; r < 3; r++) {
@@ -421,6 +452,7 @@ __device__ void cinert_cdof(S& s, const DevModel* __restrict__ m, int lane, int 
       A[3 * r + 2] = R[3 * r] * I[4] + R[3 * r + 1] * I[5] + R[3 * r + 2] * I[2];
     }
     double mass = MDL.d.mass[b];
+    if constexpr (S::HAS_PRM) { if (b == CUBE) mass = mass * s.prm[MCB_P_CUBE_MASS]; }
     double* ci = s.cinert + b * 10;
     ci[0] = A[0] * R[0] + A[1] * R[1] + A[2] * R[2] + mass * (off[1] * off[1] + off[2] * off[2]);
     ci[1] = A[3] * R[3] + A[4] * R[4] + A[5] * R[5] + mass * (off[0] * off[0] + off[2] * off[2]);
@@ -1397,6 +1429,13 @@ __device__ __forceinline__ void row_dot2(S& s, int r, const double* v, const dou
 
 // make_rows(): equality (7 robot rows), pyramidal contact rows by block type, joint-limit unit rows; then R, D
 // and the reference acceleration of every row.  Returns false if the layout's capacity is exceeded.
+// Sliding friction of a primitive pair under the env's multipliers, mixed like pair_param() (the larger side wins).  Only batches
+// without hull collisions have per-env parameters, so every contact's pair is a primitive one.
+template <class S>
+__device__ __forceinline__ double env_mu(const S& s, const PairParam& pp) {
+  return fmax(MDL.d.geom_friction[pp.g1][0] * s.prm[MCB_P_FRICTION + pp.g1], MDL.d.geom_friction[pp.g2][0] * s.prm[MCB_P_FRICTION + pp.g2]);
+}
+
 template <class S>
 __device__ bool make_rows(S& s, const DevModel* __restrict__ m, int lane, int nva) {
   // connect anchors (lanes 0..3: constraint e = lane>>1, side = lane&1)
@@ -1549,6 +1588,7 @@ __device__ bool make_rows(S& s, const DevModel* __restrict__ m, int lane, int nv
       else if (pt == 1) { p = row_c(s, r0) + (j - NH); st = SC; }
       else { p = row_f(s, r0) + j; st = SF; }
       double mu = pp.friction[0];
+      if constexpr (S::HAS_PRM) mu = env_mu(s, pp);
       p[0] = Jn + mu * Jt1;
       p[st] = Jn + (-mu) * Jt1;
       p[2 * st] = Jn + mu * Jt2;
@@ -1592,10 +1632,12 @@ __device__ bool make_rows(S& s, const DevModel* __restrict__ m, int lane, int nv
     } else {
       const PairParam& pp = PP(s.cpair[idx]);
       double mu = pp.friction[0];
+      if constexpr (S::HAS_PRM) mu = env_mu(s, pp);
       pos = s.cdist[idx];
       KB = pp.KB; solimp = pp.solimp;
       diag = pp.tran + mu * mu * pp.tran;     // the pyramid's first-row diagApprox; all rows share R = 2 mu^2 R_first
       pyr2 = pp.pyr2;
+      if constexpr (S::HAS_PRM) { const double pyr = mu / sqrt(MDL.d.impratio); pyr2 = 2 * pyr * pyr; }   // pair_param() with multiplicity 1
     }
     double imp = impedance(solimp, ipos >= 0 ? ipos : pos);
     double R = fmax(MINVAL, (1 - imp) * diag * fast_rcp(imp));      // imp in [MINIMP, MAXIMP]
@@ -1671,6 +1713,12 @@ __device__ void velocity_rne(S& s, const DevModel* __restrict__ m, int lane, int
   __syncwarp();
 }
 
+// joint damping of dof j under the env's multipliers: the arm's six hinges scale with MCB_P_ARM_DAMPING
+template <class S>
+__device__ __forceinline__ double env_damping(const S& s, int j) {
+  return j < 6 ? MDL.d.damping[j] * s.prm[MCB_P_ARM_DAMPING] : MDL.d.damping[j];
+}
+
 // actuation_smooth(): affine PD "general" actuators with ctrl and force clamps, passive damping; qfrc_smooth.
 template <class S>
 __device__ void actuation_smooth(S& s, const DevModel* __restrict__ m, int lane, int nva) {
@@ -1682,6 +1730,11 @@ __device__ void actuation_smooth(S& s, const DevModel* __restrict__ m, int lane,
     double ctrl = s.ctrl[lane];
     if (MDL.d.act_ctrllimited[lane]) ctrl = fmax(MDL.d.act_ctrlrange[lane][0], fmin(MDL.d.act_ctrlrange[lane][1], ctrl));
     const double* bp = MDL.d.act_bias[lane];
+    if constexpr (S::HAS_PRM) {         // one multiplier for the servo's kp (gain, bias[1]) and kv (bias[2]); same expression as below
+      const double p = s.prm[MCB_P_GAIN + lane];
+      const double g = MDL.d.act_gain[lane] * p, b1 = bp[1] * p, b2 = bp[2] * p;
+      force = g * ctrl + bp[0] + b1 * len + b2 * vel;
+    } else
     force = MDL.d.act_gain[lane] * ctrl + bp[0] + bp[1] * len + bp[2] * vel;
     if (MDL.d.act_forcelimited[lane]) force = fmax(MDL.d.act_forcerange[lane][0], fmin(MDL.d.act_forcerange[lane][1], force));
   }
@@ -1691,6 +1744,9 @@ __device__ void actuation_smooth(S& s, const DevModel* __restrict__ m, int lane,
     double fa = __shfl_sync(FULLMASK, force, a);
     if (lane < NV) qa += MDL.d.act_moment[a][lane] * fa;
   }
+  if constexpr (S::HAS_PRM) {
+    if (lane < nva) s.qfrc_smooth[lane] = -env_damping(s, lane) * s.qvel[lane] - s.qfrc_bias[lane] + qa;
+  } else
   if (lane < nva) s.qfrc_smooth[lane] = -MDL.d.damping[lane] * s.qvel[lane] - s.qfrc_bias[lane] + qa;
   __syncwarp();
 }
@@ -2027,7 +2083,10 @@ __device__ __noinline__ void euler(S& s, const DevModel* __restrict__ m, int lan
   const double h = MDL.d.timestep;
   if (lane < NV) s.search[lane] = lane < nva ? s.qfrc_smooth[lane] + s.qfrc_con[lane] : 0.0;   // search / Mv are free outside the solver
   __syncwarp();
-  double qacc = factor_solve_M<true>(s.M, s.H, s.search, s.Mv, lane < nva ? h * MDL.d.damping[lane] : 0.0, lane, nva);
+  double qacc;
+  if constexpr (S::HAS_PRM) qacc = factor_solve_M<true>(s.M, s.H, s.search, s.Mv, lane < nva ? h * env_damping(s, lane) : 0.0, lane, nva);
+  else
+  qacc = factor_solve_M<true>(s.M, s.H, s.search, s.Mv, lane < nva ? h * MDL.d.damping[lane] : 0.0, lane, nva);
   if (lane < nva) s.qvel[lane] += h * qacc;
   __syncwarp();
   if (lane < NH) s.qpos[lane] += h * s.qvel[lane];
@@ -2058,15 +2117,19 @@ __device__ __forceinline__ const double* init_ctrl_of(const DevModel& md, int fe
 __device__ __forceinline__ const double* grip0_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_initial_gripper_xpos : MDL.d.initial_gripper_xpos; }
 __device__ __forceinline__ double hoff_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_height_offset : MDL.d.height_offset; }
 
-// Philox4x32-10 counter RNG: one stream per env, key = seed, counter = (env, draw index)
+// Philox4x32-10 counter RNG: one stream per env, key = seed, counter = (env, draw index, stream tag).  Tag GOAL_TAG: goals and cube
+// positions; PARAM_TAG: per-env physics parameters, with a draw counter of their own, so the goal stream is the same with or without them.
+#define GOAL_TAG 0x6d79636fu
+#define PARAM_TAG 0x7072616du
 __device__ __forceinline__ void philox_round(uint32_t* c, uint32_t k0, uint32_t k1) {
   uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
   uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
   uint32_t n0 = hi1 ^ c[1] ^ k0, n1 = lo1, n2 = hi0 ^ c[3] ^ k1, n3 = lo0;
   c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
 }
+template <uint32_t TAG = GOAL_TAG>
 __device__ double philox_uniform(uint64_t seed, uint32_t env, unsigned long long& ctr) {
-  uint32_t c[4] = {(uint32_t)ctr, (uint32_t)(ctr >> 32), env, 0x6d79636fu};
+  uint32_t c[4] = {(uint32_t)ctr, (uint32_t)(ctr >> 32), env, TAG};
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
   for (int i = 0; i < 10; i++) { philox_round(c, k0, k1); k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
   ctr++;
@@ -2303,6 +2366,20 @@ __device__ void ik_update_ctrl(S& s, int lane, double grip_ctrl) {
 // reset_model (mycobot.py:207-236): init state, forward, cube xy, forward, goal.  false: layout overflow.
 template <class S>
 __device__ __noinline__ bool reset_env(S& s, const StepArgs& a, const DevModel* __restrict__ m, int lane, int env, int nba, int nva, unsigned long long& ctr) {
+  if constexpr (S::HAS_PRM) {
+    // per-env parameters: slot k ~ U[lo_k, hi_k] from draw prm_ctr + k of the parameter stream, before the first forward pass
+    if (a.draw_params) {
+      if (lane < MCB_NPARAM) {
+        unsigned long long c = s.prm_ctr + (unsigned long long)lane;
+        const double u = philox_uniform<PARAM_TAG>(a.env_seed[env], env, c);
+        const double lo = a.param_lo[lane], hi = a.param_hi[lane];
+        s.prm[lane] = fmin(hi, lo + (hi - lo) * u);
+      }
+      __syncwarp();
+      if (lane == 0) { s.prm_ctr += MCB_NPARAM; s.prm_drawn = 1; }
+      __syncwarp();
+    }
+  }
   for (int w = lane; w < NQ; w += 32) s.qpos[w] = init_qpos_of(MDL, a.cfg.fetch_env)[w];
   if (lane < NV) s.qvel[lane] = 0;
   if (lane < NU) s.ctrl[lane] = init_ctrl_of(MDL, a.cfg.fetch_env)[lane];
@@ -2391,9 +2468,10 @@ __device__ void debug_dump(S& s, const StepArgs& a, int lane, int nva) {
 // The env kernel: one warp per env, Tier<TIER>::WARPS warps per CTA.  TIER 0 is the first launch over all envs; envs whose
 // constraint set overflows a tier's layout leave every output untouched and enqueue themselves on that tier's redo list,
 // which the next tier's launch serves (grid-stride over the list; several envs per CTA in the last tier too, for lockstep).
-template <int TIER>
+// PRM: the batch has per-env physics parameters (EnvS<TIER, true>); launch() picks the instantiation from the batch.
+template <int TIER, bool PRM>
 __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(const __grid_constant__ StepArgs a) {   // (reset_env takes the arguments by reference: without __grid_constant__ the whole struct is copied to the stack)
-  typedef EnvS<TIER> S;
+  typedef EnvS<TIER, PRM> S;
   constexpr bool BIG = TIER == 2;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int wpb = Tier<TIER>::WARPS;
@@ -2447,10 +2525,16 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
     if (lane == 0) { s.mesh = a.cfg.mesh_collision; s.overflow = 0; s.iters = 0; s.nefc = 0; s.ncon = 0; s.nR = MDL.d.has_weld ? 13 : 7; s.nC = s.nF = s.nU = 0; s.refcube[0] = s.refcube[1] = s.refcube[2] = 0; }
 #ifdef MCB_CANARY
     if (lane < 2) { const double c = __longlong_as_double(0x7ff8c0decafe0000ll + lane); s.g0[lane] = c; s.g1[lane] = c; s.g2[lane] = c; s.g3[lane] = c; s.g4[lane] = c; s.g5[lane] = c; s.g6[lane] = c; s.g7[lane] = c; }
+    if constexpr (PRM) { if (lane < 2) s.gp[lane] = __longlong_as_double(0x7ff8c0decafe0000ll + lane); }
 #endif
     __syncwarp();
     unsigned long long ctr = 0;
     if (valid) { load_state(s, a.state + (size_t)env * MCB_STATE_STRIDE, lane); ctr = a.rng_ctr[env]; }
+    if constexpr (PRM) {
+      if (valid && lane < MCB_NPARAM) s.prm[lane] = a.params[(size_t)env * MCB_NPARAM + lane];
+      if (lane == 0) { s.prm_ctr = valid ? a.param_ctr[env] : 0; s.prm_drawn = 0; }
+      __syncwarp();
+    }
     double achieved[3];
     int substeps = 0;
     bool ok = valid;
@@ -2629,6 +2713,9 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
       const double* g[8] = {s.g0, s.g1, s.g2, s.g3, s.g4, s.g5, s.g6, s.g7};
       for (int k = 0; k < 8; k++)
         if (__double_as_longlong(g[k][lane]) != c) { atomicAdd(a.stats + 5, 1.0e6); printf("MCB_CANARY: guard %d of env %d (tier %d) was overwritten\n", k, env, TIER); }
+      if constexpr (PRM) {
+        if (__double_as_longlong(s.gp[lane]) != c) { atomicAdd(a.stats + 5, 1.0e6); printf("MCB_CANARY: guard %d of env %d (tier %d) was overwritten\n", 8, env, TIER); }
+      }
     }
     __syncwarp();
 #endif
@@ -2639,6 +2726,12 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         if (TIER < 2 && lane == 0) { int k = atomicAdd(a.redo_count + TIER, 1); a.redo_list[(size_t)TIER * a.n_envs + k] = env; }
       } else {
         store_state(s, a.state + (size_t)env * MCB_STATE_STRIDE, lane);
+        if constexpr (PRM) {
+          if (s.prm_drawn) {
+            if (lane < MCB_NPARAM) a.params[(size_t)env * MCB_NPARAM + lane] = s.prm[lane];
+            if (lane == 0) a.param_ctr[env] = s.prm_ctr;
+          }
+        }
         if (lane == 0) {
           a.rng_ctr[env] = ctr;
           if (a.mode == MODE_STEP) atomicAdd(a.stats + 4, 1.0);
@@ -2726,9 +2819,20 @@ __global__ void random_actions_kernel(float* act, int n, uint64_t seed, unsigned
 }
 
 // mcb_seed(): MyCobotEnv.reset(seed=) reseeds the env's generator (mycobot.py:509-510) -> new Philox key, draw counter 0
-__global__ void seed_kernel(unsigned long long* env_seed, unsigned long long* ctr, const uint8_t* mask, unsigned long long seed, int n) {
+// (pctr: the parameter draw counters of a batch with per-env parameters, or null)
+__global__ void seed_kernel(unsigned long long* env_seed, unsigned long long* ctr, unsigned long long* pctr, const uint8_t* mask, unsigned long long seed, int n) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n && (!mask || mask[i])) { env_seed[i] = seed; ctr[i] = 0; }
+  if (i < n && (!mask || mask[i])) { env_seed[i] = seed; ctr[i] = 0; if (pctr) pctr[i] = 0; }
+}
+// per-env parameters [N, MCB_NPARAM] and draw counters [N]: mode 0 batch -> caller (the nominal 1.0 and 0 when the batch has none,
+// params == null), 1 caller -> batch, 2 nominal values into the batch; any caller pointer may be null
+__global__ void params_io_kernel(double* params, unsigned long long* ctr, double* u_params, unsigned long long* u_ctr, int n, int mode) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const size_t o = (size_t)i * MCB_NPARAM;
+  if (mode == 2) { for (int k = 0; k < MCB_NPARAM; k++) params[o + k] = 1.0; ctr[i] = 0; }
+  else if (mode == 1) { if (u_params) for (int k = 0; k < MCB_NPARAM; k++) params[o + k] = u_params[o + k]; if (u_ctr) ctr[i] = u_ctr[i]; }
+  else { if (u_params) for (int k = 0; k < MCB_NPARAM; k++) u_params[o + k] = params ? params[o + k] : 1.0; if (u_ctr) u_ctr[i] = ctr ? ctr[i] : 0; }
 }
 // the part of a checkpoint mcb_get_state / mcb_set_state do not carry: RNG streams and running episode returns
 __global__ void rng_io_kernel(unsigned long long* env_seed, unsigned long long* ctr, double* ep_return, unsigned long long* u_seed, unsigned long long* u_ctr,
@@ -2822,16 +2926,53 @@ struct mcb_batch {
   int last_launches;
   long long launches_total;   // kernels this library launched on behalf of the batch (counted at the launch sites)
   int lockstep_warps, tuned;
+  // per-env physics parameters: null until mcb_batch_set_param_ranges / mcb_set_env_params turn them on
+  double* params; unsigned long long* param_ctr;
+  int draw_params;
+  double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
   // staging for the host-buffer entry point
   float* d_actions; double *d_obs, *d_ag, *d_dg, *d_fobs; void* d_reward; uint8_t* d_flags;
   float* h_actions; double *h_obs, *h_ag, *h_dg, *h_fobs; void* h_reward; uint8_t* h_flags;
 };
 
-template <int TIER> static cudaError_t set_tier_smem() {
-  cudaError_t e = cudaFuncSetAttribute(mcb_env_kernel<TIER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cta_bytes<TIER>());
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<TIER>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+template <int TIER, bool PRM = false> static cudaError_t set_tier_smem() {
+  cudaError_t e = cudaFuncSetAttribute(mcb_env_kernel<TIER, PRM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cta_bytes<TIER, PRM>());
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mcb_env_kernel<TIER, PRM>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
   return e;
 }
+template <bool PRM>
+static cudaError_t launch_tiers(mcb_batch* b, const StepArgs& a, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(b->redo_count, 0, 2 * sizeof(int), st);
+  if (e != cudaSuccess) return e;
+  if (b->big_only) iota_kernel<<<(b->n_envs + 255) / 256, 256, 0, st>>>(b->redo_list + b->n_envs, b->redo_count + 1, b->n_envs);
+  else if (b->mid_only) iota_kernel<<<(b->n_envs + 255) / 256, 256, 0, st>>>(b->redo_list, b->redo_count, b->n_envs);
+  else mcb_env_kernel<0, PRM><<<(b->n_envs + Tier<0>::WARPS - 1) / Tier<0>::WARPS, 32 * Tier<0>::WARPS, cta_bytes<0, PRM>(), st>>>(a);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  b->launches_total += 1 + (b->big_only ? 0 : 1) + 1;      // this one, the middle tier (unless last-tier-only), the last tier
+  // envs that overflowed the common layout (grid-stride over the device list; empty in contact-free workloads) ...
+  if (!b->big_only) mcb_env_kernel<1, PRM><<<b->mid_only ? (b->n_envs + Tier<1>::WARPS - 1) / Tier<1>::WARPS : b->sm_count, 32 * Tier<1>::WARPS, cta_bytes<1, PRM>(), st>>>(a);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  // ... and the few that overflowed the middle one
+  mcb_env_kernel<2, PRM><<<b->big_only ? (b->n_envs + Tier<2>::WARPS - 1) / Tier<2>::WARPS : b->sm_count, 32 * Tier<2>::WARPS, cta_bytes<2, PRM>(), st>>>(a);
+  return cudaGetLastError();
+}
+
+// The PRM = true kernels are compiled in a translation unit of their own, mcb_engine_prm.cu (this file with MCB_PRM_UNIT defined):
+// ptxas allocates registers across the call graph of a module, and the math library's slow paths (sincos argument reduction, pow)
+// are functions every env kernel calls, so further env kernels in this module would change the code of the default ones.  Apart,
+// the default kernels compile exactly as they would without per-env parameters.  These two calls are the units' interface;
+// `args` points to a StepArgs.
+cudaError_t prm_launch_tiers(mcb_batch* b, const void* args, cudaStream_t st);
+cudaError_t prm_set_tier_smem();
+#ifdef MCB_PRM_UNIT
+cudaError_t prm_launch_tiers(mcb_batch* b, const void* args, cudaStream_t st) { return launch_tiers<true>(b, *static_cast<const StepArgs*>(args), st); }
+cudaError_t prm_set_tier_smem() {
+  cudaError_t e = set_tier_smem<0, true>();
+  if (e == cudaSuccess) e = set_tier_smem<1, true>();
+  if (e == cudaSuccess) e = set_tier_smem<2, true>();
+  return e;
+}
+#else
 static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
   a.m = b->model->dev; a.n_envs = b->n_envs; a.cfg = b->cfg; a.env_seed = b->env_seed;
   a.state = b->state; a.elapsed = b->elapsed; a.ep_return = b->ep_return; a.rng_ctr = b->rng_ctr; a.stats = b->stats;
@@ -2841,18 +2982,34 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
   { const char* st_ = getenv("MCB_CANARY_SELFTEST"); a.canary_selftest = (st_ && st_[0] == '1') ? 1 : 0; }
 #endif
   a.mid_threshold = b->mid_only ? -1 : 2 * Tier<2>::WARPS * b->sm_count;    // up to two waves of the last tier are cheaper than a middle-tier pass (profiles/README.md)
-  CK(cudaMemsetAsync(b->redo_count, 0, 2 * sizeof(int), st));
-  if (b->big_only) iota_kernel<<<(b->n_envs + 255) / 256, 256, 0, st>>>(b->redo_list + b->n_envs, b->redo_count + 1, b->n_envs);
-  else if (b->mid_only) iota_kernel<<<(b->n_envs + 255) / 256, 256, 0, st>>>(b->redo_list, b->redo_count, b->n_envs);
-  else mcb_env_kernel<0><<<(b->n_envs + Tier<0>::WARPS - 1) / Tier<0>::WARPS, 32 * Tier<0>::WARPS, cta_bytes<0>(), st>>>(a);
-  CK(cudaGetLastError());
-  b->launches_total += 1 + (b->big_only ? 0 : 1) + 1;      // this one, the middle tier (unless last-tier-only), the last tier
-  // envs that overflowed the common layout (grid-stride over the device list; empty in contact-free workloads) ...
-  if (!b->big_only) mcb_env_kernel<1><<<b->mid_only ? (b->n_envs + Tier<1>::WARPS - 1) / Tier<1>::WARPS : b->sm_count, 32 * Tier<1>::WARPS, cta_bytes<1>(), st>>>(a);
-  CK(cudaGetLastError());
-  // ... and the few that overflowed the middle one
-  mcb_env_kernel<2><<<b->big_only ? (b->n_envs + Tier<2>::WARPS - 1) / Tier<2>::WARPS : b->sm_count, 32 * Tier<2>::WARPS, cta_bytes<2>(), st>>>(a);
-  CK(cudaGetLastError());
+  cudaError_t e;
+  if (!b->params) e = launch_tiers<false>(b, a, st);
+  else {
+    a.params = b->params; a.param_ctr = b->param_ctr; a.draw_params = b->draw_params;
+    memcpy(a.param_lo, b->param_lo, sizeof a.param_lo); memcpy(a.param_hi, b->param_hi, sizeof a.param_hi);
+    e = prm_launch_tiers(b, &a, st);
+  }
+  if (e != cudaSuccess) return fail("launching the step kernels", e);
+  return 0;
+}
+
+// Turns per-env parameters on: allocates them, sets every env to the nominal values (1.0, draw counter 0) and prepares the PRM
+// kernels.  Synchronises the device.  A failure leaves the batch without per-env parameters.
+static int enable_params(mcb_batch* b, const char* who) {
+  if (b->params) return 0;
+  if (b->cfg.mesh_collision) { g_err = who; g_err += ": per-env parameters are not supported with mesh_collision (hull pairs keep the model's friction)"; return -1; }
+  DevGuard guard(b->model->device);
+  if (!guard.ok) return fail("enable per-env parameters: cannot select the batch's device", cudaGetLastError());
+  const size_t N = (size_t)b->n_envs;
+  double* p = nullptr; unsigned long long* c = nullptr;
+  cudaError_t e = prm_set_tier_smem();
+  if (e == cudaSuccess) e = cudaMalloc(&p, N * MCB_NPARAM * sizeof(double));
+  if (e == cudaSuccess) e = cudaMalloc(&c, N * sizeof(unsigned long long));
+  if (e == cudaSuccess) { params_io_kernel<<<(b->n_envs + 127) / 128, 128>>>(p, c, nullptr, nullptr, b->n_envs, 2); e = cudaGetLastError(); }
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) { cudaFree(p); cudaFree(c); return fail("enable per-env parameters", e); }
+  b->launches_total++;
+  b->params = p; b->param_ctr = c;
   return 0;
 }
 
@@ -2881,11 +3038,12 @@ static cudaError_t alloc_staging(mcb_batch* b) {
   return e;
 }
 
-// A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics.
-// The buffers are allocated by the first save() and freed with the snapshot.
+// A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics,
+// and the per-env parameters with their draw counters (auto-resets redraw them).  The buffers are allocated by the first save()
+// and freed with the snapshot.
 struct Snapshot {
   const mcb_batch* b;
-  void* copy[5] = {};
+  void* copy[7] = {};
   explicit Snapshot(const mcb_batch* batch) : b(batch) {}
   ~Snapshot() { for (void* p : copy) cudaFree(p); }
   cudaError_t save(cudaStream_t st) { return transfer(true, st); }
@@ -2894,10 +3052,12 @@ struct Snapshot {
  private:
   cudaError_t transfer(bool save, cudaStream_t st) {
     const size_t N = (size_t)b->n_envs;
-    void* live[5] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats};
-    const size_t bytes[5] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double)};
+    void* live[7] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr};
+    const size_t bytes[7] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
+                             N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long)};
     cudaError_t e = cudaSuccess;
-    for (int k = 0; k < 5 && e == cudaSuccess; k++) {
+    for (int k = 0; k < 7 && e == cudaSuccess; k++) {
+      if (!live[k]) continue;      // a batch without per-env parameters
       if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes[k]);
       if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live[k], save ? live[k] : copy[k], bytes[k], cudaMemcpyDeviceToDevice, st);
     }
@@ -3074,6 +3234,7 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
 int32_t mcb_batch_destroy(mcb_batch* b) {
   if (!b) return 0;
   cudaFree(b->state); cudaFree(b->elapsed); cudaFree(b->ep_return); cudaFree(b->rng_ctr); cudaFree(b->env_seed); cudaFree(b->stats); cudaFree(b->debug); cudaFree(b->redo_count); cudaFree(b->redo_list);
+  cudaFree(b->params); cudaFree(b->param_ctr);
   free_staging(b);
   delete b;
   return 0;
@@ -3285,7 +3446,7 @@ int32_t mcb_reset_host(mcb_batch* b, const uint8_t* h_mask, const double* h_obj_
 
 int32_t mcb_seed(mcb_batch* b, uint64_t seed, const uint8_t* mask, void* stream) {
   if (!b) return fail("mcb_seed: null batch");
-  seed_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, mask, (unsigned long long)seed, b->n_envs);
+  seed_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->param_ctr, mask, (unsigned long long)seed, b->n_envs);
   CK(cudaGetLastError());
   b->launches_total++;
   if (!mask) b->seed = seed;
@@ -3304,6 +3465,36 @@ int32_t mcb_set_rng_state(mcb_batch* b, const uint64_t* env_seed, const uint64_t
   if (!b) return fail("mcb_set_rng_state: null batch");
   rng_io_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->ep_return, (unsigned long long*)env_seed,
                                                                         (unsigned long long*)draw_counter, (double*)ep_return, b->n_envs, 1);
+  CK(cudaGetLastError());
+  b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_batch_set_param_ranges(mcb_batch* b, const double* h_lo, const double* h_hi) {
+  if (!b) return fail("mcb_batch_set_param_ranges: null batch");
+  if (!h_lo != !h_hi) return fail("mcb_batch_set_param_ranges: pass both bounds, or neither to stop drawing");
+  if (!h_lo) { b->draw_params = 0; return 0; }
+  for (int k = 0; k < MCB_NPARAM; k++)
+    if (!(std::isfinite(h_lo[k]) && std::isfinite(h_hi[k]) && h_lo[k] > 0 && h_lo[k] <= h_hi[k]))
+      return fail("mcb_batch_set_param_ranges: every range must be finite with 0 < lo <= hi");
+  if (enable_params(b, "mcb_batch_set_param_ranges")) return -1;
+  memcpy(b->param_lo, h_lo, sizeof b->param_lo); memcpy(b->param_hi, h_hi, sizeof b->param_hi);
+  b->draw_params = 1;
+  return 0;
+}
+
+int32_t mcb_get_env_params(mcb_batch* b, double* params, uint64_t* draw_counter, void* stream) {
+  if (!b) return fail("mcb_get_env_params: null batch");
+  params_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->params, b->param_ctr, params, (unsigned long long*)draw_counter, b->n_envs, 0);
+  CK(cudaGetLastError());
+  b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_set_env_params(mcb_batch* b, const double* params, const uint64_t* draw_counter, void* stream) {
+  if (!b) return fail("mcb_set_env_params: null batch");
+  if (enable_params(b, "mcb_set_env_params")) return -1;
+  params_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->params, b->param_ctr, (double*)params, (unsigned long long*)draw_counter, b->n_envs, 1);
   CK(cudaGetLastError());
   b->launches_total++;
   return 0;
@@ -3354,3 +3545,4 @@ int32_t mcb_fp64_peak_probe(int32_t device, int32_t iters, double* tflops_out) {
 }  // extern "C"
 
 #include "mcb_her.cuh"
+#endif  // MCB_PRM_UNIT

@@ -18,6 +18,7 @@ from .mjcf import quat2mat, quat_mul
 
 NB, NV, NQ, NU, NHINGE, NGEOM, MAXPAIR = 13, 18, 19, 7, 12, 5, 12
 MAXHULL, MAXHPAIR = 16, 192
+CUBE_BODY = 12
 
 _d = C.c_double
 _i = C.c_int32
@@ -325,6 +326,93 @@ def reduce_model(m) -> ModelDesc:
     _set(d.key_qpos, m["key_qpos"][0])
     _set(d.key_ctrl, padu(m["key_ctrl"][0]))
     return d
+
+
+# Per-env physics parameters (include/mycobot_b200.h, MCB_NPARAM): multipliers of model fields, nominal value 1.0.
+PARAM_NAMES = ("cube_mass", "friction_floor", "friction_table", "friction_finger_r", "friction_finger_l", "friction_cube",
+               "gain_0", "gain_1", "gain_2", "gain_3", "gain_4", "gain_5", "gain_6", "arm_damping")
+NPARAM = len(PARAM_NAMES)
+P_CUBE_MASS, P_FRICTION, P_GAIN, P_ARM_DAMPING = 0, 1, 6, 13
+PARAM_GROUPS = {"friction": PARAM_NAMES[P_FRICTION:P_GAIN], "gain": PARAM_NAMES[P_GAIN:P_ARM_DAMPING]}
+
+
+def param_bounds(param_ranges, mesh_collision=False):
+    """`param_ranges` ({name: (lo, hi)}) -> (lo, hi), two float64 arrays of NPARAM.  Names are PARAM_NAMES or the groups
+    'friction' / 'gain', which give the same range to each of their slots (each slot is still drawn on its own); unlisted slots
+    get (1, 1).  Raises ValueError for unknown names, a slot named twice, bounds that are not finite or <= 0, lo > hi, and for
+    mesh_collision=True (hull pairs keep the model's friction)."""
+    if mesh_collision:
+        raise ValueError("per-env parameters are not supported with mesh_collision=True")
+    lo, hi = np.ones(NPARAM), np.ones(NPARAM)
+    seen = set()
+    for key, rng in dict(param_ranges).items():
+        slots = PARAM_GROUPS.get(key, (key,))
+        for name in slots:
+            if name not in PARAM_NAMES:
+                raise ValueError(f"unknown parameter {key!r}; known: {', '.join(PARAM_NAMES + tuple(PARAM_GROUPS))}")
+            if name in seen:
+                raise ValueError(f"parameter {name!r} is given twice")
+            seen.add(name)
+        try:
+            a, b = (float(v) for v in rng)
+        except (TypeError, ValueError):
+            raise ValueError(f"{key!r}: a range is a pair (lo, hi), got {rng!r}") from None
+        if not (np.isfinite(a) and np.isfinite(b) and a > 0 and b > 0):
+            raise ValueError(f"{key!r}: bounds must be finite and > 0, got ({a}, {b})")
+        if a > b:
+            raise ValueError(f"{key!r}: lo > hi ({a} > {b})")
+        for name in slots:
+            k = PARAM_NAMES.index(name)
+            lo[k], hi[k] = a, b
+    return lo, hi
+
+
+def _check_params(p):
+    p = np.asarray(p, dtype=np.float64)
+    if p.shape != (NPARAM,):
+        raise ValueError(f"expected {NPARAM} multipliers, got shape {p.shape}")
+    return p
+
+
+def apply_params(desc, p):
+    """A copy of the reduced model `desc` with the NPARAM multipliers `p` baked into its fields -- the model a batch without per-env
+    parameters would need to simulate what an env with parameters `p` simulates (the compiled constants stay, as on the device)."""
+    p = _check_params(p)
+    d = ModelDesc()
+    C.memmove(C.byref(d), C.byref(desc), C.sizeof(ModelDesc))
+    c = CUBE_BODY
+    d.mass[c] = d.mass[c] * p[P_CUBE_MASS]
+    for k in range(6):
+        d.inertia[c][k] = d.inertia[c][k] * p[P_CUBE_MASS]
+    for g in range(NGEOM):
+        d.geom_friction[g][0] = d.geom_friction[g][0] * p[P_FRICTION + g]
+    for u in range(int(d.nu)):
+        d.act_gain[u] = d.act_gain[u] * p[P_GAIN + u]
+        d.act_bias[u][1] = d.act_bias[u][1] * p[P_GAIN + u]
+        d.act_bias[u][2] = d.act_bias[u][2] * p[P_GAIN + u]
+    for j in range(6):
+        d.damping[j] = d.damping[j] * p[P_ARM_DAMPING]
+    return d
+
+
+def apply_params_flat(m, p):
+    """The same on the unmerged flat table (the oracle's model): body_mass / body_inertia of object0, geom_friction,
+    actuator_gain, actuator_biasprm and dof_damping.  Returns a copy; `m` is left as it was."""
+    p = _check_params(p)
+    out = type(m)(m)
+    obj = int(m["site_bodyid"][m["site_names"].index("object0")])
+    for key in ("body_mass", "body_inertia", "geom_friction", "actuator_gain", "actuator_biasprm", "dof_damping"):
+        out[key] = np.array(m[key], dtype=np.float64, copy=True)
+    out["body_mass"][obj] = out["body_mass"][obj] * p[P_CUBE_MASS]
+    out["body_inertia"][obj] = out["body_inertia"][obj] * p[P_CUBE_MASS]
+    out["geom_friction"][:, 0] = out["geom_friction"][:, 0] * p[P_FRICTION:P_FRICTION + NGEOM]
+    nu = int(m["nu"])
+    gains = p[P_GAIN:P_GAIN + nu]
+    out["actuator_gain"] = out["actuator_gain"] * gains
+    out["actuator_biasprm"][:, 1] = out["actuator_biasprm"][:, 1] * gains
+    out["actuator_biasprm"][:, 2] = out["actuator_biasprm"][:, 2] * gains
+    out["dof_damping"][:6] = out["dof_damping"][:6] * p[P_ARM_DAMPING]
+    return out
 
 
 def reduce_hulls(m):

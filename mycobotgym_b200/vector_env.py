@@ -169,14 +169,16 @@ class MyCobotVectorEnv:
                  control_steps=5, controller_type="joint", obj_range=0.1, target_in_the_air=True,
                  distance_threshold=0.01, initial_qpos=None, fetch_env=False, reward_type="sparse", frame_skip=20,
                  max_episode_steps=50, device="cuda:0", seed=0, auto_reset=True, goal_source="device", nefc_max=0,
-                 lockstep_warps=0, autotune=True, mesh_collision=False, **kwargs):
+                 lockstep_warps=0, autotune=True, mesh_collision=False, param_ranges=None, **kwargs):
         """Constructor kwargs are the reference's (mycobot.py:30-46).  `obj_range` and `initial_qpos` are accepted and only
         stored, exactly like the reference does (mycobot.py:54,56 assign them; nothing reads them: the cube is placed by
         `generate_random_point_inside_rectangle`, mycobot.py:220-222, and the start pose is qpos0 / keyframe 0).
         `lockstep_warps=0, autotune=True`: the first full `reset()` ends with one explicit `mcb_autotune` call (it
         synchronises and is never hidden inside `step`); `autotune=False` keeps the free-running default.
         `mesh_collision=True`: the convex hulls of the 28 mesh geoms collide too (MuJoCo: mjc_Convex / mjc_PlaneConvex; here one
-        MPR contact per hull pair, DESIGN.md section 4); off, only the plane / box primitives collide."""
+        MPR contact per hull pair, DESIGN.md section 4); off, only the plane / box primitives collide.
+        `param_ranges={name: (lo, hi)}`: per-env physics parameters (domain randomisation), redrawn on the device at every reset of
+        an env (`flatten.PARAM_NAMES`, groups 'friction' and 'gain'; DESIGN.md section 9).  Not available with mesh_collision."""
         if controller_type not in ("joint", "IK", "mocap"):
             raise ValueError(f"unknown controller_type {controller_type!r}")
         if fetch_env and controller_type == "joint":
@@ -188,6 +190,7 @@ class MyCobotVectorEnv:
                              "(the reference would fail on data.mocap_pos / on the missing actuators)")
         if goal_source not in ("device", "reference"):
             raise ValueError("goal_source must be 'device' or 'reference'")
+        bounds = None if param_ranges is None else flatten.param_bounds(param_ranges, mesh_collision)
         if not torch.cuda.is_available():
             raise RuntimeError("MyCobotVectorEnv needs a CUDA device; there is no CPU fallback")
         self.device = torch.device(device)
@@ -219,6 +222,11 @@ class MyCobotVectorEnv:
             h = C.c_void_p()
             _lib.check(self._L.mcb_batch_create(self._model, self.num_envs, C.byref(cfg), int(seed), C.byref(h)))
         self._batch = h
+        if bounds is not None:
+            lo, hi = (np.ascontiguousarray(x, dtype=np.float64) for x in bounds)
+            with torch.cuda.device(dev_index):
+                _lib.check(self._L.mcb_batch_set_param_ranges(h, lo.ctypes.data_as(C.c_void_p), hi.ctypes.data_as(C.c_void_p)))
+        self._has_params = bounds is not None
         self.obs_dim = self._L.mcb_batch_obs_dim(h)
         self.action_dim = self._L.mcb_batch_action_dim(h)          # 7 (joint, IK), 8 (mocap), 4 (fetch variants) (mycobot.py:90-97)
         N, dev = self.num_envs, self.device
@@ -373,6 +381,8 @@ class MyCobotVectorEnv:
                   qprev=torch.empty(N, 6, dtype=torch.float64, device=dev), mocap=torch.empty(N, 7, dtype=torch.float64, device=dev),
                   env_seed=torch.empty(N, dtype=torch.int64, device=dev), rng_counter=torch.empty(N, dtype=torch.int64, device=dev),
                   ep_return=torch.empty(N, dtype=torch.float64, device=dev))
+        if self._has_params:
+            st["params"], st["param_counter"] = self.get_params()
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_get_rng_state(self._batch, _ptr(st["env_seed"]), _ptr(st["rng_counter"]), _ptr(st["ep_return"]), self._stream()))
             _lib.check(self._L.mcb_get_state(self._batch, _ptr(st["qpos"]), _ptr(st["qvel"]), _ptr(st["ctrl"]),
@@ -381,8 +391,9 @@ class MyCobotVectorEnv:
         return st
 
     def set_state(self, qpos=None, qvel=None, ctrl=None, qacc_warmstart=None, goal=None, elapsed=None, qprev=None, mocap=None,
-                  env_seed=None, rng_counter=None, ep_return=None):
-        """Inverse of `get_state` (a full checkpoint: physics state, goals, episode clocks, RNG streams, running returns)."""
+                  env_seed=None, rng_counter=None, ep_return=None, params=None, param_counter=None):
+        """Inverse of `get_state` (a full checkpoint: physics state, goals, episode clocks, RNG streams, running returns, and the
+        per-env parameters of a batch that has them)."""
         def prep(x, shape, dt):
             if x is None:
                 return None
@@ -399,7 +410,40 @@ class MyCobotVectorEnv:
             _lib.check(self._L.mcb_set_state(self._batch, *[_ptr(t) for t in ts], self._stream()))
             if any(t is not None for t in rs):
                 _lib.check(self._L.mcb_set_rng_state(self._batch, *[_ptr(t) for t in rs], self._stream()))
-            torch.cuda.current_stream(self.device).synchronize()
+        if params is not None or param_counter is not None:
+            self.set_params(params, draw_counter=param_counter)
+        torch.cuda.current_stream(self.device).synchronize()
+
+    def get_params(self):
+        """(params float64 [N, NPARAM], draw counters int64 [N]) as device tensors: the per-env multipliers (`flatten.PARAM_NAMES`)
+        in use and how many parameter draws each env has made since it was seeded.  Without per-env parameters: 1.0 and 0."""
+        N, dev = self.num_envs, self.device
+        p = torch.empty(N, flatten.NPARAM, dtype=torch.float64, device=dev)
+        c = torch.empty(N, dtype=torch.int64, device=dev)
+        with torch.cuda.device(self._dev_index):
+            _lib.check(self._L.mcb_get_env_params(self._batch, _ptr(p), _ptr(c), self._stream()))
+        return p, c
+
+    def set_params(self, params, draw_counter=None):
+        """Fixed per-env multipliers [N, NPARAM] (evaluation, system identification); either argument may be None.  Turns per-env
+        parameters on if the batch has none; resets keep redrawing only if `param_ranges` are set."""
+        if self.mesh_collision:
+            raise ValueError("per-env parameters are not supported with mesh_collision=True")
+        N = self.num_envs
+        p = c = None
+        if params is not None:
+            p = torch.as_tensor(np.asarray(params) if not torch.is_tensor(params) else params).to(device=self.device, dtype=torch.float64).contiguous()
+            if tuple(p.shape) != (N, flatten.NPARAM):
+                raise ValueError(f"params must have shape {(N, flatten.NPARAM)}, got {tuple(p.shape)}")
+            if not bool(torch.isfinite(p).all()) or not bool((p > 0).all()):
+                raise ValueError("params must be finite and > 0")
+        if draw_counter is not None:
+            c = torch.as_tensor(np.asarray(draw_counter) if not torch.is_tensor(draw_counter) else draw_counter).to(device=self.device, dtype=torch.int64).contiguous()
+            if tuple(c.shape) != (N,):
+                raise ValueError(f"draw_counter must have shape {(N,)}, got {tuple(c.shape)}")
+        with torch.cuda.device(self._dev_index):
+            _lib.check(self._L.mcb_set_env_params(self._batch, _ptr(p), _ptr(c), self._stream()))
+        self._has_params = True
 
     def autotune(self, actions=None, steps_per_candidate=0):
         """Pick the step kernel's lockstep grouping for this batch (explicit: `step` never tunes; the constructor's
