@@ -212,7 +212,7 @@ int32_t mcb_reset_host(mcb_batch* b, const uint8_t* h_mask, const double* h_obj_
 /* replaces `self._np_random, seed = seeding.np_random(seed)` of MyCobotEnv.reset(seed=) (mycobot.py:509-510) for the
  * device sampler: the masked envs (all if mask == NULL, a device pointer) get Philox key `seed` and draw counter 0, so
  * the goals / cube positions drawn by the following resets are a function of (seed, env index) only.  Their per-env parameter
- * draw counters (mcb_batch_set_param_ranges) restart at 0 too. */
+ * and latency draw counters (mcb_batch_set_param_ranges, mcb_batch_set_latency_range) restart at 0 too. */
 int32_t mcb_seed(mcb_batch* b, uint64_t seed, const uint8_t* mask, void* stream);
 
 /* replaces MyCobotEnv.step, joint (mycobot.py:132-133,190-205) and IK (mycobot.py:134-170, utils.py:499-556) controllers
@@ -270,6 +270,27 @@ int32_t mcb_get_env_params(mcb_batch* b, double* params, uint64_t* draw_counter,
  * mcb_set_state it does not validate device data. */
 int32_t mcb_set_env_params(mcb_batch* b, const double* params, const uint64_t* draw_counter, void* stream);
 
+/* Per-env actuation latency (domain randomisation of the control delay).  Each env carries an integer latency d in substeps,
+ * 0 <= d <= cfg.frame_skip: every command the controller issues (joint ctrl; mocap pose and gripper ctrl, still computed at substep
+ * 0 from the stale frames; each IK block's DLS result) is written before substep d of its block, after the block's last substep
+ * when d == frame_skip (before the block_gripper forward pass), and until then the previous command stays in force.  A reset's
+ * command is its own (init / key ctrl and the persisting mocap pose).  d == 0 gives the results of a batch without latency bit for
+ * bit.  Latency runs in the step kernels of batches with per-env parameters (nominal multipliers if no ranges are set); it is not
+ * available with mesh_collision.
+ *
+ * mcb_batch_set_latency_range: in substeps; from the next reset on, every reset of an env (as for mcb_batch_set_param_ranges)
+ * draws d uniformly from the integers [lo, hi]: lo + min(hi - lo, floor(u * (hi - lo + 1))), one draw of the env's Philox key with
+ * a stream tag and a draw counter of their own (the goal / cube and parameter streams are unchanged; mcb_seed restarts the
+ * counter).  0 <= lo <= hi <= cfg.frame_skip, else rejected and the batch is left as it was; lo = hi = -1 stops drawing (the
+ * current values stay).  The first call turns per-env parameters on (nominal multipliers), like mcb_batch_set_param_ranges: it
+ * allocates, synchronises and cannot be captured. */
+int32_t mcb_batch_set_latency_range(mcb_batch* b, int32_t lo, int32_t hi);
+/* device pointers latency int32[N], draw_counter uint64[N], either may be NULL; a batch without latency reports 0 and 0 */
+int32_t mcb_get_env_latency(mcb_batch* b, int32_t* latency, uint64_t* draw_counter, void* stream);
+/* fixed per-env latencies (evaluation, system identification, checkpoints): device pointers as above, either may be NULL.  Turns
+ * per-env parameters on if needed.  It does not validate device data: the step kernels clamp a latency to [0, cfg.frame_skip]. */
+int32_t mcb_set_env_latency(mcb_batch* b, const int32_t* latency, const uint64_t* draw_counter, void* stream);
+
 /* replaces mujoco.mj_forward on every env (mycobot.py:213,229,306); refreshes qacc_warmstart; optional obs out */
 int32_t mcb_forward(mcb_batch* b, double* obs, double* achieved_goal, double* desired_goal, void* stream);
 
@@ -292,7 +313,7 @@ int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out
 
 /* Picks the lockstep grouping of the step kernel for this batch (cfg.lockstep_warps == 0): rolls the batch 32 steps
  * ahead (the state right after a reset is not representative), times `steps_per_candidate` (0 -> 4) steps per candidate
- * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters and statistics exactly.  `actions`
+ * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters, latencies and statistics exactly.  `actions`
  * (device float32 [N, action_dim]) are applied at every tuning step; NULL -> uniform random actions from a private
  * Philox stream.  Synchronises the stream and allocates scratch: it is never called implicitly -- mcb_step only enqueues
  * its three kernels on the caller's stream (no hidden sync, CUDA-graph capturable).  Returns the chosen grouping. */

@@ -152,6 +152,10 @@ struct StepArgs {
   unsigned long long* param_ctr;  // [N] parameter draw counters
   int draw_params;           // resets draw new parameters from U[param_lo, param_hi]
   double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
+  // actuation latency (PRM kernels only): a new command takes effect latency[env] substeps after it is issued
+  int* latency;              // [N] substeps, 0..frame_skip
+  unsigned long long* lat_ctr;    // [N] latency draw counters
+  int draw_latency, lat_lo, lat_hi;   // resets draw the latency uniformly from the integers [lat_lo, lat_hi]
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -209,8 +213,9 @@ struct EnvCore {
 };
 // PRM: the batch has per-env physics parameters (mcb_batch_set_param_ranges / mcb_set_env_params).  Batches without them run the
 // PRM = false kernels, whose record is EnvCore itself and whose code does not contain the parameter reads.  With them, the env's
-// MCB_NPARAM multipliers and its parameter draw counter are staged after the working set; `prm_drawn` marks a record a reset redrew
-// (only such records are written back).
+// MCB_NPARAM multipliers and its parameter draw counter are staged after the working set, and so are its actuation latency (substeps,
+// clamped to [0, frame_skip] when loaded) and the latency draw counter; `prm_drawn` marks a record a reset redrew (only such records
+// are written back).
 template <int TIER, bool PRM = false>
 struct EnvS : EnvCore<TIER> { enum { HAS_PRM = 0 }; };
 template <int TIER>
@@ -218,13 +223,15 @@ struct EnvS<TIER, true> : EnvCore<TIER> {
   enum { HAS_PRM = 1 };
   GUARD(gp)
   double prm[MCB_NPARAM];
-  unsigned long long prm_ctr;
-  int prm_drawn, prm_pad_;
+  unsigned long long prm_ctr, lat_ctr;
+  int prm_drawn, lat;
+  int prm_pad_[2];
 };
 static_assert(offsetof(EnvCore<0>, H) % 16 == 0 && offsetof(EnvCore<1>, H) % 16 == 0 && offsetof(EnvCore<2>, H) % 16 == 0, "factor storage must be 16-byte aligned (128-bit loads)");
 static_assert(sizeof(EnvS<0>) % 16 == 0 && sizeof(EnvS<1>) % 16 == 0 && sizeof(EnvS<2>) % 16 == 0, "per-env records must keep 16-byte alignment");
 static_assert(sizeof(EnvS<0, true>) % 16 == 0 && sizeof(EnvS<1, true>) % 16 == 0 && sizeof(EnvS<2, true>) % 16 == 0, "per-env records must keep 16-byte alignment");
-static_assert(sizeof(EnvS<0, true>) - sizeof(EnvS<0>) == 128 + 8 * (MCB_NGUARD ? 2 : 0), "the parameter record is 14 doubles, a counter and a flag");
+static_assert(sizeof(EnvS<0, true>) - sizeof(EnvS<0>) == 144 + 8 * (MCB_NGUARD ? 2 : 0),
+              "the parameter record is 14 doubles, two draw counters, a flag and the latency");
 template <int TIER, bool PRM = false> constexpr size_t cta_bytes() { return MODEL_BYTES + Tier<TIER>::WARPS * sizeof(EnvS<TIER, PRM>); }
 static_assert(cta_bytes<0>() <= 232448 && cta_bytes<1>() <= 232448 && cta_bytes<2>() <= 232448, "a CTA must fit the 227 KB of shared memory an SM offers");
 static_assert(cta_bytes<0, true>() <= 232448 && cta_bytes<1, true>() <= 232448 && cta_bytes<2, true>() <= 232448,
@@ -2118,9 +2125,11 @@ __device__ __forceinline__ const double* grip0_of(const mcb_task_cfg& c) { retur
 __device__ __forceinline__ double hoff_of(const mcb_task_cfg& c) { return c.fetch_env ? MDL.d.key_height_offset : MDL.d.height_offset; }
 
 // Philox4x32-10 counter RNG: one stream per env, key = seed, counter = (env, draw index, stream tag).  Tag GOAL_TAG: goals and cube
-// positions; PARAM_TAG: per-env physics parameters, with a draw counter of their own, so the goal stream is the same with or without them.
+// positions; PARAM_TAG: per-env physics parameters, LATENCY_TAG: actuation latency, each with a draw counter of its own, so the goal
+// stream is the same with or without them.
 #define GOAL_TAG 0x6d79636fu
 #define PARAM_TAG 0x7072616du
+#define LATENCY_TAG 0x6c61746eu
 __device__ __forceinline__ void philox_round(uint32_t* c, uint32_t k0, uint32_t k1) {
   uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
   uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
@@ -2314,7 +2323,7 @@ __device__ void ik_target(S& s, const mcb_task_cfg& cfg, const float* act, int l
 // one DLS solve: ctrl[0..5] += (J'J + 0.3 I)^-1 J' err, J = 6 x 6 site Jacobian w.r.t. the arm dofs (all other columns of
 // the reference's 6 x 18 Jacobian are zero for this site, so its 18 x 18 least-squares problem decouples exactly)
 template <class S>
-__device__ void ik_update_ctrl(S& s, int lane, double grip_ctrl) {
+__device__ void ik_update_ctrl(S& s, int lane, double grip_ctrl, double& cmd) {
   double* Jm = s.grad;          // 36 doubles of scratch: grad, search, Mv are contiguous and dead outside the solver
   double site[3];
   eef_pos_of(s, site);
@@ -2358,8 +2367,11 @@ __device__ void ik_update_ctrl(S& s, int lane, double grip_ctrl) {
   if (lane < 6) s.ik[7 + lane] = b;       // the pose error is consumed (barrier above); reuse its slots for the right-hand side
   __syncwarp();
   double dq = chol_solve_blk<0, 6, false>(s.H, s.H, s.ik + 7, s.Mv, 0.0, lane);
-  if (lane < 6) s.ctrl[lane] += dq;
-  else if (lane == 6) s.ctrl[6] = grip_ctrl;
+  if constexpr (S::HAS_PRM) cmd = lane < 6 ? s.ctrl[lane] + dq : grip_ctrl;   // lanes 0..6: the new ctrl, held until the latency has passed
+  else {
+    if (lane < 6) s.ctrl[lane] += dq;
+    else if (lane == 6) s.ctrl[6] = grip_ctrl;
+  }
   __syncwarp();
 }
 
@@ -2377,6 +2389,17 @@ __device__ __noinline__ bool reset_env(S& s, const StepArgs& a, const DevModel* 
       }
       __syncwarp();
       if (lane == 0) { s.prm_ctr += MCB_NPARAM; s.prm_drawn = 1; }
+      __syncwarp();
+    }
+    // actuation latency: one draw of the latency stream, uniform over the integers [lat_lo, lat_hi]
+    if (a.draw_latency) {
+      if (lane == 0) {
+        unsigned long long c = s.lat_ctr;
+        const double u = philox_uniform<LATENCY_TAG>(a.env_seed[env], env, c);
+        const int span = a.lat_hi - a.lat_lo;
+        s.lat = a.lat_lo + min(span, (int)floor(u * (span + 1)));
+        s.lat_ctr = c; s.prm_drawn = 1;
+      }
       __syncwarp();
     }
   }
@@ -2532,7 +2555,11 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
     if (valid) { load_state(s, a.state + (size_t)env * MCB_STATE_STRIDE, lane); ctr = a.rng_ctr[env]; }
     if constexpr (PRM) {
       if (valid && lane < MCB_NPARAM) s.prm[lane] = a.params[(size_t)env * MCB_NPARAM + lane];
-      if (lane == 0) { s.prm_ctr = valid ? a.param_ctr[env] : 0; s.prm_drawn = 0; }
+      if (lane == 0) {
+        s.prm_ctr = valid ? a.param_ctr[env] : 0; s.prm_drawn = 0;
+        s.lat_ctr = valid ? a.lat_ctr[env] : 0;
+        s.lat = valid ? min(max(a.latency[env], 0), cfg.frame_skip) : 0;    // mcb_set_env_latency does not validate device data
+      }
       __syncwarp();
     }
     double achieved[3];
@@ -2568,6 +2595,12 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
       }
       double grip_ctrl = 0;
       int nblocks = 1;
+      // PRM kernels: the command a controller issues is held in `cmd` on the lane that owns its destination `cmd_dst` and written
+      // before substep `lat` of its block (after the last one when lat == frame_skip); until then the previous command stays in force
+      double cmd = 0;
+      double* cmd_dst = nullptr;
+      int lat = 0;
+      if constexpr (PRM) lat = s.lat;
       if (mocap) {
         // mocap controller (mycobot.py:172-189 + mocap_set_action / reset_mocap2body_xpos): the mocap body goes to the
         // (stale) gripper_tcp pose plus the action deltas; the weld then drags the arm during the 20 substeps
@@ -2579,19 +2612,23 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
           if (lane < 6) s.qpos[lane] = qsave;
           __syncwarp();
           if (lane == 0) {
+            double* mdst = s.mocap;                // PRM kernels: staged in s.grad (scratch here), then held on lanes 0..7
+            if constexpr (PRM) mdst = s.grad;
             double tcp[3];
             const int b2 = MDL.d.weld_body2;
             const double* R = s.xmat + b2 * 9;
             const double* a2 = MDL.d.weld_anchor2;
             for (int r = 0; r < 3; r++) tcp[r] = s.xpos[b2 * 3 + r] + R[3 * r] * a2[0] + R[3 * r + 1] * a2[1] + R[3 * r + 2] * a2[2];
-            for (int k = 0; k < 3; k++) s.mocap[k] = tcp[k] + (double)(act[k] * 0.1f);       // float32 product, float64 sum
+            for (int k = 0; k < 3; k++) mdst[k] = tcp[k] + (double)(act[k] * 0.1f);         // float32 product, float64 sum
             const double fq[4] = {0.5, -0.5, -0.5, 0.5};
             for (int k = 0; k < 4; k++) {
               double tq = s.quat5[k];
               double want = cfg.fetch_env ? fq[k] : (double)act[3 + k];
-              s.mocap[3 + k] = tq + (want - tq);                                             // mocap_quat + (action - tcp_quat)
+              mdst[3 + k] = tq + (want - tq);                                                // mocap_quat + (action - tcp_quat)
             }
             float ag = cfg.fetch_env ? act[3] : act[7];
+            if constexpr (PRM) s.grad[7] = 0.5 + (double)ag * 0.5;
+            else
             s.ctrl[MDL.d.nu - 1] = 0.5 + (double)ag * 0.5;
           }
         }
@@ -2601,6 +2638,8 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
           float v = 0.0f;
 #pragma unroll
           for (int k = 0; k < NU; k++) if (lane == k) v = act[k];
+          if constexpr (PRM) { cmd = (double)v; cmd_dst = s.ctrl + lane; }
+          else
           s.ctrl[lane] = (double)v;
         }
       } else {
@@ -2621,11 +2660,19 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         for (int k = 0; k < 8; k++) if (k == adim - 1) ag = act[k];
         grip_ctrl = 0.5 + (double)ag * 0.5;          // actuation_center + action[-1] * actuation_range (mycobot.py:158-160)
         nblocks = cfg.control_steps;
+        if constexpr (PRM) { if (ok && lane < NU) cmd_dst = s.ctrl + lane; }
       }
       __syncwarp();
+      if constexpr (PRM) {
+        if (mocap && ok && lane < 8) { cmd = s.grad[lane]; cmd_dst = lane < 7 ? s.mocap + lane : s.ctrl + (MDL.d.nu - 1); }
+        __syncwarp();
+      }
       for (int blk = 0; blk < nblocks; blk++) {
-        if (ik && ok) ik_update_ctrl(s, lane, grip_ctrl);
+        if (ik && ok) ik_update_ctrl(s, lane, grip_ctrl, cmd);
         for (int it = 0; it < cfg.frame_skip; it++) {
+          if constexpr (PRM) {
+            if (it == lat) { if (cmd_dst) *cmd_dst = cmd; __syncwarp(); }
+          }
           if (ok) ok = forward(s, m, lane, nba, nva, lockstep);
           else if (lockstep) { for (int k = 0; k < NSYNC_FWD; k++) group_sync(lockstep); }
           if (lockstep) group_sync(lockstep);
@@ -2633,6 +2680,9 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
             if (lane < 6) s.qprev[lane] = s.qpos[lane];     // the frames now in shared memory belong to this qpos
             euler(s, m, lane, nva);
           }
+        }
+        if constexpr (PRM) {
+          if (lat == cfg.frame_skip) { if (cmd_dst) *cmd_dst = cmd; __syncwarp(); }
         }
       }
       substeps = cfg.frame_skip * nblocks;
@@ -2729,7 +2779,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         if constexpr (PRM) {
           if (s.prm_drawn) {
             if (lane < MCB_NPARAM) a.params[(size_t)env * MCB_NPARAM + lane] = s.prm[lane];
-            if (lane == 0) a.param_ctr[env] = s.prm_ctr;
+            if (lane == 0) { a.param_ctr[env] = s.prm_ctr; a.latency[env] = s.lat; a.lat_ctr[env] = s.lat_ctr; }
           }
         }
         if (lane == 0) {
@@ -2819,10 +2869,19 @@ __global__ void random_actions_kernel(float* act, int n, uint64_t seed, unsigned
 }
 
 // mcb_seed(): MyCobotEnv.reset(seed=) reseeds the env's generator (mycobot.py:509-510) -> new Philox key, draw counter 0
-// (pctr: the parameter draw counters of a batch with per-env parameters, or null)
-__global__ void seed_kernel(unsigned long long* env_seed, unsigned long long* ctr, unsigned long long* pctr, const uint8_t* mask, unsigned long long seed, int n) {
+// (pctr, lctr: the parameter and latency draw counters of a batch with per-env parameters, or null)
+__global__ void seed_kernel(unsigned long long* env_seed, unsigned long long* ctr, unsigned long long* pctr, unsigned long long* lctr, const uint8_t* mask,
+                            unsigned long long seed, int n) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n && (!mask || mask[i])) { env_seed[i] = seed; ctr[i] = 0; if (pctr) pctr[i] = 0; }
+  if (i < n && (!mask || mask[i])) { env_seed[i] = seed; ctr[i] = 0; if (pctr) pctr[i] = 0; if (lctr) lctr[i] = 0; }
+}
+// actuation latencies [N] and their draw counters [N]: set 0 batch -> caller (0 and 0 when the batch has none, lat == null),
+// set 1 caller -> batch; any caller pointer may be null
+__global__ void latency_io_kernel(int* lat, unsigned long long* ctr, int* u_lat, unsigned long long* u_ctr, int n, int set) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if (set) { if (u_lat) lat[i] = u_lat[i]; if (u_ctr) ctr[i] = u_ctr[i]; }
+  else { if (u_lat) u_lat[i] = lat ? lat[i] : 0; if (u_ctr) u_ctr[i] = lat ? ctr[i] : 0; }
 }
 // per-env parameters [N, MCB_NPARAM] and draw counters [N]: mode 0 batch -> caller (the nominal 1.0 and 0 when the batch has none,
 // params == null), 1 caller -> batch, 2 nominal values into the batch; any caller pointer may be null
@@ -2930,6 +2989,9 @@ struct mcb_batch {
   double* params; unsigned long long* param_ctr;
   int draw_params;
   double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
+  // actuation latency: allocated with the per-env parameters (0 substeps for every env until set or drawn)
+  int* latency; unsigned long long* lat_ctr;
+  int draw_latency, lat_lo, lat_hi;
   // staging for the host-buffer entry point
   float* d_actions; double *d_obs, *d_ag, *d_dg, *d_fobs; void* d_reward; uint8_t* d_flags;
   float* h_actions; double *h_obs, *h_ag, *h_dg, *h_fobs; void* h_reward; uint8_t* h_flags;
@@ -2987,29 +3049,34 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
   else {
     a.params = b->params; a.param_ctr = b->param_ctr; a.draw_params = b->draw_params;
     memcpy(a.param_lo, b->param_lo, sizeof a.param_lo); memcpy(a.param_hi, b->param_hi, sizeof a.param_hi);
+    a.latency = b->latency; a.lat_ctr = b->lat_ctr; a.draw_latency = b->draw_latency; a.lat_lo = b->lat_lo; a.lat_hi = b->lat_hi;
     e = prm_launch_tiers(b, &a, st);
   }
   if (e != cudaSuccess) return fail("launching the step kernels", e);
   return 0;
 }
 
-// Turns per-env parameters on: allocates them, sets every env to the nominal values (1.0, draw counter 0) and prepares the PRM
-// kernels.  Synchronises the device.  A failure leaves the batch without per-env parameters.
+// Turns per-env parameters on: allocates them and the actuation latencies, sets every env to the nominal values (1.0, latency 0, draw
+// counters 0) and prepares the PRM kernels.  Synchronises the device.  A failure leaves the batch without per-env parameters.
 static int enable_params(mcb_batch* b, const char* who) {
   if (b->params) return 0;
   if (b->cfg.mesh_collision) { g_err = who; g_err += ": per-env parameters are not supported with mesh_collision (hull pairs keep the model's friction)"; return -1; }
   DevGuard guard(b->model->device);
   if (!guard.ok) return fail("enable per-env parameters: cannot select the batch's device", cudaGetLastError());
   const size_t N = (size_t)b->n_envs;
-  double* p = nullptr; unsigned long long* c = nullptr;
+  double* p = nullptr; unsigned long long *c = nullptr, *lc = nullptr; int* lat = nullptr;
   cudaError_t e = prm_set_tier_smem();
   if (e == cudaSuccess) e = cudaMalloc(&p, N * MCB_NPARAM * sizeof(double));
   if (e == cudaSuccess) e = cudaMalloc(&c, N * sizeof(unsigned long long));
+  if (e == cudaSuccess) e = cudaMalloc(&lat, N * sizeof(int));
+  if (e == cudaSuccess) e = cudaMalloc(&lc, N * sizeof(unsigned long long));
+  if (e == cudaSuccess) e = cudaMemset(lat, 0, N * sizeof(int));
+  if (e == cudaSuccess) e = cudaMemset(lc, 0, N * sizeof(unsigned long long));
   if (e == cudaSuccess) { params_io_kernel<<<(b->n_envs + 127) / 128, 128>>>(p, c, nullptr, nullptr, b->n_envs, 2); e = cudaGetLastError(); }
   if (e == cudaSuccess) e = cudaDeviceSynchronize();
-  if (e != cudaSuccess) { cudaFree(p); cudaFree(c); return fail("enable per-env parameters", e); }
+  if (e != cudaSuccess) { cudaFree(p); cudaFree(c); cudaFree(lat); cudaFree(lc); return fail("enable per-env parameters", e); }
   b->launches_total++;
-  b->params = p; b->param_ctr = c;
+  b->params = p; b->param_ctr = c; b->latency = lat; b->lat_ctr = lc;
   return 0;
 }
 
@@ -3039,11 +3106,11 @@ static cudaError_t alloc_staging(mcb_batch* b) {
 }
 
 // A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics,
-// and the per-env parameters with their draw counters (auto-resets redraw them).  The buffers are allocated by the first save()
+// and the per-env parameters and actuation latencies with their draw counters (auto-resets redraw them).  The buffers are allocated by the first save()
 // and freed with the snapshot.
 struct Snapshot {
   const mcb_batch* b;
-  void* copy[7] = {};
+  void* copy[9] = {};
   explicit Snapshot(const mcb_batch* batch) : b(batch) {}
   ~Snapshot() { for (void* p : copy) cudaFree(p); }
   cudaError_t save(cudaStream_t st) { return transfer(true, st); }
@@ -3052,11 +3119,11 @@ struct Snapshot {
  private:
   cudaError_t transfer(bool save, cudaStream_t st) {
     const size_t N = (size_t)b->n_envs;
-    void* live[7] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr};
-    const size_t bytes[7] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
-                             N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long)};
+    void* live[9] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr, b->latency, b->lat_ctr};
+    const size_t bytes[9] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
+                             N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long), N * sizeof(int), N * sizeof(unsigned long long)};
     cudaError_t e = cudaSuccess;
-    for (int k = 0; k < 7 && e == cudaSuccess; k++) {
+    for (int k = 0; k < 9 && e == cudaSuccess; k++) {
       if (!live[k]) continue;      // a batch without per-env parameters
       if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes[k]);
       if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live[k], save ? live[k] : copy[k], bytes[k], cudaMemcpyDeviceToDevice, st);
@@ -3234,7 +3301,7 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
 int32_t mcb_batch_destroy(mcb_batch* b) {
   if (!b) return 0;
   cudaFree(b->state); cudaFree(b->elapsed); cudaFree(b->ep_return); cudaFree(b->rng_ctr); cudaFree(b->env_seed); cudaFree(b->stats); cudaFree(b->debug); cudaFree(b->redo_count); cudaFree(b->redo_list);
-  cudaFree(b->params); cudaFree(b->param_ctr);
+  cudaFree(b->params); cudaFree(b->param_ctr); cudaFree(b->latency); cudaFree(b->lat_ctr);
   free_staging(b);
   delete b;
   return 0;
@@ -3446,7 +3513,7 @@ int32_t mcb_reset_host(mcb_batch* b, const uint8_t* h_mask, const double* h_obj_
 
 int32_t mcb_seed(mcb_batch* b, uint64_t seed, const uint8_t* mask, void* stream) {
   if (!b) return fail("mcb_seed: null batch");
-  seed_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->param_ctr, mask, (unsigned long long)seed, b->n_envs);
+  seed_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->param_ctr, b->lat_ctr, mask, (unsigned long long)seed, b->n_envs);
   CK(cudaGetLastError());
   b->launches_total++;
   if (!mask) b->seed = seed;
@@ -3495,6 +3562,33 @@ int32_t mcb_set_env_params(mcb_batch* b, const double* params, const uint64_t* d
   if (!b) return fail("mcb_set_env_params: null batch");
   if (enable_params(b, "mcb_set_env_params")) return -1;
   params_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->params, b->param_ctr, (double*)params, (unsigned long long*)draw_counter, b->n_envs, 1);
+  CK(cudaGetLastError());
+  b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_batch_set_latency_range(mcb_batch* b, int32_t lo, int32_t hi) {
+  if (!b) return fail("mcb_batch_set_latency_range: null batch");
+  if (lo == -1 && hi == -1) { b->draw_latency = 0; return 0; }
+  if (!(0 <= lo && lo <= hi && hi <= b->cfg.frame_skip)) return fail("mcb_batch_set_latency_range: the range must satisfy 0 <= lo <= hi <= frame_skip");
+  if (enable_params(b, "mcb_batch_set_latency_range")) return -1;
+  b->lat_lo = lo; b->lat_hi = hi;
+  b->draw_latency = 1;
+  return 0;
+}
+
+int32_t mcb_get_env_latency(mcb_batch* b, int32_t* latency, uint64_t* draw_counter, void* stream) {
+  if (!b) return fail("mcb_get_env_latency: null batch");
+  latency_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->latency, b->lat_ctr, latency, (unsigned long long*)draw_counter, b->n_envs, 0);
+  CK(cudaGetLastError());
+  b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_set_env_latency(mcb_batch* b, const int32_t* latency, const uint64_t* draw_counter, void* stream) {
+  if (!b) return fail("mcb_set_env_latency: null batch");
+  if (enable_params(b, "mcb_set_env_latency")) return -1;
+  latency_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->latency, b->lat_ctr, (int*)latency, (unsigned long long*)draw_counter, b->n_envs, 1);
   CK(cudaGetLastError());
   b->launches_total++;
   return 0;

@@ -367,6 +367,35 @@ def param_bounds(param_ranges, mesh_collision=False):
     return lo, hi
 
 
+def latency_bounds(spec, frame_skip, mesh_collision=False):
+    """Actuation latency in substeps, `None | d | (lo, hi)` -> None or (lo, hi), two ints with 0 <= lo <= hi <= frame_skip (an int d
+    gives (d, d)).  Raises ValueError for non-integers (bool and float included), negative bounds, lo > hi, hi > frame_skip, and for
+    mesh_collision=True (latency runs in the kernels of batches with per-env parameters, which hull collisions do not support)."""
+    if spec is None:
+        return None
+    if mesh_collision:
+        raise ValueError("actuation latency is not supported with mesh_collision=True")
+
+    def as_int(v):
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, np.integer)):
+            raise ValueError(f"actuation latency bounds are integers (substeps), got {v!r}")
+        return int(v)
+
+    if isinstance(spec, (tuple, list)):
+        if len(spec) != 2:
+            raise ValueError(f"actuation latency is an int or a pair (lo, hi), got {spec!r}")
+        lo, hi = as_int(spec[0]), as_int(spec[1])
+    else:
+        lo = hi = as_int(spec)
+    if lo < 0:
+        raise ValueError(f"actuation latency must be >= 0, got ({lo}, {hi})")
+    if lo > hi:
+        raise ValueError(f"actuation latency: lo > hi ({lo} > {hi})")
+    if hi > frame_skip:
+        raise ValueError(f"actuation latency must be <= frame_skip ({frame_skip}), got ({lo}, {hi})")
+    return lo, hi
+
+
 def _check_params(p):
     p = np.asarray(p, dtype=np.float64)
     if p.shape != (NPARAM,):

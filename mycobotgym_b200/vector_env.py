@@ -169,7 +169,8 @@ class MyCobotVectorEnv:
                  control_steps=5, controller_type="joint", obj_range=0.1, target_in_the_air=True,
                  distance_threshold=0.01, initial_qpos=None, fetch_env=False, reward_type="sparse", frame_skip=20,
                  max_episode_steps=50, device="cuda:0", seed=0, auto_reset=True, goal_source="device", nefc_max=0,
-                 lockstep_warps=0, autotune=True, mesh_collision=False, param_ranges=None, **kwargs):
+                 lockstep_warps=0, autotune=True, mesh_collision=False, param_ranges=None, actuation_latency=None,
+                 **kwargs):
         """Constructor kwargs are the reference's (mycobot.py:30-46).  `obj_range` and `initial_qpos` are accepted and only
         stored, exactly like the reference does (mycobot.py:54,56 assign them; nothing reads them: the cube is placed by
         `generate_random_point_inside_rectangle`, mycobot.py:220-222, and the start pose is qpos0 / keyframe 0).
@@ -178,7 +179,10 @@ class MyCobotVectorEnv:
         `mesh_collision=True`: the convex hulls of the 28 mesh geoms collide too (MuJoCo: mjc_Convex / mjc_PlaneConvex; here one
         MPR contact per hull pair, DESIGN.md section 4); off, only the plane / box primitives collide.
         `param_ranges={name: (lo, hi)}`: per-env physics parameters (domain randomisation), redrawn on the device at every reset of
-        an env (`flatten.PARAM_NAMES`, groups 'friction' and 'gain'; DESIGN.md section 9).  Not available with mesh_collision."""
+        an env (`flatten.PARAM_NAMES`, groups 'friction' and 'gain'; DESIGN.md section 9).  Not available with mesh_collision.
+        `actuation_latency=d` or `(lo, hi)`: per-env actuation latency in substeps (0 <= lo <= hi <= frame_skip), drawn uniformly from
+        the integers [lo, hi] at every reset of an env: each command the controller issues takes effect that many substeps into its
+        control period (DESIGN.md section 10).  Not available with mesh_collision."""
         if controller_type not in ("joint", "IK", "mocap"):
             raise ValueError(f"unknown controller_type {controller_type!r}")
         if fetch_env and controller_type == "joint":
@@ -191,6 +195,7 @@ class MyCobotVectorEnv:
         if goal_source not in ("device", "reference"):
             raise ValueError("goal_source must be 'device' or 'reference'")
         bounds = None if param_ranges is None else flatten.param_bounds(param_ranges, mesh_collision)
+        lat_bounds = None if actuation_latency is None else flatten.latency_bounds(actuation_latency, int(frame_skip), mesh_collision)
         if not torch.cuda.is_available():
             raise RuntimeError("MyCobotVectorEnv needs a CUDA device; there is no CPU fallback")
         self.device = torch.device(device)
@@ -227,6 +232,10 @@ class MyCobotVectorEnv:
             with torch.cuda.device(dev_index):
                 _lib.check(self._L.mcb_batch_set_param_ranges(h, lo.ctypes.data_as(C.c_void_p), hi.ctypes.data_as(C.c_void_p)))
         self._has_params = bounds is not None
+        if lat_bounds is not None:
+            with torch.cuda.device(dev_index):
+                _lib.check(self._L.mcb_batch_set_latency_range(h, *lat_bounds))
+        self._has_latency = lat_bounds is not None
         self.obs_dim = self._L.mcb_batch_obs_dim(h)
         self.action_dim = self._L.mcb_batch_action_dim(h)          # 7 (joint, IK), 8 (mocap), 4 (fetch variants) (mycobot.py:90-97)
         N, dev = self.num_envs, self.device
@@ -383,6 +392,8 @@ class MyCobotVectorEnv:
                   ep_return=torch.empty(N, dtype=torch.float64, device=dev))
         if self._has_params:
             st["params"], st["param_counter"] = self.get_params()
+        if self._has_latency:
+            st["latency"], st["latency_counter"] = self.get_latency()
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_get_rng_state(self._batch, _ptr(st["env_seed"]), _ptr(st["rng_counter"]), _ptr(st["ep_return"]), self._stream()))
             _lib.check(self._L.mcb_get_state(self._batch, _ptr(st["qpos"]), _ptr(st["qvel"]), _ptr(st["ctrl"]),
@@ -391,9 +402,9 @@ class MyCobotVectorEnv:
         return st
 
     def set_state(self, qpos=None, qvel=None, ctrl=None, qacc_warmstart=None, goal=None, elapsed=None, qprev=None, mocap=None,
-                  env_seed=None, rng_counter=None, ep_return=None, params=None, param_counter=None):
+                  env_seed=None, rng_counter=None, ep_return=None, params=None, param_counter=None, latency=None, latency_counter=None):
         """Inverse of `get_state` (a full checkpoint: physics state, goals, episode clocks, RNG streams, running returns, and the
-        per-env parameters of a batch that has them)."""
+        per-env parameters and actuation latencies of a batch that has them)."""
         def prep(x, shape, dt):
             if x is None:
                 return None
@@ -412,6 +423,8 @@ class MyCobotVectorEnv:
                 _lib.check(self._L.mcb_set_rng_state(self._batch, *[_ptr(t) for t in rs], self._stream()))
         if params is not None or param_counter is not None:
             self.set_params(params, draw_counter=param_counter)
+        if latency is not None or latency_counter is not None:
+            self.set_latency(latency, draw_counter=latency_counter)
         torch.cuda.current_stream(self.device).synchronize()
 
     def get_params(self):
@@ -444,6 +457,40 @@ class MyCobotVectorEnv:
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_set_env_params(self._batch, _ptr(p), _ptr(c), self._stream()))
         self._has_params = True
+
+    def get_latency(self):
+        """(latency int32 [N], draw counters int64 [N]) as device tensors: each env's actuation latency in substeps and how many
+        latency draws it has made since it was seeded.  Without latency: 0 and 0."""
+        N, dev = self.num_envs, self.device
+        d = torch.empty(N, dtype=torch.int32, device=dev)
+        c = torch.empty(N, dtype=torch.int64, device=dev)
+        with torch.cuda.device(self._dev_index):
+            _lib.check(self._L.mcb_get_env_latency(self._batch, _ptr(d), _ptr(c), self._stream()))
+        return d, c
+
+    def set_latency(self, latency, draw_counter=None):
+        """Fixed per-env actuation latencies [N] in substeps, integers in [0, frame_skip] (evaluation, system identification); either
+        argument may be None.  Turns latency on if the batch has none; resets keep redrawing only if `actuation_latency` is set."""
+        if self.mesh_collision:
+            raise ValueError("actuation latency is not supported with mesh_collision=True")
+        N = self.num_envs
+        d = c = None
+        if latency is not None:
+            d = torch.as_tensor(np.asarray(latency) if not torch.is_tensor(latency) else latency)
+            if d.dtype.is_floating_point or d.dtype.is_complex or d.dtype == torch.bool:
+                raise ValueError(f"latency must be an integer tensor, got {d.dtype}")
+            if tuple(d.shape) != (N,):
+                raise ValueError(f"latency must have shape {(N,)}, got {tuple(d.shape)}")
+            if N and (int(d.min()) < 0 or int(d.max()) > self.frame_skip):
+                raise ValueError(f"latency must lie in [0, frame_skip={self.frame_skip}]")
+            d = d.to(device=self.device, dtype=torch.int32).contiguous()
+        if draw_counter is not None:
+            c = torch.as_tensor(np.asarray(draw_counter) if not torch.is_tensor(draw_counter) else draw_counter).to(device=self.device, dtype=torch.int64).contiguous()
+            if tuple(c.shape) != (N,):
+                raise ValueError(f"draw_counter must have shape {(N,)}, got {tuple(c.shape)}")
+        with torch.cuda.device(self._dev_index):
+            _lib.check(self._L.mcb_set_env_latency(self._batch, _ptr(d), _ptr(c), self._stream()))
+        self._has_latency = True
 
     def autotune(self, actions=None, steps_per_candidate=0):
         """Pick the step kernel's lockstep grouping for this batch (explicit: `step` never tunes; the constructor's

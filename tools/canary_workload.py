@@ -1,7 +1,8 @@
 """Workload of the guard-word (MCB_CANARY) build: every controller, every layout tier, resets, reward shaping, a held grasp.
 Run with MCB_LIB pointing at libmycobot_b200_canary.so; prints `CANARY_OK <anomalies>` (tests/test_gpu_canary.py).
 `--params`: the same cases with per-env physics parameters drawn at every reset (tests/test_gpu_env_params.py); the hull-collision
-cases, which do not support them, are left out."""
+cases, which do not support them, are left out.  `--latency`: the same cases with an actuation latency drawn from (0, frame_skip) at
+every reset (tests/test_gpu_latency.py); the hull-collision cases are left out too."""
 import os
 import sys
 
@@ -15,6 +16,7 @@ from mycobotgym_b200.vector_env import MyCobotVectorEnv  # noqa: E402
 
 assert "canary" in _lib.LIB_PATH, _lib.LIB_PATH
 PARAMS = "--params" in sys.argv[1:]
+LATENCY = "--latency" in sys.argv[1:]
 RANGES = {"cube_mass": (0.5, 2.0), "friction": (0.7, 1.3), "gain": (0.8, 1.2), "arm_damping": (0.5, 2.0)}
 gen = torch.Generator(device="cuda")
 gen.manual_seed(0)
@@ -41,6 +43,10 @@ for name, kw, n, adim, steps in CASES:
         if kw.get("mesh_collision"):
             continue
         kw = dict(kw, param_ranges=RANGES)
+    if LATENCY:
+        if kw.get("mesh_collision"):
+            continue
+        kw = dict(kw, actuation_latency=(0, 20))
     env = MyCobotVectorEnv(num_envs=n, seed=3, autotune=False, **kw)
     env.reset()
     env.set_state(elapsed=torch.arange(n, dtype=torch.int32) % 50)
