@@ -291,6 +291,26 @@ int32_t mcb_get_env_latency(mcb_batch* b, int32_t* latency, uint64_t* draw_count
  * per-env parameters on if needed.  It does not validate device data: the step kernels clamp a latency to [0, cfg.frame_skip]. */
 int32_t mcb_set_env_latency(mcb_batch* b, const int32_t* latency, const uint64_t* draw_counter, void* stream);
 
+/* Per-env applied forces (MuJoCo's data.qfrc_applied and data.xfrc_applied on the reduced model), persistent state like in MuJoCo:
+ * they act on every substep of every mcb_step, on the block_gripper forward pass, on mcb_forward and on mcb_debug_forward (whose
+ * qfrc_bias then includes -J' xfrc, so that its qfrc_smooth equals MuJoCo's).  Actuation latency does not delay them.
+ *   qfrc: double[N, MCB_NV], a generalized force per dof, added to qfrc_smooth (mj_fwdAcceleration).
+ *   xfrc: double[N, MCB_NB, 6], per jointed body (mcb_model_desc order) a world-frame force (0:3) and torque (3:6) applied at the
+ *         body's composite centre of mass xpos + xmat * ipos through the body's Jacobian at the current pose (mj_xfrcAccumulate).  For
+ *         the cube that is MuJoCo's xipos; for a body with merged fixed children it is the merged body's centre of mass.
+ * Every reset of an env (mcb_reset, mcb_reset_host, the auto-reset and the bad-simulation reset inside mcb_step) sets its forces to
+ * zero (mj_resetData) before its first forward pass.  In reach envs without reward_shaping the cube is frozen and its forces (body 12,
+ * dofs 12..17) are ignored.  Zero forces give the results of a batch without forces bit for bit.  Forces run in the step kernels of
+ * batches with per-env parameters (nominal multipliers if no ranges are set); they are not available with mesh_collision.
+ *
+ * mcb_set_env_applied: device pointers, either may be NULL (that array is left as it is).  It does not validate device data, like
+ * mcb_set_state: a non-finite force ends the env's episode through the bad-simulation guard, whose reset clears it.  The first call
+ * turns forces on (zero for every env) and per-env parameters with them: it allocates, synchronises and cannot be captured.  Later
+ * calls are one kernel on `stream` and can be captured, so a graph replays steps with whatever the caller's arrays hold. */
+int32_t mcb_set_env_applied(mcb_batch* b, const double* qfrc, const double* xfrc, void* stream);
+/* device pointers as above, either may be NULL; a batch without forces reports zeros */
+int32_t mcb_get_env_applied(mcb_batch* b, double* qfrc, double* xfrc, void* stream);
+
 /* replaces mujoco.mj_forward on every env (mycobot.py:213,229,306); refreshes qacc_warmstart; optional obs out */
 int32_t mcb_forward(mcb_batch* b, double* obs, double* achieved_goal, double* desired_goal, void* stream);
 
@@ -313,7 +333,7 @@ int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out
 
 /* Picks the lockstep grouping of the step kernel for this batch (cfg.lockstep_warps == 0): rolls the batch 32 steps
  * ahead (the state right after a reset is not representative), times `steps_per_candidate` (0 -> 4) steps per candidate
- * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters, latencies and statistics exactly.  `actions`
+ * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters, latencies, applied forces and statistics exactly.  `actions`
  * (device float32 [N, action_dim]) are applied at every tuning step; NULL -> uniform random actions from a private
  * Philox stream.  Synchronises the stream and allocates scratch: it is never called implicitly -- mcb_step only enqueues
  * its three kernels on the caller's stream (no hidden sync, CUDA-graph capturable).  Returns the chosen grouping. */

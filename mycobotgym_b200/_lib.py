@@ -32,6 +32,7 @@ EXPORTS = [
     "mcb_her_sample", "mcb_reset_host", "mcb_seed", "mcb_get_rng_state", "mcb_set_rng_state", "mcb_last_fallback_list", "mcb_total_launches", "mcb_hull_desc_size", "mcb_model_set_hulls",
     "mcb_batch_set_param_ranges", "mcb_get_env_params", "mcb_set_env_params",
     "mcb_batch_set_latency_range", "mcb_get_env_latency", "mcb_set_env_latency",
+    "mcb_set_env_applied", "mcb_get_env_applied",
 ]
 
 
@@ -113,6 +114,8 @@ def load():
     L.mcb_batch_set_latency_range.argtypes = [vp, i32, i32]
     L.mcb_get_env_latency.argtypes = [vp, vp, vp, vp]
     L.mcb_set_env_latency.argtypes = [vp, vp, vp, vp]
+    L.mcb_set_env_applied.argtypes = [vp, vp, vp, vp]
+    L.mcb_get_env_applied.argtypes = [vp, vp, vp, vp]
     L.mcb_total_launches.argtypes = [vp]
     L.mcb_total_launches.restype = i64
     L.mcb_her_create.argtypes = [i32, i32, i32, i32, i32, i32, dbl, u64, C.POINTER(vp)]

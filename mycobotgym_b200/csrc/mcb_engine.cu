@@ -66,6 +66,7 @@
 #define CUBE 12
 #define NMNZ_MAX 96
 #define RM_INEQ 0x10000  // rmeta bit: inequality row (limit / contact)
+#define NFRC (NV + NB * 6)  // applied forces per env: qfrc_applied[NV], then xfrc_applied[NB][6] (world force 0:3, torque 3:6)
 
 namespace {
 
@@ -156,6 +157,8 @@ struct StepArgs {
   int* latency;              // [N] substeps, 0..frame_skip
   unsigned long long* lat_ctr;    // [N] latency draw counters
   int draw_latency, lat_lo, lat_hi;   // resets draw the latency uniformly from the integers [lat_lo, lat_hi]
+  // applied forces (PRM kernels only; null: the batch has none): qfrc_applied (NV) then xfrc_applied (NB x 6) per env
+  double* frc;               // [N, NFRC]
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -215,7 +218,8 @@ struct EnvCore {
 // PRM = false kernels, whose record is EnvCore itself and whose code does not contain the parameter reads.  With them, the env's
 // MCB_NPARAM multipliers and its parameter draw counter are staged after the working set, and so are its actuation latency (substeps,
 // clamped to [0, frame_skip] when loaded) and the latency draw counter; `prm_drawn` marks a record a reset redrew (only such records
-// are written back).
+// are written back).  `frc` points to the env's applied forces in global memory (read there, L1 / L2-resident, not staged): null when
+// the batch has none or once a reset in this launch cleared them; the commit zeroes the row of an env whose pointer was cleared.
 template <int TIER, bool PRM = false>
 struct EnvS : EnvCore<TIER> { enum { HAS_PRM = 0 }; };
 template <int TIER>
@@ -225,13 +229,13 @@ struct EnvS<TIER, true> : EnvCore<TIER> {
   double prm[MCB_NPARAM];
   unsigned long long prm_ctr, lat_ctr;
   int prm_drawn, lat;
-  int prm_pad_[2];
+  const double* frc;
 };
 static_assert(offsetof(EnvCore<0>, H) % 16 == 0 && offsetof(EnvCore<1>, H) % 16 == 0 && offsetof(EnvCore<2>, H) % 16 == 0, "factor storage must be 16-byte aligned (128-bit loads)");
 static_assert(sizeof(EnvS<0>) % 16 == 0 && sizeof(EnvS<1>) % 16 == 0 && sizeof(EnvS<2>) % 16 == 0, "per-env records must keep 16-byte alignment");
 static_assert(sizeof(EnvS<0, true>) % 16 == 0 && sizeof(EnvS<1, true>) % 16 == 0 && sizeof(EnvS<2, true>) % 16 == 0, "per-env records must keep 16-byte alignment");
 static_assert(sizeof(EnvS<0, true>) - sizeof(EnvS<0>) == 144 + 8 * (MCB_NGUARD ? 2 : 0),
-              "the parameter record is 14 doubles, two draw counters, a flag and the latency");
+              "the parameter record is 14 doubles, two draw counters, a flag, the latency and the applied-force pointer");
 template <int TIER, bool PRM = false> constexpr size_t cta_bytes() { return MODEL_BYTES + Tier<TIER>::WARPS * sizeof(EnvS<TIER, PRM>); }
 static_assert(cta_bytes<0>() <= 232448 && cta_bytes<1>() <= 232448 && cta_bytes<2>() <= 232448, "a CTA must fit the 227 KB of shared memory an SM offers");
 static_assert(cta_bytes<0, true>() <= 232448 && cta_bytes<1, true>() <= 232448 && cta_bytes<2, true>() <= 232448,
@@ -1658,7 +1662,7 @@ __device__ bool make_rows(S& s, const DevModel* __restrict__ m, int lane, int nv
   return s.overflow == 0;
 }
 
-// velocity_rne(): cvel, cdof_dot, bias forces (RNE with zero qacc).
+// velocity_rne(): cvel, cdof_dot, bias forces (RNE with zero qacc).  PRM kernels with applied forces: qfrc_bias - J' xfrc_applied.
 template <class S>
 __device__ void velocity_rne(S& s, const DevModel* __restrict__ m, int lane, int nba, int nva) {
   tree_down(s.cvel, s.cdof, s.qvel, 0.0, lane);
@@ -1706,6 +1710,25 @@ __device__ void velocity_rne(S& s, const DevModel* __restrict__ m, int lane, int
     cross_force(t1, s.cvel + lane * 6, t);
     for (int c = 0; c < 6; c++) f[c] += t1[c];
   }
+  if constexpr (S::HAS_PRM) {
+    // xfrc_applied (mj_xfrcAccumulate): the world wrench at the body's centre of mass joins the body's force as the spatial force
+    // about its tree's reference point, with the opposite sign; tree_up and the cdof projection below then give qfrc_bias - J' xfrc
+    const double* fr = s.frc;
+    if (fr && lane < nba) {
+      const double* w = fr + NV + lane * 6;
+      double off[3] = {0.0, 0.0, 0.0};   // the cube's reference point is its centre of mass
+      if (lane != CUBE) {
+        const double* R = s.xmat + lane * 9;
+        const double* ip = MDL.d.ipos[lane];
+#pragma unroll
+        for (int r = 0; r < 3; r++) off[r] = s.xpos[lane * 3 + r] + R[3 * r] * ip[0] + R[3 * r + 1] * ip[1] + R[3 * r + 2] * ip[2] - MDL.d.ref_robot[r];
+      }
+      double tq[3];
+      cross3(tq, off, w);
+      f[0] -= w[3] + tq[0]; f[1] -= w[4] + tq[1]; f[2] -= w[5] + tq[2];
+      f[3] -= w[0]; f[4] -= w[1]; f[5] -= w[2];
+    }
+  }
   __syncwarp();
   if (lane < nba) for (int c = 0; c < 6; c++) s.cacc[lane * 6 + c] = f[c];  // cacc now holds cfrc_body
   __syncwarp();
@@ -1752,7 +1775,12 @@ __device__ void actuation_smooth(S& s, const DevModel* __restrict__ m, int lane,
     if (lane < NV) qa += MDL.d.act_moment[a][lane] * fa;
   }
   if constexpr (S::HAS_PRM) {
-    if (lane < nva) s.qfrc_smooth[lane] = -env_damping(s, lane) * s.qvel[lane] - s.qfrc_bias[lane] + qa;
+    if (lane < nva) {
+      double q = -env_damping(s, lane) * s.qvel[lane] - s.qfrc_bias[lane] + qa;
+      const double* fr = s.frc;
+      if (fr) q += fr[lane];       // qfrc_applied (xfrc_applied is in qfrc_bias, velocity_rne)
+      s.qfrc_smooth[lane] = q;
+    }
   } else
   if (lane < nva) s.qfrc_smooth[lane] = -MDL.d.damping[lane] * s.qvel[lane] - s.qfrc_bias[lane] + qa;
   __syncwarp();
@@ -2402,6 +2430,8 @@ __device__ __noinline__ bool reset_env(S& s, const StepArgs& a, const DevModel* 
       }
       __syncwarp();
     }
+    // applied forces: every reset clears them (mj_resetData), before its first forward pass; the commit zeroes the env's row
+    if (lane == 0) s.frc = nullptr;
   }
   for (int w = lane; w < NQ; w += 32) s.qpos[w] = init_qpos_of(MDL, a.cfg.fetch_env)[w];
   if (lane < NV) s.qvel[lane] = 0;
@@ -2559,6 +2589,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         s.prm_ctr = valid ? a.param_ctr[env] : 0; s.prm_drawn = 0;
         s.lat_ctr = valid ? a.lat_ctr[env] : 0;
         s.lat = valid ? min(max(a.latency[env], 0), cfg.frame_skip) : 0;    // mcb_set_env_latency does not validate device data
+        s.frc = valid && a.frc ? a.frc + (size_t)env * NFRC : nullptr;
       }
       __syncwarp();
     }
@@ -2781,6 +2812,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
             if (lane < MCB_NPARAM) a.params[(size_t)env * MCB_NPARAM + lane] = s.prm[lane];
             if (lane == 0) { a.param_ctr[env] = s.prm_ctr; a.latency[env] = s.lat; a.lat_ctr[env] = s.lat_ctr; }
           }
+          if (a.frc && !s.frc) { for (int w = lane; w < NFRC; w += 32) a.frc[(size_t)env * NFRC + w] = 0.0; }   // a reset cleared the forces
         }
         if (lane == 0) {
           a.rng_ctr[env] = ctr;
@@ -2893,6 +2925,18 @@ __global__ void params_io_kernel(double* params, unsigned long long* ctr, double
   else if (mode == 1) { if (u_params) for (int k = 0; k < MCB_NPARAM; k++) params[o + k] = u_params[o + k]; if (u_ctr) ctr[i] = u_ctr[i]; }
   else { if (u_params) for (int k = 0; k < MCB_NPARAM; k++) u_params[o + k] = params ? params[o + k] : 1.0; if (u_ctr) u_ctr[i] = ctr ? ctr[i] : 0; }
 }
+// applied forces [N, NFRC] <-> qfrc [N, NV] and xfrc [N, NB, 6]: set 0 batch -> caller (zeros when the batch has none, frc == null),
+// set 1 caller -> batch; either caller pointer may be null.  One thread per (env, slot).
+__global__ void applied_io_kernel(double* frc, double* u_qfrc, double* u_xfrc, int n, int set) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)n * NFRC) return;
+  const long long env = i / NFRC;
+  const int k = (int)(i - env * NFRC);
+  double* u = k < NV ? (u_qfrc ? u_qfrc + env * NV + k : nullptr) : (u_xfrc ? u_xfrc + env * (NB * 6) + (k - NV) : nullptr);
+  if (!u) return;
+  if (set) frc[i] = *u;
+  else *u = frc ? frc[i] : 0.0;
+}
 // the part of a checkpoint mcb_get_state / mcb_set_state do not carry: RNG streams and running episode returns
 __global__ void rng_io_kernel(unsigned long long* env_seed, unsigned long long* ctr, double* ep_return, unsigned long long* u_seed, unsigned long long* u_ctr,
                               double* u_ret, int n, int write) {
@@ -2992,6 +3036,8 @@ struct mcb_batch {
   // actuation latency: allocated with the per-env parameters (0 substeps for every env until set or drawn)
   int* latency; unsigned long long* lat_ctr;
   int draw_latency, lat_lo, lat_hi;
+  // applied forces [N, NFRC]: null until mcb_set_env_applied turns them on (which turns per-env parameters on too)
+  double* frc;
   // staging for the host-buffer entry point
   float* d_actions; double *d_obs, *d_ag, *d_dg, *d_fobs; void* d_reward; uint8_t* d_flags;
   float* h_actions; double *h_obs, *h_ag, *h_dg, *h_fobs; void* h_reward; uint8_t* h_flags;
@@ -3050,6 +3096,7 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
     a.params = b->params; a.param_ctr = b->param_ctr; a.draw_params = b->draw_params;
     memcpy(a.param_lo, b->param_lo, sizeof a.param_lo); memcpy(a.param_hi, b->param_hi, sizeof a.param_hi);
     a.latency = b->latency; a.lat_ctr = b->lat_ctr; a.draw_latency = b->draw_latency; a.lat_lo = b->lat_lo; a.lat_hi = b->lat_hi;
+    a.frc = b->frc;
     e = prm_launch_tiers(b, &a, st);
   }
   if (e != cudaSuccess) return fail("launching the step kernels", e);
@@ -3106,11 +3153,11 @@ static cudaError_t alloc_staging(mcb_batch* b) {
 }
 
 // A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics,
-// and the per-env parameters and actuation latencies with their draw counters (auto-resets redraw them).  The buffers are allocated by the first save()
-// and freed with the snapshot.
+// the per-env parameters and actuation latencies with their draw counters (auto-resets redraw them), and the applied forces
+// (resets clear them).  The buffers are allocated by the first save() and freed with the snapshot.
 struct Snapshot {
   const mcb_batch* b;
-  void* copy[9] = {};
+  void* copy[10] = {};
   explicit Snapshot(const mcb_batch* batch) : b(batch) {}
   ~Snapshot() { for (void* p : copy) cudaFree(p); }
   cudaError_t save(cudaStream_t st) { return transfer(true, st); }
@@ -3119,12 +3166,13 @@ struct Snapshot {
  private:
   cudaError_t transfer(bool save, cudaStream_t st) {
     const size_t N = (size_t)b->n_envs;
-    void* live[9] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr, b->latency, b->lat_ctr};
-    const size_t bytes[9] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
-                             N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long), N * sizeof(int), N * sizeof(unsigned long long)};
+    void* live[10] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr, b->latency, b->lat_ctr, b->frc};
+    const size_t bytes[10] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
+                              N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long), N * sizeof(int), N * sizeof(unsigned long long),
+                              N * NFRC * sizeof(double)};
     cudaError_t e = cudaSuccess;
-    for (int k = 0; k < 9 && e == cudaSuccess; k++) {
-      if (!live[k]) continue;      // a batch without per-env parameters
+    for (int k = 0; k < 10 && e == cudaSuccess; k++) {
+      if (!live[k]) continue;      // a batch without per-env parameters or applied forces
       if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes[k]);
       if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live[k], save ? live[k] : copy[k], bytes[k], cudaMemcpyDeviceToDevice, st);
     }
@@ -3301,7 +3349,7 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
 int32_t mcb_batch_destroy(mcb_batch* b) {
   if (!b) return 0;
   cudaFree(b->state); cudaFree(b->elapsed); cudaFree(b->ep_return); cudaFree(b->rng_ctr); cudaFree(b->env_seed); cudaFree(b->stats); cudaFree(b->debug); cudaFree(b->redo_count); cudaFree(b->redo_list);
-  cudaFree(b->params); cudaFree(b->param_ctr); cudaFree(b->latency); cudaFree(b->lat_ctr);
+  cudaFree(b->params); cudaFree(b->param_ctr); cudaFree(b->latency); cudaFree(b->lat_ctr); cudaFree(b->frc);
   free_staging(b);
   delete b;
   return 0;
@@ -3589,6 +3637,40 @@ int32_t mcb_set_env_latency(mcb_batch* b, const int32_t* latency, const uint64_t
   if (!b) return fail("mcb_set_env_latency: null batch");
   if (enable_params(b, "mcb_set_env_latency")) return -1;
   latency_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->latency, b->lat_ctr, (int*)latency, (unsigned long long*)draw_counter, b->n_envs, 1);
+  CK(cudaGetLastError());
+  b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_set_env_applied(mcb_batch* b, const double* qfrc, const double* xfrc, void* stream) {
+  if (!b) return fail("mcb_set_env_applied: null batch");
+  if (b->cfg.mesh_collision) return fail("mcb_set_env_applied: applied forces are not supported with mesh_collision");
+  if (!b->frc) {
+    // first call: zeroed forces for every env, and the PRM kernels that read them; synchronises (not capturable)
+    if (enable_params(b, "mcb_set_env_applied")) return -1;
+    DevGuard guard(b->model->device);
+    if (!guard.ok) return fail("mcb_set_env_applied: cannot select the batch's device", cudaGetLastError());
+    double* f = nullptr;
+    const size_t bytes = (size_t)b->n_envs * NFRC * sizeof(double);
+    cudaError_t e = cudaMalloc(&f, bytes);
+    if (e == cudaSuccess) e = cudaMemset(f, 0, bytes);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) { cudaFree(f); return fail("mcb_set_env_applied: allocating the forces", e); }
+    b->frc = f;
+  }
+  if (!qfrc && !xfrc) return 0;
+  const long long n = (long long)b->n_envs * NFRC;
+  applied_io_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(b->frc, (double*)qfrc, (double*)xfrc, b->n_envs, 1);
+  CK(cudaGetLastError());
+  b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_get_env_applied(mcb_batch* b, double* qfrc, double* xfrc, void* stream) {
+  if (!b) return fail("mcb_get_env_applied: null batch");
+  if (!qfrc && !xfrc) return 0;
+  const long long n = (long long)b->n_envs * NFRC;
+  applied_io_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(b->frc, qfrc, xfrc, b->n_envs, 0);
   CK(cudaGetLastError());
   b->launches_total++;
   return 0;

@@ -19,6 +19,9 @@ from .mjcf import quat2mat, quat_mul
 NB, NV, NQ, NU, NHINGE, NGEOM, MAXPAIR = 13, 18, 19, 7, 12, 5, 12
 MAXHULL, MAXHPAIR = 16, 192
 CUBE_BODY = 12
+# the jointed bodies of the reduced model in mcb_model_desc order (the rows of xfrc_applied): fixed bodies are merged into these
+BODY_NAMES = ("link1", "link2", "link3", "link4", "link5", "link6", "right_gear_link", "right_finger_link", "left_gear_link",
+              "left_finger_link", "right_hinge_link", "left_hinge_link", "object0")
 
 _d = C.c_double
 _i = C.c_int32
@@ -394,6 +397,31 @@ def latency_bounds(spec, frame_skip, mesh_collision=False):
     if hi > frame_skip:
         raise ValueError(f"actuation latency must be <= frame_skip ({frame_skip}), got ({lo}, {hi})")
     return lo, hi
+
+
+def applied_forces(qfrc_applied, xfrc_applied, num_envs, mesh_collision=False):
+    """Checks the arguments of `MyCobotVectorEnv.set_applied_forces` and returns them as contiguous float64 torch tensors (None
+    stays None; input on the CPU stays there): qfrc_applied (N, NV) generalized forces, xfrc_applied (N, NB, 6) world-frame force
+    and torque per body of BODY_NAMES.  Raises ValueError for another shape, a non-finite value, and for mesh_collision=True."""
+    import torch
+
+    if mesh_collision:
+        raise ValueError("applied forces are not supported with mesh_collision=True")
+    out = []
+    for name, x, shape in (("qfrc_applied", qfrc_applied, (num_envs, NV)), ("xfrc_applied", xfrc_applied, (num_envs, NB, 6))):
+        if x is None:
+            out.append(None)
+            continue
+        t = x if torch.is_tensor(x) else torch.as_tensor(np.asarray(x))
+        if t.dtype.is_complex or t.dtype == torch.bool:
+            raise ValueError(f"{name} must be real, got {t.dtype}")
+        if tuple(t.shape) != shape:
+            raise ValueError(f"{name} must have shape {shape}, got {tuple(t.shape)}")
+        t = t.to(dtype=torch.float64).contiguous()
+        if not bool(torch.isfinite(t).all()):
+            raise ValueError(f"{name} must be finite")
+        out.append(t)
+    return tuple(out)
 
 
 def _check_params(p):

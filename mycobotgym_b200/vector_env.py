@@ -236,6 +236,7 @@ class MyCobotVectorEnv:
             with torch.cuda.device(dev_index):
                 _lib.check(self._L.mcb_batch_set_latency_range(h, *lat_bounds))
         self._has_latency = lat_bounds is not None
+        self._has_forces = False
         self.obs_dim = self._L.mcb_batch_obs_dim(h)
         self.action_dim = self._L.mcb_batch_action_dim(h)          # 7 (joint, IK), 8 (mocap), 4 (fetch variants) (mycobot.py:90-97)
         N, dev = self.num_envs, self.device
@@ -394,6 +395,8 @@ class MyCobotVectorEnv:
             st["params"], st["param_counter"] = self.get_params()
         if self._has_latency:
             st["latency"], st["latency_counter"] = self.get_latency()
+        if self._has_forces:
+            st["qfrc_applied"], st["xfrc_applied"] = self.get_applied_forces()
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_get_rng_state(self._batch, _ptr(st["env_seed"]), _ptr(st["rng_counter"]), _ptr(st["ep_return"]), self._stream()))
             _lib.check(self._L.mcb_get_state(self._batch, _ptr(st["qpos"]), _ptr(st["qvel"]), _ptr(st["ctrl"]),
@@ -402,9 +405,10 @@ class MyCobotVectorEnv:
         return st
 
     def set_state(self, qpos=None, qvel=None, ctrl=None, qacc_warmstart=None, goal=None, elapsed=None, qprev=None, mocap=None,
-                  env_seed=None, rng_counter=None, ep_return=None, params=None, param_counter=None, latency=None, latency_counter=None):
+                  env_seed=None, rng_counter=None, ep_return=None, params=None, param_counter=None, latency=None, latency_counter=None,
+                  qfrc_applied=None, xfrc_applied=None):
         """Inverse of `get_state` (a full checkpoint: physics state, goals, episode clocks, RNG streams, running returns, and the
-        per-env parameters and actuation latencies of a batch that has them)."""
+        per-env parameters, actuation latencies and applied forces of a batch that has them)."""
         def prep(x, shape, dt):
             if x is None:
                 return None
@@ -425,6 +429,8 @@ class MyCobotVectorEnv:
             self.set_params(params, draw_counter=param_counter)
         if latency is not None or latency_counter is not None:
             self.set_latency(latency, draw_counter=latency_counter)
+        if qfrc_applied is not None or xfrc_applied is not None:
+            self.set_applied_forces(qfrc_applied, xfrc_applied)
         torch.cuda.current_stream(self.device).synchronize()
 
     def get_params(self):
@@ -491,6 +497,32 @@ class MyCobotVectorEnv:
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_set_env_latency(self._batch, _ptr(d), _ptr(c), self._stream()))
         self._has_latency = True
+
+    def get_applied_forces(self):
+        """(qfrc_applied float64 [N, 18], xfrc_applied float64 [N, 13, 6]) as device tensors: the forces the step applies (see
+        `set_applied_forces`).  Without forces: zeros."""
+        N, dev = self.num_envs, self.device
+        q = torch.empty(N, flatten.NV, dtype=torch.float64, device=dev)
+        x = torch.empty(N, flatten.NB, 6, dtype=torch.float64, device=dev)
+        with torch.cuda.device(self._dev_index):
+            _lib.check(self._L.mcb_get_env_applied(self._batch, _ptr(q), _ptr(x), self._stream()))
+        return q, x
+
+    def set_applied_forces(self, qfrc_applied=None, xfrc_applied=None):
+        """Per-env external forces, MuJoCo's `data.qfrc_applied` and `data.xfrc_applied` on the reduced model (DESIGN.md section 11):
+        `qfrc_applied` [N, 18] generalized forces, `xfrc_applied` [N, 13, 6] a world-frame force (0:3) and torque (3:6) per body of
+        `flatten.BODY_NAMES`, applied at the body's centre of mass.  Torch or numpy input; None leaves that array as it is.  The
+        forces persist: they act on every substep of every following step until set again, and every reset of an env sets its
+        forces to zero.  In reach envs without reward_shaping the cube is frozen and its forces are ignored.  The first call turns
+        forces on (it synchronises).  Every call checks its input on the host (a synchronisation), so it is not capturable itself: call
+        it between the replays of a captured step graph, which then use the new values (the C call `mcb_set_env_applied` on checked
+        device arrays is one kernel on the stream and can be captured).  Not available with mesh_collision."""
+        q, x = flatten.applied_forces(qfrc_applied, xfrc_applied, self.num_envs, self.mesh_collision)
+        q = None if q is None else q.to(self.device)
+        x = None if x is None else x.to(self.device)
+        with torch.cuda.device(self._dev_index):
+            _lib.check(self._L.mcb_set_env_applied(self._batch, _ptr(q), _ptr(x), self._stream()))
+        self._has_forces = True
 
     def autotune(self, actions=None, steps_per_candidate=0):
         """Pick the step kernel's lockstep grouping for this batch (explicit: `step` never tunes; the constructor's

@@ -2,7 +2,9 @@
 Run with MCB_LIB pointing at libmycobot_b200_canary.so; prints `CANARY_OK <anomalies>` (tests/test_gpu_canary.py).
 `--params`: the same cases with per-env physics parameters drawn at every reset (tests/test_gpu_env_params.py); the hull-collision
 cases, which do not support them, are left out.  `--latency`: the same cases with an actuation latency drawn from (0, frame_skip) at
-every reset (tests/test_gpu_latency.py); the hull-collision cases are left out too."""
+every reset (tests/test_gpu_latency.py); the hull-collision cases are left out too.  `--forces`: the same cases with random applied
+forces (qfrc_applied and xfrc_applied) set before every step (tests/test_gpu_applied_forces.py); the hull-collision cases are left
+out too."""
 import os
 import sys
 
@@ -17,6 +19,7 @@ from mycobotgym_b200.vector_env import MyCobotVectorEnv  # noqa: E402
 assert "canary" in _lib.LIB_PATH, _lib.LIB_PATH
 PARAMS = "--params" in sys.argv[1:]
 LATENCY = "--latency" in sys.argv[1:]
+FORCES = "--forces" in sys.argv[1:]
 RANGES = {"cube_mass": (0.5, 2.0), "friction": (0.7, 1.3), "gain": (0.8, 1.2), "arm_damping": (0.5, 2.0)}
 gen = torch.Generator(device="cuda")
 gen.manual_seed(0)
@@ -47,6 +50,8 @@ for name, kw, n, adim, steps in CASES:
         if kw.get("mesh_collision"):
             continue
         kw = dict(kw, actuation_latency=(0, 20))
+    if FORCES and kw.get("mesh_collision"):
+        continue
     env = MyCobotVectorEnv(num_envs=n, seed=3, autotune=False, **kw)
     env.reset()
     env.set_state(elapsed=torch.arange(n, dtype=torch.int32) % 50)
@@ -62,6 +67,9 @@ for name, kw, n, adim, steps in CASES:
         if name == "pick":
             a[:200, :6] = torch.as_tensor(g["qpos0"][:6], device="cuda", dtype=torch.float32)
             a[:200, 6] = 0.8
+        if FORCES:
+            env.set_applied_forces(torch.randn(n, 18, device="cuda", generator=gen) * 0.05,
+                                   torch.randn(n, 13, 6, device="cuda", generator=gen) * torch.tensor([0.2] * 3 + [0.01] * 3, device="cuda"))
         env.step(a)
         if t == 2:
             env.reset(mask=(torch.arange(n) % 3 == 0))
