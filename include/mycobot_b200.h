@@ -47,6 +47,10 @@ extern "C" {
 #define MCB_P_GAIN 6         /* 6..12: actuator u: act_gain[u], act_bias[u][1] and act_bias[u][2] (the servo's kp and kv); mocap variant: u = 0 only */
 #define MCB_P_ARM_DAMPING 13 /* damping[0..5], in the passive force and in Euler's implicit term */
 
+/* Contact output (mcb_set_contact_output): contact slots per env, and doubles per slot: dist, pos[3], frame[9], force[6]. */
+#define MCB_MAXCON 24
+#define MCB_CONTACT_DOUBLES 19
+
 /* Flattened, reduced model (host memory; copied to the device by mcb_model_create).
  * Replaces the compiled mjModel the reference builds in MujocoEnv.__init__ (mycobot.py:69-75). */
 typedef struct mcb_model_desc {
@@ -311,6 +315,28 @@ int32_t mcb_set_env_applied(mcb_batch* b, const double* qfrc, const double* xfrc
 /* device pointers as above, either may be NULL; a batch without forces reports zeros */
 int32_t mcb_get_env_applied(mcb_batch* b, double* qfrc, double* xfrc, void* stream);
 
+/* Per-env contact output (MuJoCo's data.contact with mj_contactForce).  After every mcb_step, mcb_reset and mcb_forward (and their
+ * _host forms), each env that call wrote holds the contacts of its last forward pass, what data.contact / efc_force hold when the
+ * reference returns: the last substep's (contacts at its pre-integration state, forces of its Newton solve), the block_gripper forward
+ * pass's for block_gripper batches, and the reset's for an env that auto-reset (or hit the bad-simulation reset) in the step, so that
+ * the contacts line up with obs.  For such an env the final triple, if registered, receives the contacts of the terminal state before
+ * the reset, the ones the step's reward was computed from; like final_obs, rows of the other envs are left untouched.  A masked
+ * mcb_reset writes the masked envs only; mcb_set_state writes nothing (the next mcb_forward refreshes the contacts).
+ *   ncon: int32[N] contacts in use.
+ *   geom: int32[N, MCB_MAXCON, 3] geom1, geom2 (ids of the MCB_NGEOM primitive geoms in mcb_model_desc order), dim (condim).
+ *   con:  double[N, MCB_MAXCON, MCB_CONTACT_DOUBLES] dist, pos[3], frame[9] (rows: normal, first and second tangent), force[6]:
+ *         mj_contactForce in the contact frame (mju_decodePyramid): force[0] is the sum of the contact's 2 (dim - 1) pyramid forces,
+ *         force[i + 1] = (p[2i] - p[2i + 1]) mu[i] for i < dim - 1 with mu = (sliding, sliding[, torsional]), the rest 0.  Sliding
+ *         friction is the env's mixed value under its per-env parameters.
+ * Slots >= ncon are zero with geom ids -1 and dim 0, so a plain sum over slots is correct.  Contacts that the last layout tier drops
+ * because their constraint rows do not fit are not reported (they are counted in stats[5] and absent from ncon).  All six pointers are
+ * caller-owned device arrays that stay valid while registered; the final triple may be NULL (no final output), and all NULL turns the
+ * output off.  Turning it on turns per-env parameters on (nominal values if no ranges are set).  The call synchronises the device;
+ * steps captured in a CUDA graph afterwards write to the registered arrays.  mcb_autotune restores them exactly.  Not available with
+ * mesh_collision (hull contacts are out of scope). */
+int32_t mcb_set_contact_output(mcb_batch* b, int32_t* ncon, int32_t* geom, double* con, int32_t* final_ncon, int32_t* final_geom,
+                               double* final_con);
+
 /* replaces mujoco.mj_forward on every env (mycobot.py:213,229,306); refreshes qacc_warmstart; optional obs out */
 int32_t mcb_forward(mcb_batch* b, double* obs, double* achieved_goal, double* desired_goal, void* stream);
 
@@ -333,7 +359,7 @@ int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out
 
 /* Picks the lockstep grouping of the step kernel for this batch (cfg.lockstep_warps == 0): rolls the batch 32 steps
  * ahead (the state right after a reset is not representative), times `steps_per_candidate` (0 -> 4) steps per candidate
- * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters, latencies, applied forces and statistics exactly.  `actions`
+ * from that state, keeps the fastest and restores state, episode clocks, RNG streams, per-env parameters, latencies, applied forces, contact output and statistics exactly.  `actions`
  * (device float32 [N, action_dim]) are applied at every tuning step; NULL -> uniform random actions from a private
  * Philox stream.  Synchronises the stream and allocates scratch: it is never called implicitly -- mcb_step only enqueues
  * its three kernels on the caller's stream (no hidden sync, CUDA-graph capturable).  Returns the chosen grouping. */

@@ -33,6 +33,7 @@ EXPORTS = [
     "mcb_batch_set_param_ranges", "mcb_get_env_params", "mcb_set_env_params",
     "mcb_batch_set_latency_range", "mcb_get_env_latency", "mcb_set_env_latency",
     "mcb_set_env_applied", "mcb_get_env_applied",
+    "mcb_set_contact_output",
 ]
 
 
@@ -116,6 +117,7 @@ def load():
     L.mcb_set_env_latency.argtypes = [vp, vp, vp, vp]
     L.mcb_set_env_applied.argtypes = [vp, vp, vp, vp]
     L.mcb_get_env_applied.argtypes = [vp, vp, vp, vp]
+    L.mcb_set_contact_output.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.mcb_total_launches.argtypes = [vp]
     L.mcb_total_launches.restype = i64
     L.mcb_her_create.argtypes = [i32, i32, i32, i32, i32, i32, dbl, u64, C.POINTER(vp)]

@@ -159,6 +159,12 @@ struct StepArgs {
   int draw_latency, lat_lo, lat_hi;   // resets draw the latency uniformly from the integers [lat_lo, lat_hi]
   // applied forces (PRM kernels only; null: the batch has none): qfrc_applied (NV) then xfrc_applied (NB x 6) per env
   double* frc;               // [N, NFRC]
+  // contact output (PRM kernels only; null con_n: off): the contacts of each written env's last forward pass, and (con_fn set) those
+  // of the terminal state before an auto-reset; ncon [N], geom1 / geom2 / dim [N, MCB_MAXCON, 3], dist pos frame force [N, MCB_MAXCON, 19]
+  int *con_n, *con_geom;
+  double* con;
+  int *con_fn, *con_fgeom;
+  double* con_f;
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -171,6 +177,7 @@ template <int TIER> struct Tier;
 template <> struct Tier<0> { enum { WARPS = 16, NROW = 48, POOL = 460, MAXC = 8 }; };
 template <> struct Tier<1> { enum { WARPS = 10, NROW = 88, POOL = 1230, MAXC = 14 }; };
 template <> struct Tier<2> { enum { WARPS = 5, NROW = 176, POOL = 2432, MAXC = 24 }; };
+static_assert(Tier<2>::MAXC == MCB_MAXCON, "the contact output holds every contact the last tier keeps");
 template <int TIER>
 struct EnvCore {
   // MCB_CANARY build (tests/test_gpu_canary.py; compute-sanitizer is closed on the GPU pool): guard words between the arrays of
@@ -2517,6 +2524,44 @@ __device__ void debug_dump(S& s, const StepArgs& a, int lane, int nva) {
   }
 }
 
+// Contact output of env `env` from the last forward pass (PRM kernels): lane c < ncon writes contact c -- geom1, geom2, dim; dist, pos,
+// frame, and mj_contactForce in the contact frame (mju_decodePyramid) -- and lanes past ncon zero-fill the empty slots (geom ids -1),
+// so every call rewrites the env's whole row.  Pyramid forces are recomputed from eJaref, which is current at every exit of
+// Newton::solve (eJv is not: it holds J search or D active there), with the formula of update_cost_grad: -D jar on active rows.
+template <class S>
+__device__ __noinline__ void write_contacts(const S& s, int* dst_n, int* dst_geom, double* dst_con, int env, int lane) {
+  static_assert(S::HAS_PRM, "the contact output runs in the kernels with per-env parameters (env_mu)");
+  const int ncon = s.ncon;
+  if (lane == 0) dst_n[env] = ncon;
+  if (lane < MCB_MAXCON) {
+    int* g = dst_geom + ((size_t)env * MCB_MAXCON + lane) * 3;
+    double* o = dst_con + ((size_t)env * MCB_MAXCON + lane) * MCB_CONTACT_DOUBLES;
+    if (lane < ncon) {
+      const PairParam& pp = PP(s.cpair[lane]);
+      const int dim = pp.dim, r0 = s.crow[lane];
+      g[0] = pp.g1; g[1] = pp.g2; g[2] = dim;
+      o[0] = s.cdist[lane];
+      for (int k = 0; k < 3; k++) o[1 + k] = s.cpos[lane * 3 + k];
+      for (int k = 0; k < 9; k++) o[4 + k] = s.cframe[lane * 9 + k];
+      double p[6];
+      for (int k = 0; k < 6; k++) {
+        const double jar = k < 2 * (dim - 1) ? s.eJaref[r0 + k] : 0.0;   // contact rows are inequalities: active iff jar < 0
+        p[k] = jar < 0 ? -s.eD[r0 + k] * jar : 0.0;
+      }
+      const double mu = env_mu(s, pp);                                     // sliding (both tangents); torsional: pp.friction[1]
+      o[13] = p[0] + p[1] + p[2] + p[3] + p[4] + p[5];
+      o[14] = (p[0] - p[1]) * mu;
+      o[15] = (p[2] - p[3]) * mu;
+      o[16] = dim == 4 ? (p[4] - p[5]) * pp.friction[1] : 0.0;
+      o[17] = 0.0; o[18] = 0.0;
+    } else {
+      g[0] = -1; g[1] = -1; g[2] = 0;
+      for (int k = 0; k < MCB_CONTACT_DOUBLES; k++) o[k] = 0.0;
+    }
+  }
+  __syncwarp();
+}
+
 // ------------------------------------------------------------------------------------------------
 // The env kernel: one warp per env, Tier<TIER>::WARPS warps per CTA.  TIER 0 is the first launch over all envs; envs whose
 // constraint set overflows a tier's layout leave every output untouched and enqueue themselves on that tier's redo list,
@@ -2601,6 +2646,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
       if (ok) ok = reset_env(s, a, m, lane, env, nba, nva, ctr);
       if (ok) {
         write_obs(s, m, cfg, lane, env, a.obs, a.ag, a.dg, achieved);
+        if constexpr (PRM) { if (a.con_n) write_contacts(s, a.con_n, a.con_geom, a.con, env, lane); }
         if (lane == 0) { a.elapsed[env] = 0; a.ep_return[env] = 0; }
       }
       substeps = 2;
@@ -2611,6 +2657,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         __syncwarp();
         write_obs(s, m, cfg, lane, env, a.obs, a.ag, a.dg, achieved);
         if (a.debug && env == a.debug_env) debug_dump(s, a, lane, nva);
+        if constexpr (PRM) { if (a.con_n) write_contacts(s, a.con_n, a.con_geom, a.con, env, lane); }
       }
       substeps = 1;
     } else {
@@ -2772,10 +2819,14 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
             double dummy[3];
             write_obs(s, m, cfg, lane, env, a.final_obs, nullptr, nullptr, dummy);
           }
+          if constexpr (PRM) { if (a.con_fn) write_contacts(s, a.con_fn, a.con_fgeom, a.con_f, env, lane); }   // the terminal state's
           ok = reset_env(s, a, m, lane, env, nba, nva, ctr);
           if (ok) write_obs(s, m, cfg, lane, env, a.obs, a.ag, a.dg, achieved);
           el = 0; epret = 0; substeps += 2;
         }
+        // the last forward pass: the substep loop's or the block_gripper one (euler, write_obs and the reward leave the rows alone),
+        // or the reset's for an env that was just reset
+        if constexpr (PRM) { if (ok && a.con_n) write_contacts(s, a.con_n, a.con_geom, a.con, env, lane); }
         if (ok && lane == 0) {
           if (cfg.reward_type == 0) ((float*)a.reward)[env] = -(float)(dist > cfg.distance_threshold);
           else ((double*)a.reward)[env] = rew;
@@ -3038,6 +3089,9 @@ struct mcb_batch {
   int draw_latency, lat_lo, lat_hi;
   // applied forces [N, NFRC]: null until mcb_set_env_applied turns them on (which turns per-env parameters on too)
   double* frc;
+  // contact output: caller-owned device arrays (mcb_set_contact_output), null when off; the final triple is optional
+  int *con_n, *con_geom; double* con;
+  int *con_fn, *con_fgeom; double* con_f;
   // staging for the host-buffer entry point
   float* d_actions; double *d_obs, *d_ag, *d_dg, *d_fobs; void* d_reward; uint8_t* d_flags;
   float* h_actions; double *h_obs, *h_ag, *h_dg, *h_fobs; void* h_reward; uint8_t* h_flags;
@@ -3097,6 +3151,7 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
     memcpy(a.param_lo, b->param_lo, sizeof a.param_lo); memcpy(a.param_hi, b->param_hi, sizeof a.param_hi);
     a.latency = b->latency; a.lat_ctr = b->lat_ctr; a.draw_latency = b->draw_latency; a.lat_lo = b->lat_lo; a.lat_hi = b->lat_hi;
     a.frc = b->frc;
+    a.con_n = b->con_n; a.con_geom = b->con_geom; a.con = b->con; a.con_fn = b->con_fn; a.con_fgeom = b->con_fgeom; a.con_f = b->con_f;
     e = prm_launch_tiers(b, &a, st);
   }
   if (e != cudaSuccess) return fail("launching the step kernels", e);
@@ -3153,11 +3208,12 @@ static cudaError_t alloc_staging(mcb_batch* b) {
 }
 
 // A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics,
-// the per-env parameters and actuation latencies with their draw counters (auto-resets redraw them), and the applied forces
-// (resets clear them).  The buffers are allocated by the first save() and freed with the snapshot.
+// the per-env parameters and actuation latencies with their draw counters (auto-resets redraw them), the applied forces
+// (resets clear them) and the registered contact output.  The buffers are allocated by the first save() and freed with the snapshot.
 struct Snapshot {
+  enum { NBUF = 16 };
   const mcb_batch* b;
-  void* copy[10] = {};
+  void* copy[NBUF] = {};
   explicit Snapshot(const mcb_batch* batch) : b(batch) {}
   ~Snapshot() { for (void* p : copy) cudaFree(p); }
   cudaError_t save(cudaStream_t st) { return transfer(true, st); }
@@ -3166,13 +3222,16 @@ struct Snapshot {
  private:
   cudaError_t transfer(bool save, cudaStream_t st) {
     const size_t N = (size_t)b->n_envs;
-    void* live[10] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr, b->latency, b->lat_ctr, b->frc};
-    const size_t bytes[10] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
-                              N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long), N * sizeof(int), N * sizeof(unsigned long long),
-                              N * NFRC * sizeof(double)};
+    void* live[NBUF] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr, b->latency, b->lat_ctr, b->frc,
+                        b->con_n, b->con_geom, b->con, b->con_fn, b->con_fgeom, b->con_f};
+    const size_t NC = N * MCB_MAXCON;
+    const size_t bytes[NBUF] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
+                                N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long), N * sizeof(int), N * sizeof(unsigned long long),
+                                N * NFRC * sizeof(double), N * sizeof(int), NC * 3 * sizeof(int), NC * MCB_CONTACT_DOUBLES * sizeof(double),
+                                N * sizeof(int), NC * 3 * sizeof(int), NC * MCB_CONTACT_DOUBLES * sizeof(double)};
     cudaError_t e = cudaSuccess;
-    for (int k = 0; k < 10 && e == cudaSuccess; k++) {
-      if (!live[k]) continue;      // a batch without per-env parameters or applied forces
+    for (int k = 0; k < NBUF && e == cudaSuccess; k++) {
+      if (!live[k]) continue;      // a batch without per-env parameters, applied forces or contact output
       if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes[k]);
       if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live[k], save ? live[k] : copy[k], bytes[k], cudaMemcpyDeviceToDevice, st);
     }
@@ -3673,6 +3732,25 @@ int32_t mcb_get_env_applied(mcb_batch* b, double* qfrc, double* xfrc, void* stre
   applied_io_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(b->frc, qfrc, xfrc, b->n_envs, 0);
   CK(cudaGetLastError());
   b->launches_total++;
+  return 0;
+}
+
+int32_t mcb_set_contact_output(mcb_batch* b, int32_t* ncon, int32_t* geom, double* con, int32_t* final_ncon, int32_t* final_geom, double* final_con) {
+  if (!b) return fail("mcb_set_contact_output: null batch");
+  const bool on = ncon || geom || con, fin = final_ncon || final_geom || final_con;
+  if (on && !(ncon && geom && con)) return fail("mcb_set_contact_output: ncon, geom and con are given together");
+  if (fin && !(final_ncon && final_geom && final_con)) return fail("mcb_set_contact_output: final_ncon, final_geom and final_con are given together");
+  if (fin && !on) return fail("mcb_set_contact_output: the final contacts need ncon, geom and con too");
+  if (on) {
+    if (b->cfg.mesh_collision) return fail("mcb_set_contact_output: contact output is not supported with mesh_collision");
+    if (enable_params(b, "mcb_set_contact_output")) return -1;
+  }
+  // launches already enqueued write to the arrays registered before
+  DevGuard guard(b->model->device);
+  if (!guard.ok) return fail("mcb_set_contact_output: cannot select the batch's device", cudaGetLastError());
+  CK(cudaDeviceSynchronize());
+  b->con_n = ncon; b->con_geom = geom; b->con = con;
+  b->con_fn = final_ncon; b->con_fgeom = final_geom; b->con_f = final_con;
   return 0;
 }
 

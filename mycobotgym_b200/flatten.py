@@ -22,6 +22,9 @@ CUBE_BODY = 12
 # the jointed bodies of the reduced model in mcb_model_desc order (the rows of xfrc_applied): fixed bodies are merged into these
 BODY_NAMES = ("link1", "link2", "link3", "link4", "link5", "link6", "right_gear_link", "right_finger_link", "left_gear_link",
               "left_finger_link", "right_hinge_link", "left_hinge_link", "object0")
+# the primitive geoms in mcb_model_desc order: the geom ids of the contact output (MyCobotVectorEnv.contacts)
+GEOM_NAMES = ("floor", "table", "right_finger_layer", "left_finger_layer", "object0")
+MAXCON, CONTACT_DOUBLES = 24, 19     # MCB_MAXCON contact slots per env, MCB_CONTACT_DOUBLES per slot: dist, pos3, frame9, force6
 
 _d = C.c_double
 _i = C.c_int32

@@ -170,7 +170,7 @@ class MyCobotVectorEnv:
                  distance_threshold=0.01, initial_qpos=None, fetch_env=False, reward_type="sparse", frame_skip=20,
                  max_episode_steps=50, device="cuda:0", seed=0, auto_reset=True, goal_source="device", nefc_max=0,
                  lockstep_warps=0, autotune=True, mesh_collision=False, param_ranges=None, actuation_latency=None,
-                 **kwargs):
+                 contact_output=False, **kwargs):
         """Constructor kwargs are the reference's (mycobot.py:30-46).  `obj_range` and `initial_qpos` are accepted and only
         stored, exactly like the reference does (mycobot.py:54,56 assign them; nothing reads them: the cube is placed by
         `generate_random_point_inside_rectangle`, mycobot.py:220-222, and the start pose is qpos0 / keyframe 0).
@@ -182,7 +182,9 @@ class MyCobotVectorEnv:
         an env (`flatten.PARAM_NAMES`, groups 'friction' and 'gain'; DESIGN.md section 9).  Not available with mesh_collision.
         `actuation_latency=d` or `(lo, hi)`: per-env actuation latency in substeps (0 <= lo <= hi <= frame_skip), drawn uniformly from
         the integers [lo, hi] at every reset of an env: each command the controller issues takes effect that many substeps into its
-        control period (DESIGN.md section 10).  Not available with mesh_collision."""
+        control period (DESIGN.md section 10).  Not available with mesh_collision.
+        `contact_output=True`: every step, reset and forward writes the contacts of each env's last forward pass and their forces
+        into persistent device buffers, read with `contacts()` (DESIGN.md section 12).  Not available with mesh_collision."""
         if controller_type not in ("joint", "IK", "mocap"):
             raise ValueError(f"unknown controller_type {controller_type!r}")
         if fetch_env and controller_type == "joint":
@@ -196,6 +198,8 @@ class MyCobotVectorEnv:
             raise ValueError("goal_source must be 'device' or 'reference'")
         bounds = None if param_ranges is None else flatten.param_bounds(param_ranges, mesh_collision)
         lat_bounds = None if actuation_latency is None else flatten.latency_bounds(actuation_latency, int(frame_skip), mesh_collision)
+        if contact_output and mesh_collision:
+            raise ValueError("contact output is not supported with mesh_collision=True")
         if not torch.cuda.is_available():
             raise RuntimeError("MyCobotVectorEnv needs a CUDA device; there is no CPU fallback")
         self.device = torch.device(device)
@@ -250,6 +254,18 @@ class MyCobotVectorEnv:
         self._trunc = torch.zeros(N, dtype=torch.uint8, device=dev)
         self._succ = torch.zeros(N, dtype=torch.uint8, device=dev)
         self._stats = torch.zeros(8, dtype=f64, device=dev)
+        self._contacts = None
+        if contact_output:
+            # (ncon, geom1 / geom2 / dim, dist pos frame force) for the last forward pass, then for the terminal state of auto-reset envs
+            bufs = tuple((torch.zeros(N, dtype=torch.int32, device=dev),
+                          torch.full((N, flatten.MAXCON, 3), -1, dtype=torch.int32, device=dev),
+                          torch.zeros(N, flatten.MAXCON, flatten.CONTACT_DOUBLES, dtype=f64, device=dev)) for _ in range(2))
+            for b in bufs:
+                b[1][..., 2] = 0
+            torch.cuda.synchronize(dev)
+            with torch.cuda.device(dev_index):
+                _lib.check(self._L.mcb_set_contact_output(h, *(_ptr(t) for b in bufs for t in b)))
+            self._contacts = bufs
         self.initial_gripper_xpos = np.array((self._desc.key_initial_gripper_xpos if fetch_env else self._desc.initial_gripper_xpos)[:])
         self.height_offset = float(self._desc.key_height_offset if fetch_env else self._desc.height_offset)
         self._sampler = ReferenceGoalSampler(N, self.height_offset, self.initial_gripper_xpos[:2], self.has_object,
@@ -360,6 +376,9 @@ class MyCobotVectorEnv:
             if self.goal_source == "reference":
                 if bool(done.any()):
                     self._final_obs.copy_(self._obs)
+                    if self._contacts is not None:
+                        for dst, src in zip(self._contacts[1], self._contacts[0]):
+                            dst.copy_(src)
                     self.reset(mask=done)
             info["final_observation"] = self._final_obs
             info["_final_observation"] = done
@@ -523,6 +542,26 @@ class MyCobotVectorEnv:
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_set_env_applied(self._batch, _ptr(q), _ptr(x), self._stream()))
         self._has_forces = True
+
+    def contacts(self, final=False):
+        """The contacts of each env's last forward pass (MuJoCo's `data.contact` with `mj_contactForce`), as named views of the env's
+        persistent device buffers (batches made with `contact_output=True`; same aliasing contract as `step`: the next step, reset or
+        forward overwrites them, clone to keep):
+          ncon int32 [N]; geom int32 [N, 24, 2] (geom1, geom2: indices into `flatten.GEOM_NAMES`); dim int32 [N, 24] (condim);
+          dist [N, 24]; pos [N, 24, 3] (world); frame [N, 24, 3, 3] (rows: normal from geom1 to geom2, then the two tangents);
+          force [N, 24, 6]: the force on geom2 (geom1 takes its opposite) in the contact frame: normal, tangent 1, tangent 2,
+          torsional (condim 4), 0, 0.
+        Slots >= ncon are zero with geom ids -1.  After a step: the last substep's contacts (the block_gripper forward pass's if
+        block_gripper), or the reset's for an env that auto-reset.  `final=True`: for envs that auto-reset in the last step, the
+        contacts of the terminal state (those the step's reward saw); rows of other envs are left as they were.  The world-frame
+        force of every contact is
+          torch.einsum("nckj,nck->ncj", c["frame"], c["force"][..., :3])   # frame[..., :3, :].transpose . force[..., :3]
+        Contacts the last layout tier drops for lack of constraint rows are not reported (DESIGN.md section 12)."""
+        if self._contacts is None:
+            raise RuntimeError("contact output is off: make the env with contact_output=True")
+        n, g, c = self._contacts[1 if final else 0]
+        return dict(ncon=n, geom=g[..., :2], dim=g[..., 2], dist=c[..., 0], pos=c[..., 1:4], frame=c[..., 4:13].unflatten(-1, (3, 3)),
+                    force=c[..., 13:19])
 
     def autotune(self, actions=None, steps_per_candidate=0):
         """Pick the step kernel's lockstep grouping for this batch (explicit: `step` never tunes; the constructor's

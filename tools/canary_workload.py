@@ -4,7 +4,8 @@ Run with MCB_LIB pointing at libmycobot_b200_canary.so; prints `CANARY_OK <anoma
 cases, which do not support them, are left out.  `--latency`: the same cases with an actuation latency drawn from (0, frame_skip) at
 every reset (tests/test_gpu_latency.py); the hull-collision cases are left out too.  `--forces`: the same cases with random applied
 forces (qfrc_applied and xfrc_applied) set before every step (tests/test_gpu_applied_forces.py); the hull-collision cases are left
-out too."""
+out too.  `--contacts`: the same cases with contact output on (tests/test_gpu_contacts.py), plus a forward pass; the hull-collision
+cases are left out too."""
 import os
 import sys
 
@@ -20,6 +21,7 @@ assert "canary" in _lib.LIB_PATH, _lib.LIB_PATH
 PARAMS = "--params" in sys.argv[1:]
 LATENCY = "--latency" in sys.argv[1:]
 FORCES = "--forces" in sys.argv[1:]
+CONTACTS = "--contacts" in sys.argv[1:]
 RANGES = {"cube_mass": (0.5, 2.0), "friction": (0.7, 1.3), "gain": (0.8, 1.2), "arm_damping": (0.5, 2.0)}
 gen = torch.Generator(device="cuda")
 gen.manual_seed(0)
@@ -50,8 +52,10 @@ for name, kw, n, adim, steps in CASES:
         if kw.get("mesh_collision"):
             continue
         kw = dict(kw, actuation_latency=(0, 20))
-    if FORCES and kw.get("mesh_collision"):
+    if (FORCES or CONTACTS) and kw.get("mesh_collision"):
         continue
+    if CONTACTS:
+        kw = dict(kw, contact_output=True)
     env = MyCobotVectorEnv(num_envs=n, seed=3, autotune=False, **kw)
     env.reset()
     env.set_state(elapsed=torch.arange(n, dtype=torch.int32) % 50)
@@ -73,6 +77,8 @@ for name, kw, n, adim, steps in CASES:
         env.step(a)
         if t == 2:
             env.reset(mask=(torch.arange(n) % 3 == 0))
+    if CONTACTS:
+        env.forward()
     s = env.stats().cpu().numpy()
     print(f"{name:24s} env_steps {int(s[4]):7d}  left tier 0 / 1 in the last step {env.last_fallback_envs()}  anomalies {s[5]:.0f}", flush=True)
     total += s[5]
