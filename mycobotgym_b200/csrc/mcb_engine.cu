@@ -124,6 +124,27 @@ enum { ST_QPOS = 0, ST_QVEL = ST_QPOS + NQ, ST_CTRL = ST_QVEL + NV, ST_WARM = ST
        ST_MOCAP = ST_QPREV + 6, ST_END = ST_MOCAP + 7 };
 static_assert(ST_END <= MCB_STATE_STRIDE, "the state record must fit its stride");
 
+// The per-env extensions of a batch, read by the PRM kernels only: one record, held by the batch and copied whole into StepArgs.
+struct EnvExt {
+  // per-env physics parameters
+  double* params;            // [N, MCB_NPARAM] multipliers
+  unsigned long long* param_ctr;  // [N] parameter draw counters
+  int draw_params;           // resets draw new parameters from U[param_lo, param_hi]
+  double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
+  // actuation latency: a new command takes effect latency[env] substeps after it is issued
+  int* latency;              // [N] substeps, 0..frame_skip
+  unsigned long long* lat_ctr;    // [N] latency draw counters
+  int draw_latency, lat_lo, lat_hi;   // resets draw the latency uniformly from the integers [lat_lo, lat_hi]
+  // applied forces (null: the batch has none): qfrc_applied (NV) then xfrc_applied (NB x 6) per env
+  double* frc;               // [N, NFRC]
+  // contact output (caller-owned; null con_n: off): the contacts of each written env's last forward pass, and (con_fn set) those
+  // of the terminal state before an auto-reset; ncon [N], geom1 / geom2 / dim [N, MCB_MAXCON, 3], dist pos frame force [N, MCB_MAXCON, 19]
+  int *con_n, *con_geom;
+  double* con;
+  int *con_fn, *con_fgeom;
+  double* con_f;
+};
+
 struct StepArgs {
   const DevModel* m;
   int n_envs, mode;
@@ -148,23 +169,7 @@ struct StepArgs {
   double* debug;             // optional debug dump of env debug_env
   int debug_env;
   int canary_selftest;       // MCB_CANARY build + MCB_CANARY_SELFTEST=1 in the environment: every env writes one double past cpos[] on purpose
-  // per-env physics parameters (read by the PRM kernels only)
-  double* params;            // [N, MCB_NPARAM] multipliers
-  unsigned long long* param_ctr;  // [N] parameter draw counters
-  int draw_params;           // resets draw new parameters from U[param_lo, param_hi]
-  double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
-  // actuation latency (PRM kernels only): a new command takes effect latency[env] substeps after it is issued
-  int* latency;              // [N] substeps, 0..frame_skip
-  unsigned long long* lat_ctr;    // [N] latency draw counters
-  int draw_latency, lat_lo, lat_hi;   // resets draw the latency uniformly from the integers [lat_lo, lat_hi]
-  // applied forces (PRM kernels only; null: the batch has none): qfrc_applied (NV) then xfrc_applied (NB x 6) per env
-  double* frc;               // [N, NFRC]
-  // contact output (PRM kernels only; null con_n: off): the contacts of each written env's last forward pass, and (con_fn set) those
-  // of the terminal state before an auto-reset; ncon [N], geom1 / geom2 / dim [N, MCB_MAXCON, 3], dist pos frame force [N, MCB_MAXCON, 19]
-  int *con_n, *con_geom;
-  double* con;
-  int *con_fn, *con_fgeom;
-  double* con_f;
+  EnvExt x;                  // the batch's per-env extensions (PRM kernels only)
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -2415,11 +2420,11 @@ template <class S>
 __device__ __noinline__ bool reset_env(S& s, const StepArgs& a, const DevModel* __restrict__ m, int lane, int env, int nba, int nva, unsigned long long& ctr) {
   if constexpr (S::HAS_PRM) {
     // per-env parameters: slot k ~ U[lo_k, hi_k] from draw prm_ctr + k of the parameter stream, before the first forward pass
-    if (a.draw_params) {
+    if (a.x.draw_params) {
       if (lane < MCB_NPARAM) {
         unsigned long long c = s.prm_ctr + (unsigned long long)lane;
         const double u = philox_uniform<PARAM_TAG>(a.env_seed[env], env, c);
-        const double lo = a.param_lo[lane], hi = a.param_hi[lane];
+        const double lo = a.x.param_lo[lane], hi = a.x.param_hi[lane];
         s.prm[lane] = fmin(hi, lo + (hi - lo) * u);
       }
       __syncwarp();
@@ -2427,12 +2432,12 @@ __device__ __noinline__ bool reset_env(S& s, const StepArgs& a, const DevModel* 
       __syncwarp();
     }
     // actuation latency: one draw of the latency stream, uniform over the integers [lat_lo, lat_hi]
-    if (a.draw_latency) {
+    if (a.x.draw_latency) {
       if (lane == 0) {
         unsigned long long c = s.lat_ctr;
         const double u = philox_uniform<LATENCY_TAG>(a.env_seed[env], env, c);
-        const int span = a.lat_hi - a.lat_lo;
-        s.lat = a.lat_lo + min(span, (int)floor(u * (span + 1)));
+        const int span = a.x.lat_hi - a.x.lat_lo;
+        s.lat = a.x.lat_lo + min(span, (int)floor(u * (span + 1)));
         s.lat_ctr = c; s.prm_drawn = 1;
       }
       __syncwarp();
@@ -2629,12 +2634,12 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
     unsigned long long ctr = 0;
     if (valid) { load_state(s, a.state + (size_t)env * MCB_STATE_STRIDE, lane); ctr = a.rng_ctr[env]; }
     if constexpr (PRM) {
-      if (valid && lane < MCB_NPARAM) s.prm[lane] = a.params[(size_t)env * MCB_NPARAM + lane];
+      if (valid && lane < MCB_NPARAM) s.prm[lane] = a.x.params[(size_t)env * MCB_NPARAM + lane];
       if (lane == 0) {
-        s.prm_ctr = valid ? a.param_ctr[env] : 0; s.prm_drawn = 0;
-        s.lat_ctr = valid ? a.lat_ctr[env] : 0;
-        s.lat = valid ? min(max(a.latency[env], 0), cfg.frame_skip) : 0;    // mcb_set_env_latency does not validate device data
-        s.frc = valid && a.frc ? a.frc + (size_t)env * NFRC : nullptr;
+        s.prm_ctr = valid ? a.x.param_ctr[env] : 0; s.prm_drawn = 0;
+        s.lat_ctr = valid ? a.x.lat_ctr[env] : 0;
+        s.lat = valid ? min(max(a.x.latency[env], 0), cfg.frame_skip) : 0;    // mcb_set_env_latency does not validate device data
+        s.frc = valid && a.x.frc ? a.x.frc + (size_t)env * NFRC : nullptr;
       }
       __syncwarp();
     }
@@ -2646,7 +2651,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
       if (ok) ok = reset_env(s, a, m, lane, env, nba, nva, ctr);
       if (ok) {
         write_obs(s, m, cfg, lane, env, a.obs, a.ag, a.dg, achieved);
-        if constexpr (PRM) { if (a.con_n) write_contacts(s, a.con_n, a.con_geom, a.con, env, lane); }
+        if constexpr (PRM) { if (a.x.con_n) write_contacts(s, a.x.con_n, a.x.con_geom, a.x.con, env, lane); }
         if (lane == 0) { a.elapsed[env] = 0; a.ep_return[env] = 0; }
       }
       substeps = 2;
@@ -2657,7 +2662,7 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         __syncwarp();
         write_obs(s, m, cfg, lane, env, a.obs, a.ag, a.dg, achieved);
         if (a.debug && env == a.debug_env) debug_dump(s, a, lane, nva);
-        if constexpr (PRM) { if (a.con_n) write_contacts(s, a.con_n, a.con_geom, a.con, env, lane); }
+        if constexpr (PRM) { if (a.x.con_n) write_contacts(s, a.x.con_n, a.x.con_geom, a.x.con, env, lane); }
       }
       substeps = 1;
     } else {
@@ -2819,14 +2824,14 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
             double dummy[3];
             write_obs(s, m, cfg, lane, env, a.final_obs, nullptr, nullptr, dummy);
           }
-          if constexpr (PRM) { if (a.con_fn) write_contacts(s, a.con_fn, a.con_fgeom, a.con_f, env, lane); }   // the terminal state's
+          if constexpr (PRM) { if (a.x.con_fn) write_contacts(s, a.x.con_fn, a.x.con_fgeom, a.x.con_f, env, lane); }   // the terminal state's
           ok = reset_env(s, a, m, lane, env, nba, nva, ctr);
           if (ok) write_obs(s, m, cfg, lane, env, a.obs, a.ag, a.dg, achieved);
           el = 0; epret = 0; substeps += 2;
         }
         // the last forward pass: the substep loop's or the block_gripper one (euler, write_obs and the reward leave the rows alone),
         // or the reset's for an env that was just reset
-        if constexpr (PRM) { if (ok && a.con_n) write_contacts(s, a.con_n, a.con_geom, a.con, env, lane); }
+        if constexpr (PRM) { if (ok && a.x.con_n) write_contacts(s, a.x.con_n, a.x.con_geom, a.x.con, env, lane); }
         if (ok && lane == 0) {
           if (cfg.reward_type == 0) ((float*)a.reward)[env] = -(float)(dist > cfg.distance_threshold);
           else ((double*)a.reward)[env] = rew;
@@ -2860,10 +2865,10 @@ __global__ void __launch_bounds__(32 * Tier<TIER>::WARPS, 1) mcb_env_kernel(cons
         store_state(s, a.state + (size_t)env * MCB_STATE_STRIDE, lane);
         if constexpr (PRM) {
           if (s.prm_drawn) {
-            if (lane < MCB_NPARAM) a.params[(size_t)env * MCB_NPARAM + lane] = s.prm[lane];
-            if (lane == 0) { a.param_ctr[env] = s.prm_ctr; a.latency[env] = s.lat; a.lat_ctr[env] = s.lat_ctr; }
+            if (lane < MCB_NPARAM) a.x.params[(size_t)env * MCB_NPARAM + lane] = s.prm[lane];
+            if (lane == 0) { a.x.param_ctr[env] = s.prm_ctr; a.x.latency[env] = s.lat; a.x.lat_ctr[env] = s.lat_ctr; }
           }
-          if (a.frc && !s.frc) { for (int w = lane; w < NFRC; w += 32) a.frc[(size_t)env * NFRC + w] = 0.0; }   // a reset cleared the forces
+          if (a.x.frc && !s.frc) { for (int w = lane; w < NFRC; w += 32) a.x.frc[(size_t)env * NFRC + w] = 0.0; }   // a reset cleared the forces
         }
         if (lane == 0) {
           a.rng_ctr[env] = ctr;
@@ -2904,32 +2909,6 @@ __global__ void init_state_kernel(double* state, int* elapsed, double* ep_return
   elapsed[i] = 0; ep_return[i] = 0; ctr[i] = 0; env_seed[i] = seed;
 }
 
-// gather / scatter between the resident state record and caller arrays
-__global__ void state_io_kernel(double* state, int* elapsed, int n, double* qpos, double* qvel, double* ctrl, double* warm, double* goal, int* el, double* qprev, double* mocap, int write) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  double* st = state + (size_t)i * MCB_STATE_STRIDE;
-  if (write) {
-    if (qpos) { for (int k = 0; k < NQ; k++) st[ST_QPOS + k] = qpos[(size_t)i * NQ + k]; for (int k = 0; k < 6; k++) st[ST_QPREV + k] = st[ST_QPOS + k]; }
-    if (qvel) for (int k = 0; k < NV; k++) st[ST_QVEL + k] = qvel[(size_t)i * NV + k];
-    if (ctrl) for (int k = 0; k < NU; k++) st[ST_CTRL + k] = ctrl[(size_t)i * NU + k];
-    if (warm) for (int k = 0; k < NV; k++) st[ST_WARM + k] = warm[(size_t)i * NV + k];
-    if (goal) for (int k = 0; k < 3; k++) st[ST_GOAL + k] = goal[(size_t)i * 3 + k];
-    if (el) elapsed[i] = el[i];
-    if (qprev) for (int k = 0; k < 6; k++) st[ST_QPREV + k] = qprev[(size_t)i * 6 + k];
-    if (mocap) for (int k = 0; k < 7; k++) st[ST_MOCAP + k] = mocap[(size_t)i * 7 + k];
-  } else {
-    if (qpos) for (int k = 0; k < NQ; k++) qpos[(size_t)i * NQ + k] = st[ST_QPOS + k];
-    if (qvel) for (int k = 0; k < NV; k++) qvel[(size_t)i * NV + k] = st[ST_QVEL + k];
-    if (ctrl) for (int k = 0; k < NU; k++) ctrl[(size_t)i * NU + k] = st[ST_CTRL + k];
-    if (warm) for (int k = 0; k < NV; k++) warm[(size_t)i * NV + k] = st[ST_WARM + k];
-    if (goal) for (int k = 0; k < 3; k++) goal[(size_t)i * 3 + k] = st[ST_GOAL + k];
-    if (el) el[i] = elapsed[i];
-    if (qprev) for (int k = 0; k < 6; k++) qprev[(size_t)i * 6 + k] = st[ST_QPREV + k];
-    if (mocap) for (int k = 0; k < 7; k++) mocap[(size_t)i * 7 + k] = st[ST_MOCAP + k];
-  }
-}
-
 // DFMA throughput probe: 8 independent chains per thread
 __global__ void dfma_probe_kernel(double* out, int iters) {
   double a0 = threadIdx.x * 1e-9, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -2958,43 +2937,43 @@ __global__ void seed_kernel(unsigned long long* env_seed, unsigned long long* ct
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n && (!mask || mask[i])) { env_seed[i] = seed; ctr[i] = 0; if (pctr) pctr[i] = 0; if (lctr) lctr[i] = 0; }
 }
-// actuation latencies [N] and their draw counters [N]: set 0 batch -> caller (0 and 0 when the batch has none, lat == null),
-// set 1 caller -> batch; any caller pointer may be null
-__global__ void latency_io_kernel(int* lat, unsigned long long* ctr, int* u_lat, unsigned long long* u_ctr, int n, int set) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  if (set) { if (u_lat) lat[i] = u_lat[i]; if (u_ctr) ctr[i] = u_ctr[i]; }
-  else { if (u_lat) u_lat[i] = lat ? lat[i] : 0; if (u_ctr) u_ctr[i] = lat ? ctr[i] : 0; }
+// A row copy between a batch's arrays and caller arrays, one thread per (env, column): up to IO_MAXBLK column blocks, each the columns
+// [col, col + width) of a batch array with rows of `stride` elements of `elem` (4 or 8) bytes <-> the first `width` columns of a
+// caller array with rows of `ustride` elements.  GET: batch -> caller, a null batch array reads as the bit pattern `absent`; SET:
+// caller -> batch; FILL: `absent` -> batch.  No two blocks of a list write the same element, so their order does not matter.
+enum { IO_GET, IO_SET, IO_FILL, IO_MAXBLK = 8 };
+struct IoBlock { char *arr, *user; int stride, col, width, ustride, elem; unsigned long long absent; };
+struct IoList {
+  int dir, n = 0, width = 0;     // width: the columns of all blocks, per env
+  IoBlock blk[IO_MAXBLK];
+  // adds a block unless it has no caller array (a GET or SET call leaves such an array alone)
+  template <class T> IoList& add(T* arr, int stride, int col, int width, const void* user, T absent = T(), int ustride = 0) {
+    static_assert(sizeof(T) == 4 || sizeof(T) == 8, "4- or 8-byte elements");
+    if (!user && dir != IO_FILL) return *this;
+    IoBlock& c = blk[n++];
+    c = {(char*)arr, (char*)user, stride, col, width, ustride ? ustride : width, (int)sizeof(T), 0};
+    memcpy(&c.absent, &absent, sizeof(T));
+    this->width += width;
+    return *this;
+  }
+};
+template <class T> __device__ void copy_element(int dir, const IoBlock& c, size_t ia, size_t iu) {
+  T* arr = reinterpret_cast<T*>(c.arr);
+  T* user = reinterpret_cast<T*>(c.user);
+  const T absent = (T)c.absent;
+  if (dir == IO_GET) user[iu] = arr ? arr[ia] : absent;
+  else arr[ia] = dir == IO_SET ? user[iu] : absent;
 }
-// per-env parameters [N, MCB_NPARAM] and draw counters [N]: mode 0 batch -> caller (the nominal 1.0 and 0 when the batch has none,
-// params == null), 1 caller -> batch, 2 nominal values into the batch; any caller pointer may be null
-__global__ void params_io_kernel(double* params, unsigned long long* ctr, double* u_params, unsigned long long* u_ctr, int n, int mode) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const size_t o = (size_t)i * MCB_NPARAM;
-  if (mode == 2) { for (int k = 0; k < MCB_NPARAM; k++) params[o + k] = 1.0; ctr[i] = 0; }
-  else if (mode == 1) { if (u_params) for (int k = 0; k < MCB_NPARAM; k++) params[o + k] = u_params[o + k]; if (u_ctr) ctr[i] = u_ctr[i]; }
-  else { if (u_params) for (int k = 0; k < MCB_NPARAM; k++) u_params[o + k] = params ? params[o + k] : 1.0; if (u_ctr) u_ctr[i] = ctr ? ctr[i] : 0; }
-}
-// applied forces [N, NFRC] <-> qfrc [N, NV] and xfrc [N, NB, 6]: set 0 batch -> caller (zeros when the batch has none, frc == null),
-// set 1 caller -> batch; either caller pointer may be null.  One thread per (env, slot).
-__global__ void applied_io_kernel(double* frc, double* u_qfrc, double* u_xfrc, int n, int set) {
+__global__ void copy_rows_kernel(const __grid_constant__ IoList l, int n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (long long)n * NFRC) return;
-  const long long env = i / NFRC;
-  const int k = (int)(i - env * NFRC);
-  double* u = k < NV ? (u_qfrc ? u_qfrc + env * NV + k : nullptr) : (u_xfrc ? u_xfrc + env * (NB * 6) + (k - NV) : nullptr);
-  if (!u) return;
-  if (set) frc[i] = *u;
-  else *u = frc ? frc[i] : 0.0;
-}
-// the part of a checkpoint mcb_get_state / mcb_set_state do not carry: RNG streams and running episode returns
-__global__ void rng_io_kernel(unsigned long long* env_seed, unsigned long long* ctr, double* ep_return, unsigned long long* u_seed, unsigned long long* u_ctr,
-                              double* u_ret, int n, int write) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  if (write) { if (u_seed) env_seed[i] = u_seed[i]; if (u_ctr) ctr[i] = u_ctr[i]; if (u_ret) ep_return[i] = u_ret[i]; }
-  else { if (u_seed) u_seed[i] = env_seed[i]; if (u_ctr) u_ctr[i] = ctr[i]; if (u_ret) u_ret[i] = ep_return[i]; }
+  if (i >= (long long)n * l.width) return;
+  const long long env = i / l.width;
+  int k = (int)(i - env * l.width), j = 0;
+  while (k >= l.blk[j].width) k -= l.blk[j++].width;
+  const IoBlock& c = l.blk[j];
+  const size_t ia = (size_t)env * c.stride + c.col + k, iu = (size_t)env * c.ustride + k;
+  if (c.elem == 8) copy_element<unsigned long long>(l.dir, c, ia, iu);
+  else copy_element<unsigned int>(l.dir, c, ia, iu);
 }
 __global__ void iota_kernel(int* list, int* count, int n) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -3080,18 +3059,9 @@ struct mcb_batch {
   int last_launches;
   long long launches_total;   // kernels this library launched on behalf of the batch (counted at the launch sites)
   int lockstep_warps, tuned;
-  // per-env physics parameters: null until mcb_batch_set_param_ranges / mcb_set_env_params turn them on
-  double* params; unsigned long long* param_ctr;
-  int draw_params;
-  double param_lo[MCB_NPARAM], param_hi[MCB_NPARAM];
-  // actuation latency: allocated with the per-env parameters (0 substeps for every env until set or drawn)
-  int* latency; unsigned long long* lat_ctr;
-  int draw_latency, lat_lo, lat_hi;
-  // applied forces [N, NFRC]: null until mcb_set_env_applied turns them on (which turns per-env parameters on too)
-  double* frc;
-  // contact output: caller-owned device arrays (mcb_set_contact_output), null when off; the final triple is optional
-  int *con_n, *con_geom; double* con;
-  int *con_fn, *con_fgeom; double* con_f;
+  // per-env extensions: the parameters and latencies are null until a call turns per-env parameters on (enable_params), the applied
+  // forces until mcb_set_env_applied, the contact output until mcb_set_contact_output registers the caller's arrays
+  EnvExt x;
   // staging for the host-buffer entry point
   float* d_actions; double *d_obs, *d_ag, *d_dg, *d_fobs; void* d_reward; uint8_t* d_flags;
   float* h_actions; double *h_obs, *h_ag, *h_dg, *h_fobs; void* h_reward; uint8_t* h_flags;
@@ -3144,41 +3114,82 @@ static int launch(mcb_batch* b, StepArgs& a, cudaStream_t st) {
   { const char* st_ = getenv("MCB_CANARY_SELFTEST"); a.canary_selftest = (st_ && st_[0] == '1') ? 1 : 0; }
 #endif
   a.mid_threshold = b->mid_only ? -1 : 2 * Tier<2>::WARPS * b->sm_count;    // up to two waves of the last tier are cheaper than a middle-tier pass (profiles/README.md)
-  cudaError_t e;
-  if (!b->params) e = launch_tiers<false>(b, a, st);
-  else {
-    a.params = b->params; a.param_ctr = b->param_ctr; a.draw_params = b->draw_params;
-    memcpy(a.param_lo, b->param_lo, sizeof a.param_lo); memcpy(a.param_hi, b->param_hi, sizeof a.param_hi);
-    a.latency = b->latency; a.lat_ctr = b->lat_ctr; a.draw_latency = b->draw_latency; a.lat_lo = b->lat_lo; a.lat_hi = b->lat_hi;
-    a.frc = b->frc;
-    a.con_n = b->con_n; a.con_geom = b->con_geom; a.con = b->con; a.con_fn = b->con_fn; a.con_fgeom = b->con_fgeom; a.con_f = b->con_f;
-    e = prm_launch_tiers(b, &a, st);
-  }
+  a.x = b->x;
+  const cudaError_t e = b->x.params ? prm_launch_tiers(b, &a, st) : launch_tiers<false>(b, a, st);
   if (e != cudaSuccess) return fail("launching the step kernels", e);
   return 0;
+}
+
+// Every device array of a batch, described once: its member, its size (bytes per env plus a fixed part), the group it is allocated
+// with and whether a Snapshot carries it (what a step changes).  G_CONTACT arrays are the caller's (mcb_set_contact_output); the
+// batch allocates and frees the others.  A null array is absent: per-env parameters, applied forces or contact output are off.
+enum { G_CORE, G_PARAMS, G_FORCES, G_CONTACT };
+struct BatchArray { size_t off, per_env, fixed; int group; bool saved; };
+static const BatchArray kBatchArrays[] = {
+    {offsetof(mcb_batch, state), MCB_STATE_STRIDE * sizeof(double), 0, G_CORE, true},
+    {offsetof(mcb_batch, ep_return), sizeof(double), 0, G_CORE, true},
+    {offsetof(mcb_batch, elapsed), sizeof(int), 0, G_CORE, true},
+    {offsetof(mcb_batch, rng_ctr), sizeof(unsigned long long), 0, G_CORE, true},
+    {offsetof(mcb_batch, stats), 0, 8 * sizeof(double), G_CORE, true},
+    {offsetof(mcb_batch, env_seed), sizeof(unsigned long long), 0, G_CORE, false},
+    {offsetof(mcb_batch, redo_count), 0, 2 * sizeof(int), G_CORE, false},
+    {offsetof(mcb_batch, redo_list), 2 * sizeof(int), 0, G_CORE, false},
+    {offsetof(mcb_batch, debug), 0, DEBUG_DOUBLES * sizeof(double), G_CORE, false},
+    {offsetof(mcb_batch, x.params), MCB_NPARAM * sizeof(double), 0, G_PARAMS, true},
+    {offsetof(mcb_batch, x.param_ctr), sizeof(unsigned long long), 0, G_PARAMS, true},
+    {offsetof(mcb_batch, x.latency), sizeof(int), 0, G_PARAMS, true},
+    {offsetof(mcb_batch, x.lat_ctr), sizeof(unsigned long long), 0, G_PARAMS, true},
+    {offsetof(mcb_batch, x.frc), NFRC * sizeof(double), 0, G_FORCES, true},
+    {offsetof(mcb_batch, x.con_n), sizeof(int), 0, G_CONTACT, true},
+    {offsetof(mcb_batch, x.con_geom), MCB_MAXCON * 3 * sizeof(int), 0, G_CONTACT, true},
+    {offsetof(mcb_batch, x.con), MCB_MAXCON * MCB_CONTACT_DOUBLES * sizeof(double), 0, G_CONTACT, true},
+    {offsetof(mcb_batch, x.con_fn), sizeof(int), 0, G_CONTACT, true},
+    {offsetof(mcb_batch, x.con_fgeom), MCB_MAXCON * 3 * sizeof(int), 0, G_CONTACT, true},
+    {offsetof(mcb_batch, x.con_f), MCB_MAXCON * MCB_CONTACT_DOUBLES * sizeof(double), 0, G_CONTACT, true},
+};
+enum { NARRAY = sizeof kBatchArrays / sizeof kBatchArrays[0] };
+static void*& array_of(mcb_batch* b, const BatchArray& d) { return *reinterpret_cast<void**>(reinterpret_cast<char*>(b) + d.off); }
+static size_t bytes_of(const mcb_batch* b, const BatchArray& d) { return (size_t)b->n_envs * d.per_env + d.fixed; }
+
+static void free_group(mcb_batch* b, int group) {
+  for (const BatchArray& d : kBatchArrays)
+    if (d.group == group) { cudaFree(array_of(b, d)); array_of(b, d) = nullptr; }
+}
+// Allocates the arrays of one group, zero-filled, all or none (a failure leaves the group null).  Synchronises the device.
+static cudaError_t alloc_group(mcb_batch* b, int group) {
+  cudaError_t e = cudaSuccess;
+  for (const BatchArray& d : kBatchArrays) {
+    if (d.group != group || e != cudaSuccess) continue;
+    void* p = nullptr;
+    e = cudaMalloc(&p, bytes_of(b, d));
+    if (e == cudaSuccess) { array_of(b, d) = p; e = cudaMemset(p, 0, bytes_of(b, d)); }
+  }
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) free_group(b, group);
+  return e;
+}
+
+// One launch of copy_rows_kernel over the batch's envs (a list without blocks launches too: one launch per ABI call).
+static cudaError_t copy_rows(mcb_batch* b, const IoList& l, cudaStream_t st) {
+  const long long n = (long long)b->n_envs * l.width;
+  copy_rows_kernel<<<n ? (unsigned)((n + 255) / 256) : 1u, 256, 0, st>>>(l, b->n_envs);
+  const cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) b->launches_total++;
+  return e;
 }
 
 // Turns per-env parameters on: allocates them and the actuation latencies, sets every env to the nominal values (1.0, latency 0, draw
 // counters 0) and prepares the PRM kernels.  Synchronises the device.  A failure leaves the batch without per-env parameters.
 static int enable_params(mcb_batch* b, const char* who) {
-  if (b->params) return 0;
+  if (b->x.params) return 0;
   if (b->cfg.mesh_collision) { g_err = who; g_err += ": per-env parameters are not supported with mesh_collision (hull pairs keep the model's friction)"; return -1; }
   DevGuard guard(b->model->device);
   if (!guard.ok) return fail("enable per-env parameters: cannot select the batch's device", cudaGetLastError());
-  const size_t N = (size_t)b->n_envs;
-  double* p = nullptr; unsigned long long *c = nullptr, *lc = nullptr; int* lat = nullptr;
   cudaError_t e = prm_set_tier_smem();
-  if (e == cudaSuccess) e = cudaMalloc(&p, N * MCB_NPARAM * sizeof(double));
-  if (e == cudaSuccess) e = cudaMalloc(&c, N * sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaMalloc(&lat, N * sizeof(int));
-  if (e == cudaSuccess) e = cudaMalloc(&lc, N * sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaMemset(lat, 0, N * sizeof(int));
-  if (e == cudaSuccess) e = cudaMemset(lc, 0, N * sizeof(unsigned long long));
-  if (e == cudaSuccess) { params_io_kernel<<<(b->n_envs + 127) / 128, 128>>>(p, c, nullptr, nullptr, b->n_envs, 2); e = cudaGetLastError(); }
+  if (e == cudaSuccess) e = alloc_group(b, G_PARAMS);
+  if (e == cudaSuccess) e = copy_rows(b, IoList{IO_FILL}.add(b->x.params, MCB_NPARAM, 0, MCB_NPARAM, nullptr, 1.0), nullptr);
   if (e == cudaSuccess) e = cudaDeviceSynchronize();
-  if (e != cudaSuccess) { cudaFree(p); cudaFree(c); cudaFree(lat); cudaFree(lc); return fail("enable per-env parameters", e); }
-  b->launches_total++;
-  b->params = p; b->param_ctr = c; b->latency = lat; b->lat_ctr = lc;
+  if (e != cudaSuccess) { free_group(b, G_PARAMS); return fail("enable per-env parameters", e); }
   return 0;
 }
 
@@ -3207,33 +3218,25 @@ static cudaError_t alloc_staging(mcb_batch* b) {
   return e;
 }
 
-// A device copy of what a step changes in a batch: state records, episode returns, elapsed steps, RNG draw counters, statistics,
-// the per-env parameters and actuation latencies with their draw counters (auto-resets redraw them), the applied forces
-// (resets clear them) and the registered contact output.  The buffers are allocated by the first save() and freed with the snapshot.
+// A device copy of what a step changes in a batch: the arrays of kBatchArrays marked `saved` that the batch has.  The buffers are
+// allocated by the first save() and freed with the snapshot.
 struct Snapshot {
-  enum { NBUF = 16 };
-  const mcb_batch* b;
-  void* copy[NBUF] = {};
-  explicit Snapshot(const mcb_batch* batch) : b(batch) {}
+  mcb_batch* b;
+  void* copy[NARRAY] = {};
+  explicit Snapshot(mcb_batch* batch) : b(batch) {}
   ~Snapshot() { for (void* p : copy) cudaFree(p); }
   cudaError_t save(cudaStream_t st) { return transfer(true, st); }
   cudaError_t restore(cudaStream_t st) { return transfer(false, st); }
 
  private:
   cudaError_t transfer(bool save, cudaStream_t st) {
-    const size_t N = (size_t)b->n_envs;
-    void* live[NBUF] = {b->state, b->ep_return, b->elapsed, b->rng_ctr, b->stats, b->params, b->param_ctr, b->latency, b->lat_ctr, b->frc,
-                        b->con_n, b->con_geom, b->con, b->con_fn, b->con_fgeom, b->con_f};
-    const size_t NC = N * MCB_MAXCON;
-    const size_t bytes[NBUF] = {N * MCB_STATE_STRIDE * sizeof(double), N * sizeof(double), N * sizeof(int), N * sizeof(unsigned long long), 8 * sizeof(double),
-                                N * MCB_NPARAM * sizeof(double), N * sizeof(unsigned long long), N * sizeof(int), N * sizeof(unsigned long long),
-                                N * NFRC * sizeof(double), N * sizeof(int), NC * 3 * sizeof(int), NC * MCB_CONTACT_DOUBLES * sizeof(double),
-                                N * sizeof(int), NC * 3 * sizeof(int), NC * MCB_CONTACT_DOUBLES * sizeof(double)};
     cudaError_t e = cudaSuccess;
-    for (int k = 0; k < NBUF && e == cudaSuccess; k++) {
-      if (!live[k]) continue;      // a batch without per-env parameters, applied forces or contact output
-      if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes[k]);
-      if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live[k], save ? live[k] : copy[k], bytes[k], cudaMemcpyDeviceToDevice, st);
+    for (int k = 0; k < NARRAY && e == cudaSuccess; k++) {
+      const BatchArray& d = kBatchArrays[k];
+      void* live = array_of(b, d);
+      if (!d.saved || !live) continue;
+      if (save && !copy[k]) e = cudaMalloc(&copy[k], bytes_of(b, d));
+      if (e == cudaSuccess) e = cudaMemcpyAsync(save ? copy[k] : live, save ? live : copy[k], bytes_of(b, d), cudaMemcpyDeviceToDevice, st);
     }
     return e;
   }
@@ -3380,24 +3383,10 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
   if (e == cudaSuccess) e = set_tier_smem<1>();
   if (e == cudaSuccess) e = set_tier_smem<2>();
   if (e != cudaSuccess) { delete b; return fail("cudaFuncSetAttribute(shared memory)", e); }
-  size_t N = (size_t)n_envs;
-  // partial allocations are released on failure (mcb_batch_destroy frees whatever is non-null)
-#define CKB(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { mcb_batch_destroy(b); return fail(#call, e_); } } while (0)
-  CKB(cudaMalloc(&b->state, N * MCB_STATE_STRIDE * sizeof(double)));
-  CKB(cudaMalloc(&b->elapsed, N * sizeof(int)));
-  CKB(cudaMalloc(&b->ep_return, N * sizeof(double)));
-  CKB(cudaMalloc(&b->rng_ctr, N * sizeof(unsigned long long)));
-  CKB(cudaMalloc(&b->env_seed, N * sizeof(unsigned long long)));
-  CKB(cudaMalloc(&b->stats, 8 * sizeof(double)));
-  CKB(cudaMalloc(&b->redo_count, 2 * sizeof(int)));
-  CKB(cudaMalloc(&b->redo_list, 2 * N * sizeof(int)));
-  CKB(cudaMemset(b->redo_count, 0, 2 * sizeof(int)));
-  CKB(cudaMalloc(&b->debug, DEBUG_DOUBLES * sizeof(double)));
-  CKB(cudaMemset(b->stats, 0, 8 * sizeof(double)));
+  if ((e = alloc_group(b, G_CORE)) != cudaSuccess) { delete b; return fail("mcb_batch_create: allocating the batch", e); }
   init_state_kernel<<<(n_envs + 127) / 128, 128>>>(b->state, b->elapsed, b->ep_return, b->rng_ctr, b->env_seed, (unsigned long long)seed, m->dev, n_envs, cfg->fetch_env);
-  CKB(cudaGetLastError());
-  CKB(cudaDeviceSynchronize());
-#undef CKB
+  if ((e = cudaGetLastError()) == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) { mcb_batch_destroy(b); return fail("mcb_batch_create: init_state_kernel", e); }
   b->launches_total = 1;
   b->lockstep_warps = cfg->lockstep_warps ? cfg->lockstep_warps : 1;   // 0: free-running until mcb_autotune() is called (explicitly: mcb_step never tunes)
   b->tuned = cfg->lockstep_warps != 0;
@@ -3407,8 +3396,7 @@ int32_t mcb_batch_create(mcb_model* m, int32_t n_envs, const mcb_task_cfg* cfg, 
 
 int32_t mcb_batch_destroy(mcb_batch* b) {
   if (!b) return 0;
-  cudaFree(b->state); cudaFree(b->elapsed); cudaFree(b->ep_return); cudaFree(b->rng_ctr); cudaFree(b->env_seed); cudaFree(b->stats); cudaFree(b->debug); cudaFree(b->redo_count); cudaFree(b->redo_list);
-  cudaFree(b->params); cudaFree(b->param_ctr); cudaFree(b->latency); cudaFree(b->lat_ctr); cudaFree(b->frc);
+  for (const BatchArray& d : kBatchArrays) if (d.group != G_CONTACT) cudaFree(array_of(b, d));
   free_staging(b);
   delete b;
   return 0;
@@ -3521,20 +3509,24 @@ int32_t mcb_debug_forward(mcb_batch* b, int32_t env, int32_t what, double* h_out
   return DEBUG_DOUBLES;
 }
 
+// the columns of the state record and the elapsed steps: mcb_get_state / mcb_set_state
+static IoList state_cols(mcb_batch* b, int dir, const double* qpos, const double* qvel, const double* ctrl, const double* warm, const double* goal,
+                         const int32_t* elapsed, const double* qprev, const double* mocap) {
+  const int S = MCB_STATE_STRIDE;
+  return IoList{dir}.add(b->state, S, ST_QPOS, NQ, qpos).add(b->state, S, ST_QVEL, NV, qvel).add(b->state, S, ST_CTRL, NU, ctrl).add(b->state, S, ST_WARM, NV, warm)
+      .add(b->state, S, ST_GOAL, 3, goal).add(b->elapsed, 1, 0, 1, elapsed).add(b->state, S, ST_QPREV, 6, qprev).add(b->state, S, ST_MOCAP, 7, mocap);
+}
 int32_t mcb_get_state(mcb_batch* b, double* qpos, double* qvel, double* ctrl, double* warm, double* goal, int32_t* elapsed, double* qprev, double* mocap, void* stream) {
   if (!b) return fail("mcb_get_state: null batch");
-  state_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->state, b->elapsed, b->n_envs, qpos, qvel, ctrl, warm, goal, elapsed, qprev, mocap, 0);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, state_cols(b, IO_GET, qpos, qvel, ctrl, warm, goal, elapsed, qprev, mocap), (cudaStream_t)stream));
   return 0;
 }
 int32_t mcb_set_state(mcb_batch* b, const double* qpos, const double* qvel, const double* ctrl, const double* warm, const double* goal,
                       const int32_t* elapsed, const double* qprev, const double* mocap, void* stream) {
   if (!b) return fail("mcb_set_state: null batch");
-  state_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->state, b->elapsed, b->n_envs, (double*)qpos, (double*)qvel, (double*)ctrl,
-                                                                             (double*)warm, (double*)goal, (int*)elapsed, (double*)qprev, (double*)mocap, 1);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  IoList l = state_cols(b, IO_SET, qpos, qvel, ctrl, warm, goal, elapsed, qprev, mocap);
+  if (qpos && !qprev) l.add(b->state, MCB_STATE_STRIDE, ST_QPREV, 6, qpos, 0.0, NQ);     // qprev := qpos[0:6]
+  CK(copy_rows(b, l, (cudaStream_t)stream));
   return 0;
 }
 
@@ -3620,7 +3612,7 @@ int32_t mcb_reset_host(mcb_batch* b, const uint8_t* h_mask, const double* h_obj_
 
 int32_t mcb_seed(mcb_batch* b, uint64_t seed, const uint8_t* mask, void* stream) {
   if (!b) return fail("mcb_seed: null batch");
-  seed_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->param_ctr, b->lat_ctr, mask, (unsigned long long)seed, b->n_envs);
+  seed_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->x.param_ctr, b->x.lat_ctr, mask, (unsigned long long)seed, b->n_envs);
   CK(cudaGetLastError());
   b->launches_total++;
   if (!mask) b->seed = seed;
@@ -3629,109 +3621,93 @@ int32_t mcb_seed(mcb_batch* b, uint64_t seed, const uint8_t* mask, void* stream)
 
 int32_t mcb_get_rng_state(mcb_batch* b, uint64_t* env_seed, uint64_t* draw_counter, double* ep_return, void* stream) {
   if (!b) return fail("mcb_get_rng_state: null batch");
-  rng_io_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->ep_return, (unsigned long long*)env_seed,
-                                                                        (unsigned long long*)draw_counter, ep_return, b->n_envs, 0);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, IoList{IO_GET}.add(b->env_seed, 1, 0, 1, env_seed).add(b->rng_ctr, 1, 0, 1, draw_counter).add(b->ep_return, 1, 0, 1, ep_return),
+                (cudaStream_t)stream));
   return 0;
 }
 int32_t mcb_set_rng_state(mcb_batch* b, const uint64_t* env_seed, const uint64_t* draw_counter, const double* ep_return, void* stream) {
   if (!b) return fail("mcb_set_rng_state: null batch");
-  rng_io_kernel<<<(b->n_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(b->env_seed, b->rng_ctr, b->ep_return, (unsigned long long*)env_seed,
-                                                                        (unsigned long long*)draw_counter, (double*)ep_return, b->n_envs, 1);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, IoList{IO_SET}.add(b->env_seed, 1, 0, 1, env_seed).add(b->rng_ctr, 1, 0, 1, draw_counter).add(b->ep_return, 1, 0, 1, ep_return),
+                (cudaStream_t)stream));
   return 0;
 }
 
 int32_t mcb_batch_set_param_ranges(mcb_batch* b, const double* h_lo, const double* h_hi) {
   if (!b) return fail("mcb_batch_set_param_ranges: null batch");
   if (!h_lo != !h_hi) return fail("mcb_batch_set_param_ranges: pass both bounds, or neither to stop drawing");
-  if (!h_lo) { b->draw_params = 0; return 0; }
+  if (!h_lo) { b->x.draw_params = 0; return 0; }
   for (int k = 0; k < MCB_NPARAM; k++)
     if (!(std::isfinite(h_lo[k]) && std::isfinite(h_hi[k]) && h_lo[k] > 0 && h_lo[k] <= h_hi[k]))
       return fail("mcb_batch_set_param_ranges: every range must be finite with 0 < lo <= hi");
   if (enable_params(b, "mcb_batch_set_param_ranges")) return -1;
-  memcpy(b->param_lo, h_lo, sizeof b->param_lo); memcpy(b->param_hi, h_hi, sizeof b->param_hi);
-  b->draw_params = 1;
+  memcpy(b->x.param_lo, h_lo, sizeof b->x.param_lo); memcpy(b->x.param_hi, h_hi, sizeof b->x.param_hi);
+  b->x.draw_params = 1;
   return 0;
 }
 
+// a batch without per-env parameters reads as the nominal 1.0 and draw counter 0
+static IoList param_cols(mcb_batch* b, int dir, const double* params, const uint64_t* draw_counter) {
+  return IoList{dir}.add(b->x.params, MCB_NPARAM, 0, MCB_NPARAM, params, 1.0).add(b->x.param_ctr, 1, 0, 1, draw_counter);
+}
 int32_t mcb_get_env_params(mcb_batch* b, double* params, uint64_t* draw_counter, void* stream) {
   if (!b) return fail("mcb_get_env_params: null batch");
-  params_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->params, b->param_ctr, params, (unsigned long long*)draw_counter, b->n_envs, 0);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, param_cols(b, IO_GET, params, draw_counter), (cudaStream_t)stream));
   return 0;
 }
 
 int32_t mcb_set_env_params(mcb_batch* b, const double* params, const uint64_t* draw_counter, void* stream) {
   if (!b) return fail("mcb_set_env_params: null batch");
   if (enable_params(b, "mcb_set_env_params")) return -1;
-  params_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->params, b->param_ctr, (double*)params, (unsigned long long*)draw_counter, b->n_envs, 1);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, param_cols(b, IO_SET, params, draw_counter), (cudaStream_t)stream));
   return 0;
 }
 
 int32_t mcb_batch_set_latency_range(mcb_batch* b, int32_t lo, int32_t hi) {
   if (!b) return fail("mcb_batch_set_latency_range: null batch");
-  if (lo == -1 && hi == -1) { b->draw_latency = 0; return 0; }
+  if (lo == -1 && hi == -1) { b->x.draw_latency = 0; return 0; }
   if (!(0 <= lo && lo <= hi && hi <= b->cfg.frame_skip)) return fail("mcb_batch_set_latency_range: the range must satisfy 0 <= lo <= hi <= frame_skip");
   if (enable_params(b, "mcb_batch_set_latency_range")) return -1;
-  b->lat_lo = lo; b->lat_hi = hi;
-  b->draw_latency = 1;
+  b->x.lat_lo = lo; b->x.lat_hi = hi;
+  b->x.draw_latency = 1;
   return 0;
 }
 
 int32_t mcb_get_env_latency(mcb_batch* b, int32_t* latency, uint64_t* draw_counter, void* stream) {
   if (!b) return fail("mcb_get_env_latency: null batch");
-  latency_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->latency, b->lat_ctr, latency, (unsigned long long*)draw_counter, b->n_envs, 0);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, IoList{IO_GET}.add(b->x.latency, 1, 0, 1, latency).add(b->x.lat_ctr, 1, 0, 1, draw_counter), (cudaStream_t)stream));
   return 0;
 }
 
 int32_t mcb_set_env_latency(mcb_batch* b, const int32_t* latency, const uint64_t* draw_counter, void* stream) {
   if (!b) return fail("mcb_set_env_latency: null batch");
   if (enable_params(b, "mcb_set_env_latency")) return -1;
-  latency_io_kernel<<<(b->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(b->latency, b->lat_ctr, (int*)latency, (unsigned long long*)draw_counter, b->n_envs, 1);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, IoList{IO_SET}.add(b->x.latency, 1, 0, 1, latency).add(b->x.lat_ctr, 1, 0, 1, draw_counter), (cudaStream_t)stream));
   return 0;
 }
 
+// applied forces [N, NFRC] as qfrc [N, NV] and xfrc [N, NB, 6]; a batch without forces reads as zeros
+static IoList applied_cols(mcb_batch* b, int dir, const double* qfrc, const double* xfrc) {
+  return IoList{dir}.add(b->x.frc, NFRC, 0, NV, qfrc).add(b->x.frc, NFRC, NV, NB * 6, xfrc);
+}
 int32_t mcb_set_env_applied(mcb_batch* b, const double* qfrc, const double* xfrc, void* stream) {
   if (!b) return fail("mcb_set_env_applied: null batch");
   if (b->cfg.mesh_collision) return fail("mcb_set_env_applied: applied forces are not supported with mesh_collision");
-  if (!b->frc) {
+  if (!b->x.frc) {
     // first call: zeroed forces for every env, and the PRM kernels that read them; synchronises (not capturable)
     if (enable_params(b, "mcb_set_env_applied")) return -1;
     DevGuard guard(b->model->device);
     if (!guard.ok) return fail("mcb_set_env_applied: cannot select the batch's device", cudaGetLastError());
-    double* f = nullptr;
-    const size_t bytes = (size_t)b->n_envs * NFRC * sizeof(double);
-    cudaError_t e = cudaMalloc(&f, bytes);
-    if (e == cudaSuccess) e = cudaMemset(f, 0, bytes);
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();
-    if (e != cudaSuccess) { cudaFree(f); return fail("mcb_set_env_applied: allocating the forces", e); }
-    b->frc = f;
+    if (const cudaError_t e = alloc_group(b, G_FORCES)) return fail("mcb_set_env_applied: allocating the forces", e);
   }
   if (!qfrc && !xfrc) return 0;
-  const long long n = (long long)b->n_envs * NFRC;
-  applied_io_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(b->frc, (double*)qfrc, (double*)xfrc, b->n_envs, 1);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, applied_cols(b, IO_SET, qfrc, xfrc), (cudaStream_t)stream));
   return 0;
 }
 
 int32_t mcb_get_env_applied(mcb_batch* b, double* qfrc, double* xfrc, void* stream) {
   if (!b) return fail("mcb_get_env_applied: null batch");
   if (!qfrc && !xfrc) return 0;
-  const long long n = (long long)b->n_envs * NFRC;
-  applied_io_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(b->frc, qfrc, xfrc, b->n_envs, 0);
-  CK(cudaGetLastError());
-  b->launches_total++;
+  CK(copy_rows(b, applied_cols(b, IO_GET, qfrc, xfrc), (cudaStream_t)stream));
   return 0;
 }
 
@@ -3749,8 +3725,8 @@ int32_t mcb_set_contact_output(mcb_batch* b, int32_t* ncon, int32_t* geom, doubl
   DevGuard guard(b->model->device);
   if (!guard.ok) return fail("mcb_set_contact_output: cannot select the batch's device", cudaGetLastError());
   CK(cudaDeviceSynchronize());
-  b->con_n = ncon; b->con_geom = geom; b->con = con;
-  b->con_fn = final_ncon; b->con_fgeom = final_geom; b->con_f = final_con;
+  b->x.con_n = ncon; b->x.con_geom = geom; b->x.con = con;
+  b->x.con_fn = final_ncon; b->x.con_fgeom = final_geom; b->x.con_f = final_con;
   return 0;
 }
 

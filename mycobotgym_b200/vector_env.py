@@ -162,6 +162,12 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+# The optional groups of get_state() / set_state(): group -> (its two keys, the getter, the setter taking the two arrays)
+_OPTIONAL = {"params": (("params", "param_counter"), "get_params", "set_params"),
+             "latency": (("latency", "latency_counter"), "get_latency", "set_latency"),
+             "forces": (("qfrc_applied", "xfrc_applied"), "get_applied_forces", "set_applied_forces")}
+
+
 class MyCobotVectorEnv:
     metadata = {"render_modes": [], "render_fps": 25}
 
@@ -235,12 +241,11 @@ class MyCobotVectorEnv:
             lo, hi = (np.ascontiguousarray(x, dtype=np.float64) for x in bounds)
             with torch.cuda.device(dev_index):
                 _lib.check(self._L.mcb_batch_set_param_ranges(h, lo.ctypes.data_as(C.c_void_p), hi.ctypes.data_as(C.c_void_p)))
-        self._has_params = bounds is not None
         if lat_bounds is not None:
             with torch.cuda.device(dev_index):
                 _lib.check(self._L.mcb_batch_set_latency_range(h, *lat_bounds))
-        self._has_latency = lat_bounds is not None
-        self._has_forces = False
+        # the optional groups of get_state(): those turned on by a constructor argument or a set_* call
+        self._groups = {g for g, on in (("params", bounds is not None), ("latency", lat_bounds is not None)) if on}
         self.obs_dim = self._L.mcb_batch_obs_dim(h)
         self.action_dim = self._L.mcb_batch_action_dim(h)          # 7 (joint, IK), 8 (mocap), 4 (fetch variants) (mycobot.py:90-97)
         N, dev = self.num_envs, self.device
@@ -283,6 +288,13 @@ class MyCobotVectorEnv:
     # ------------------------------------------------------------------ helpers
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _get(self, getter, *arrays):
+        """New device tensors [N, *shape] of the given (shape, dtype), filled by one C getter (batch, pointers..., stream)."""
+        ts = tuple(torch.empty(self.num_envs, *shape, dtype=dt, device=self.device) for shape, dt in arrays)
+        with torch.cuda.device(self._dev_index):
+            _lib.check(getter(self._batch, *(_ptr(t) for t in ts), self._stream()))
+        return ts
 
     def _obs_dict(self):
         return {"observation": self._obs, "achieved_goal": self._ag, "desired_goal": self._dg}
@@ -410,12 +422,9 @@ class MyCobotVectorEnv:
                   qprev=torch.empty(N, 6, dtype=torch.float64, device=dev), mocap=torch.empty(N, 7, dtype=torch.float64, device=dev),
                   env_seed=torch.empty(N, dtype=torch.int64, device=dev), rng_counter=torch.empty(N, dtype=torch.int64, device=dev),
                   ep_return=torch.empty(N, dtype=torch.float64, device=dev))
-        if self._has_params:
-            st["params"], st["param_counter"] = self.get_params()
-        if self._has_latency:
-            st["latency"], st["latency_counter"] = self.get_latency()
-        if self._has_forces:
-            st["qfrc_applied"], st["xfrc_applied"] = self.get_applied_forces()
+        for g, (keys, get, _) in _OPTIONAL.items():
+            if g in self._groups:
+                st.update(zip(keys, getattr(self, get)()))
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_get_rng_state(self._batch, _ptr(st["env_seed"]), _ptr(st["rng_counter"]), _ptr(st["ep_return"]), self._stream()))
             _lib.check(self._L.mcb_get_state(self._batch, _ptr(st["qpos"]), _ptr(st["qvel"]), _ptr(st["ctrl"]),
@@ -444,23 +453,18 @@ class MyCobotVectorEnv:
             _lib.check(self._L.mcb_set_state(self._batch, *[_ptr(t) for t in ts], self._stream()))
             if any(t is not None for t in rs):
                 _lib.check(self._L.mcb_set_rng_state(self._batch, *[_ptr(t) for t in rs], self._stream()))
-        if params is not None or param_counter is not None:
-            self.set_params(params, draw_counter=param_counter)
-        if latency is not None or latency_counter is not None:
-            self.set_latency(latency, draw_counter=latency_counter)
-        if qfrc_applied is not None or xfrc_applied is not None:
-            self.set_applied_forces(qfrc_applied, xfrc_applied)
+        given = dict(params=params, param_counter=param_counter, latency=latency, latency_counter=latency_counter,
+                     qfrc_applied=qfrc_applied, xfrc_applied=xfrc_applied)
+        for keys, _, set_ in _OPTIONAL.values():
+            a, b = (given[k] for k in keys)
+            if a is not None or b is not None:
+                getattr(self, set_)(a, b)
         torch.cuda.current_stream(self.device).synchronize()
 
     def get_params(self):
         """(params float64 [N, NPARAM], draw counters int64 [N]) as device tensors: the per-env multipliers (`flatten.PARAM_NAMES`)
         in use and how many parameter draws each env has made since it was seeded.  Without per-env parameters: 1.0 and 0."""
-        N, dev = self.num_envs, self.device
-        p = torch.empty(N, flatten.NPARAM, dtype=torch.float64, device=dev)
-        c = torch.empty(N, dtype=torch.int64, device=dev)
-        with torch.cuda.device(self._dev_index):
-            _lib.check(self._L.mcb_get_env_params(self._batch, _ptr(p), _ptr(c), self._stream()))
-        return p, c
+        return self._get(self._L.mcb_get_env_params, ((flatten.NPARAM,), torch.float64), ((), torch.int64))
 
     def set_params(self, params, draw_counter=None):
         """Fixed per-env multipliers [N, NPARAM] (evaluation, system identification); either argument may be None.  Turns per-env
@@ -481,17 +485,12 @@ class MyCobotVectorEnv:
                 raise ValueError(f"draw_counter must have shape {(N,)}, got {tuple(c.shape)}")
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_set_env_params(self._batch, _ptr(p), _ptr(c), self._stream()))
-        self._has_params = True
+        self._groups.add("params")
 
     def get_latency(self):
         """(latency int32 [N], draw counters int64 [N]) as device tensors: each env's actuation latency in substeps and how many
         latency draws it has made since it was seeded.  Without latency: 0 and 0."""
-        N, dev = self.num_envs, self.device
-        d = torch.empty(N, dtype=torch.int32, device=dev)
-        c = torch.empty(N, dtype=torch.int64, device=dev)
-        with torch.cuda.device(self._dev_index):
-            _lib.check(self._L.mcb_get_env_latency(self._batch, _ptr(d), _ptr(c), self._stream()))
-        return d, c
+        return self._get(self._L.mcb_get_env_latency, ((), torch.int32), ((), torch.int64))
 
     def set_latency(self, latency, draw_counter=None):
         """Fixed per-env actuation latencies [N] in substeps, integers in [0, frame_skip] (evaluation, system identification); either
@@ -515,17 +514,12 @@ class MyCobotVectorEnv:
                 raise ValueError(f"draw_counter must have shape {(N,)}, got {tuple(c.shape)}")
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_set_env_latency(self._batch, _ptr(d), _ptr(c), self._stream()))
-        self._has_latency = True
+        self._groups.add("latency")
 
     def get_applied_forces(self):
         """(qfrc_applied float64 [N, 18], xfrc_applied float64 [N, 13, 6]) as device tensors: the forces the step applies (see
         `set_applied_forces`).  Without forces: zeros."""
-        N, dev = self.num_envs, self.device
-        q = torch.empty(N, flatten.NV, dtype=torch.float64, device=dev)
-        x = torch.empty(N, flatten.NB, 6, dtype=torch.float64, device=dev)
-        with torch.cuda.device(self._dev_index):
-            _lib.check(self._L.mcb_get_env_applied(self._batch, _ptr(q), _ptr(x), self._stream()))
-        return q, x
+        return self._get(self._L.mcb_get_env_applied, ((flatten.NV,), torch.float64), ((flatten.NB, 6), torch.float64))
 
     def set_applied_forces(self, qfrc_applied=None, xfrc_applied=None):
         """Per-env external forces, MuJoCo's `data.qfrc_applied` and `data.xfrc_applied` on the reduced model (DESIGN.md section 11):
@@ -541,7 +535,7 @@ class MyCobotVectorEnv:
         x = None if x is None else x.to(self.device)
         with torch.cuda.device(self._dev_index):
             _lib.check(self._L.mcb_set_env_applied(self._batch, _ptr(q), _ptr(x), self._stream()))
-        self._has_forces = True
+        self._groups.add("forces")
 
     def contacts(self, final=False):
         """The contacts of each env's last forward pass (MuJoCo's `data.contact` with `mj_contactForce`), as named views of the env's
